@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark: the mplan2vdl-emitted TPC-H Q6 plan over synthetic SF100 lineitem
 columns resident in HBM (BASELINE.json north_star), executed by libvdl_cuda.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--query q06|q01] [--sf 100]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--query q06|q01] [--sf 100] [--dump-outputs DIR]
 
 One "step" = one execution of the plan over the whole (sharded) table: ONE launch of the fused scan-fold
 kernel per GPU, whose last thread block [exchanges the partial tables with the other GPUs through peer memory
@@ -14,6 +14,7 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import re
 import statistics
 import subprocess
 import sys
@@ -188,6 +189,24 @@ def check_parity(cat, query: str, sf: float, result: dict, chunk_rows: int = 40_
             "mismatched_outputs": bad, "oracle_seconds": round(co.seconds, 2), "seconds": round(time.perf_counter() - t0, 2)}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(result: dict, out_dir: str, seed: int = 0) -> None:
+    """Every result column as <out_dir>/<name>.npy in float64, so that two builds of the project can be compared output
+    for output.  Integer results beyond 2**53 (fixed-point sums at large scale factors) are rounded to the nearest double,
+    so a difference in their last units does not show.  Past DUMP_BYTES in all, every column keeps the same seeded sample
+    of its rows, in row order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keep = max(1, (DUMP_BYTES // max(len(result), 1) - 128) // 8)      # 128: the .npy header
+    for name, col in result.items():
+        col = np.asarray(col)
+        if len(col) > keep:
+            col = col[np.sort(np.random.default_rng(seed).choice(len(col), keep, replace=False))]
+        np.save(os.path.join(out_dir, re.sub(r"[^A-Za-z0-9_.-]", "_", name) + ".npy"), col.astype(np.float64))
+
+
 def workload_config(args):
     """Identical for both arms (--impl ours / reference): a function of the command line only."""
     from mplan2vdl_b200 import synth, tpch
@@ -227,7 +246,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the whole-table CPU-oracle check of the result")
     ap.add_argument("--int64-results", action="store_true", help="every result column crosses PCIe as int64 (default: int32 where the values provably fit)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/<output>.npy "
+                    "(float64, so integers beyond 2**53, such as Q1's fixed-point sums at SF100, are rounded; a seeded "
+                    "sample of the rows when the result exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm runs on a prefix of the table, its result is not the workload's")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -329,6 +355,8 @@ def main():
     result = sharded.global_result() if sharded.tail_mode else {k: np.array(v, copy=True) for k, v in result.items()}
     launches = ctx.launch_count - launches0
     clocks = sampler.stop() if rank == 0 else {}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(result, args.dump_outputs)
     if world > 1:
         t = torch.tensor([dev_ms, kern_mean], dtype=torch.float64, device=f"cuda:{local}")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from mplan2vdl_b200 import synth, tpch, tpch_queries, vlite
-from util import assert_same, host_columns, run_gpu, run_oracle
+from util import FIXTURES, assert_same, host_columns, needs_reference, run_gpu, run_oracle
 
 SF = 0.01
 QUERIES = ["q06", "q01", "q03", "q05"]
@@ -120,13 +120,11 @@ def test_without_the_cleanup_passes_the_program_is_longer_and_means_the_same(cat
     assert_same(run_oracle(raw, cols), run_oracle(clean, cols))
 
 
+@needs_reference
 def test_catalogue_from_the_four_metadata_files_is_the_built_in_one(catalog):
-    import os
     from mplan2vdl_b200 import mplan
     from mplan2vdl_b200.meta import load_metadata_files
-    d = "/root/reference/tests/tpch10noorder"
-    if not os.path.isdir(d):
-        pytest.skip("reference fixtures not mounted (GPU box)")
+    d = FIXTURES
     cat = load_metadata_files(f"{d}/bounds.csv", f"{d}/storage.csv", f"{d}/schema.msqldump", f"{d}/dictionary.csv")
     for n in ("01", "05", "16"):
         src = open(f"{d}/{n}.sql.mplan").read()

@@ -9,10 +9,7 @@ import pytest
 
 import ir_eval
 from mplan2vdl_b200 import mplan, tpch, vlite
-from util import assert_same, host_columns, run_gpu, run_oracle
-
-FIXTURES = "/root/reference/tests/tpch10noorder"
-needs_reference = pytest.mark.skipif(not os.path.isdir(FIXTURES), reason="reference fixtures not mounted (GPU box)")
+from util import FIXTURES, assert_same, host_columns, needs_reference, run_gpu, run_oracle
 
 PAIRS = "\n".join(["1,Load,a.x", "2,Load,b.y", "3,CrossProductOuter,Id 1,Id 2", "4,CrossProductInner,Id 1,Id 2",
                    "5,Gather,Id 1,Id 3,val", "6,Gather,Id 2,Id 4,val", "7,Multiply,val,Id 5,val,Id 6,val",

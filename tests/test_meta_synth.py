@@ -1,13 +1,10 @@
 """Metadata loaders (reference file formats) and the synthetic recipe."""
-import os
-
 import numpy as np
 import pytest
 
 from mplan2vdl_b200 import meta, synth
 from oracle.oracle import gen_column
-
-REF = "/root/reference/tests/tpch10noorder"
+from util import FIXTURES, needs_reference
 
 
 def test_loaders_on_a_tiny_directory(tmp_path):
@@ -36,9 +33,9 @@ def test_bad_record_width_is_rejected(tmp_path):
         meta.read_bounds(str(tmp_path / "bounds.csv"))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+@needs_reference
 def test_builtin_catalog_is_the_reference_metadata():
-    assert meta.load_metadata(REF).to_json() == meta.builtin_catalog().to_json()
+    assert meta.load_metadata(FIXTURES).to_json() == meta.builtin_catalog().to_json()
 
 
 def test_builtin_catalog_facts(catalog):

@@ -5,10 +5,7 @@ import os
 import pytest
 
 from mplan2vdl_b200 import mplan, tpch_queries, vlite
-from util import host_columns, plan_text, run_oracle
-
-FIXTURES = "/root/reference/tests/tpch10noorder"
-needs_reference = pytest.mark.skipif(not os.path.isdir(FIXTURES), reason="reference fixtures not mounted (GPU box)")
+from util import FIXTURES, host_columns, needs_reference, plan_text, run_oracle
 
 
 @needs_reference

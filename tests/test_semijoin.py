@@ -11,10 +11,8 @@ import pytest
 import ir_eval
 from mplan2vdl_b200 import mplan, synth, tpch, tpch_queries, vlite
 from mplan2vdl_b200.vlite import Bin, GroupBy, Join, Lit, Project, Ref, Select, Table
-from util import assert_same, host_columns, plan_text, run_oracle
+from util import FIXTURES, assert_same, host_columns, needs_reference, plan_text, run_oracle
 
-FIXTURES = "/root/reference/tests/tpch10noorder"
-needs_reference = pytest.mark.skipif(not os.path.isdir(FIXTURES), reason="reference fixtures not mounted (GPU box)")
 SF = 0.01
 
 

@@ -3,10 +3,18 @@ import os
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+
+# The reference translator's own MonetDB plans and metadata files (tests/tpch10noorder of an orm011/mplan2vdl checkout)
+# are not part of this repository.  The tests that translate them run when MPLAN2VDL_REFERENCE names such a checkout.
+REFERENCE = os.environ.get("MPLAN2VDL_REFERENCE", "")
+FIXTURES = os.path.join(REFERENCE, "tests", "tpch10noorder") if REFERENCE else ""
+needs_reference = pytest.mark.skipif(not os.path.isdir(FIXTURES),
+                                     reason="needs MPLAN2VDL_REFERENCE: a checkout of the reference translator (orm011/mplan2vdl)")
 
 from mplan2vdl_b200 import synth  # noqa: E402
 from oracle.oracle import Oracle, gen_column  # noqa: E402
