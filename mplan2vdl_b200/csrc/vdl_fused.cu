@@ -415,14 +415,16 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     }
     a.soff = k.soff[a.col];
     a.w4 = k.width[a.col] == 4;
-    // narrow: leaf and a + b*leaf provably fit int32 given the column's exact min/max (cf. inferBounds, Vlite.hs:417-467)
+    // narrow: leaf and a + b*leaf provably fit int32 given the column's exact min/max (cf. inferBounds, Vlite.hs:417-467).
+    // The narrow device code (affine32) shifts the LOW WORD of an 8-byte value, so the raw values must fit int32 as well:
+    // (x >> shr) fitting is not enough when x itself does not.
     i64 cmin, cmax;
     int rc2 = vdl_column_analyze(ctx, desc->column[a.col], &cmin, &cmax);
     if (rc2) { place_rc = rc2; return; }
     __int128 l0 = cmin >> a.shr, l1 = cmax >> a.shr;
     __int128 v0 = (__int128)a.a + (__int128)a.b * l0, v1 = (__int128)a.a + (__int128)a.b * l1;
     auto fits = [](__int128 x) { return x >= INT32_MIN && x <= INT32_MAX; };
-    a.narrow = cmin <= cmax && fits(l0) && fits(l1) && fits(v0) && fits(v1) && fits(a.a) && fits(a.b);
+    a.narrow = cmin <= cmax && fits(cmin) && fits(cmax) && fits(l0) && fits(l1) && fits(v0) && fits(v1) && fits(a.a) && fits(a.b);
     bound[&a] = Bound{std::min(v0, v1), std::max(v0, v1)};
   };
   auto derive = [&]() -> int {
@@ -430,11 +432,11 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
       KPred &p = k.pred[i];
       p.soff = k.soff[p.col];
       p.w4 = k.width[p.col] == 4;
-      if (!p.w4) {   // 8-byte column: when the column statistics say every (shifted) value fits int32, read low words only
-        i64 cmin, cmax;
+      if (!p.w4) {   // 8-byte column: when the column statistics say every raw value fits int32, read low words only
+        i64 cmin, cmax;  // (the device shifts the low word: a raw value beyond int32 whose shifted value fits still needs all 8 bytes)
         int rc2 = vdl_column_analyze(ctx, desc->column[p.col], &cmin, &cmax);
         if (rc2) return rc2;
-        if ((cmin >> p.shr) >= INT32_MIN && (cmax >> p.shr) <= INT32_MAX) p.w4 = 2;
+        if (cmin >= INT32_MIN && cmax <= INT32_MAX) p.w4 = 2;
       }
       if (p.w4) {   // values of a 4-byte column (shifted or not) lie in int32: clamp the bounds, compare in 32 bits
         i64 lo = std::max<i64>(p.lo, INT32_MIN), hi = std::min<i64>((i64)((u64)p.lo + p.span), INT32_MAX);
