@@ -182,6 +182,13 @@ int vdl_op_partition(vdl_ctx *ctx, vdl_vec data, int64_t pivot_from, int64_t piv
                      int64_t pivot_count, vdl_vec *out);
 /* FoldSum/Min/Max/Choose/Count (Vdl.hs:255-264): one output per run of equal consecutive groups. */
 int vdl_op_fold(vdl_ctx *ctx, int fold_op, vdl_vec groups, vdl_vec data, vdl_vec *out);
+/* ORDER BY / LIMIT, which the emitter cannot express: positions 0..n-1 of the nkeys key vectors (equal length n) ordered
+ * lexicographically over the keys compared as signed int64 (int32 sign-extended, ranges read as their values), key i
+ * descending when descending[i] != 0 (descending may be NULL: all ascending); ties keep row order (stable).  out has
+ * min(limit, n) entries (limit < 0: n); gathering any vector of length n by it gives its rows in that order.  nkeys = 0:
+ * positions 0..limit-1 (limit >= 0; the caller knows n).  Keys of unequal length: VDL_EINVAL. */
+#define VDL_MAX_ORDER_KEYS 8
+int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const int *descending, int64_t limit, vdl_vec *out);
 
 /* ---- fused select -> map -> fold -------------------------------------------------------
  * One launch that scans up to VDL_MAX_COLS columns of one table, applies a conjunction of range
@@ -429,6 +436,13 @@ int vdl_plan_output(vdl_plan *p, int i, const char **name, const int64_t **data,
  * vdl_plan_output_typed returns dtype 4 (int32 data) or 8 (int64); vdl_plan_output fails for a column delivered as int32. */
 int vdl_plan_set_typed_outputs(vdl_plan *p, int on);
 int vdl_plan_output_typed(vdl_plan *p, int i, const char **name, const void **data, int64_t *len, int *dtype);
+/* ORDER BY key_output[0..nkeys) (output indices, descending[i] = 1: DESC) LIMIT limit, applied to every later
+ * vdl_plan_run / vdl_plan_finish before the results are copied to the host (vdl_op_order's order: ties keep the plan's own
+ * row order; nkeys = 0 with limit >= 0: the first `limit` rows).  nkeys = 0 and limit < 0: off (the default).  The outputs
+ * must then all have one length (vdl_plan_finish fails with VDL_EINVAL naming two that differ); vdl_plan_output reports the
+ * limited length.  Excludes the sharded tail (a rank holds only a slice of the result): with vdl_plan_tail_enable(p, 1)
+ * in force this fails with VDL_EUNSUPPORTED, and so does that call while an order is set. */
+int vdl_plan_set_order(vdl_plan *p, int nkeys, const int *key_output, const int *descending, int64_t limit);
 int vdl_plan_destroy(vdl_plan *p);
 
 /* ---- several GPUs of one box driven from ONE process (SURVEY.md section 8 b, e) ----------------------------------------

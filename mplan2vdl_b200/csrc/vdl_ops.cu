@@ -902,6 +902,285 @@ extern "C" int vdl_op_partition(vdl_ctx *ctx, vdl_vec data, int64_t pfrom, int64
   return VDL_OK;
 }
 
+// ---------------------------------------------------------------------------------- Order (ORDER BY / LIMIT)
+// Every key becomes its distance from its minimum (ascending) or from its maximum (descending) in uint64 -- exact at
+// INT64_MIN / INT64_MAX, where -x is not -- and the distances are bit-packed: the last key in the least significant bits,
+// each key in the bits its range needs, a constant key in none.  Keys that do not fit one 64-bit word spill into further
+// words (word 0 least significant).  A full order is Partition's stable LSD radix sort (radix_hist_kernel,
+// device_exclusive_scan, radix_scatter_kernel), least significant word first, over the bits that are set.  With a LIMIT a
+// radix select comes first: the pack kernel also counts the top 8-bit digit, the host finds the digit at which the count
+// reaches the limit, the rows at or below it are compacted in row order by FoldSelect (so ties stay stable) -- refined digit
+// by digit while there are many more of them than the limit -- and only those candidates are sorted.
+struct OrderArgs {
+  Operand key[VDL_MAX_ORDER_KEYS];
+  u64 base[VDL_MAX_ORDER_KEYS];     // minimum (ascending) or maximum (descending)
+  int desc[VDL_MAX_ORDER_KEYS];
+  int word[VDL_MAX_ORDER_KEYS];     // packed word of the key; -1: constant key (or no key)
+  int shift[VDL_MAX_ORDER_KEYS];    // its lowest bit in that word
+  int nkeys, nwords, top_shift;     // top_shift: lowest bit of the most significant word's top digit
+};
+
+__global__ void __launch_bounds__(256) order_minmax_kernel(const __grid_constant__ OrderArgs a, i64 n, i64 *mm /* [min, max] per key */) {
+  const i64 stride = (i64)gridDim.x * blockDim.x;
+  for (int k = 0; k < a.nkeys; k++) {
+    i64 lo = INT64_MAX, hi = INT64_MIN;
+    for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+      const i64 v = op_ld(a.key[k], i);
+      lo = v < lo ? v : lo;
+      hi = v > hi ? v : hi;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const i64 x = __shfl_xor_sync(0xffffffffu, lo, o), y = __shfl_xor_sync(0xffffffffu, hi, o);
+      lo = x < lo ? x : lo;
+      hi = y > hi ? y : hi;
+    }
+    if ((threadIdx.x & 31) == 0) {
+      atomicMin((long long *)&mm[2 * k], (long long)lo);
+      atomicMax((long long *)&mm[2 * k + 1], (long long)hi);
+    }
+  }
+}
+
+// words[w * n + i] = packed word w of row i; HIST: hist[d] += rows whose most significant word has top digit d (shared
+// counters, one global atomic per digit and block)
+template <bool HIST>
+__global__ void __launch_bounds__(256) order_pack_kernel(const __grid_constant__ OrderArgs a, i64 n, u64 *__restrict__ words,
+                                                         unsigned long long *__restrict__ hist) {
+  __shared__ unsigned h[256];
+  if (HIST) {
+    h[threadIdx.x] = 0;
+    __syncthreads();
+  }
+  const i64 stride = (i64)gridDim.x * blockDim.x;
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    u64 v[VDL_MAX_ORDER_KEYS];
+#pragma unroll
+    for (int k = 0; k < VDL_MAX_ORDER_KEYS; k++) {
+      v[k] = 0;
+      if (a.word[k] >= 0) {
+        const u64 x = (u64)op_ld(a.key[k], i);
+        v[k] = (a.desc[k] ? a.base[k] - x : x - a.base[k]) << a.shift[k];
+      }
+    }
+#pragma unroll
+    for (int w = 0; w < VDL_MAX_ORDER_KEYS; w++) {
+      if (w >= a.nwords) break;
+      u64 acc = 0;
+#pragma unroll
+      for (int k = 0; k < VDL_MAX_ORDER_KEYS; k++) acc |= a.word[k] == w ? v[k] : 0;
+      words[(i64)w * n + i] = acc;
+      if (HIST && w == a.nwords - 1) atomicAdd(&h[(acc >> a.top_shift) & 255], 1u);
+    }
+  }
+  if (HIST) {
+    __syncthreads();
+    if (h[threadIdx.x]) atomicAdd(&hist[threadIdx.x], (unsigned long long)h[threadIdx.x]);
+  }
+}
+
+// the next digit, bits [s_new, s_old), of the rows whose bits from s_old up equal `prefix`
+__global__ void __launch_bounds__(256) order_refine_hist_kernel(const u64 *__restrict__ top, i64 n, int s_old, u64 prefix, int s_new,
+                                                                unsigned long long *__restrict__ hist) {
+  __shared__ unsigned h[256];
+  h[threadIdx.x] = 0;
+  __syncthreads();
+  const u64 mask = (1ull << (s_old - s_new)) - 1;
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+    const u64 x = top[i];
+    if ((x >> s_old) == prefix) atomicAdd(&h[(x >> s_new) & mask], 1u);
+  }
+  __syncthreads();
+  if (h[threadIdx.x]) atomicAdd(&hist[threadIdx.x], (unsigned long long)h[threadIdx.x]);
+}
+
+__global__ void __launch_bounds__(256) order_candidate_kernel(const u64 *__restrict__ top, i64 n, int s, u64 prefix, int *__restrict__ flag) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) flag[i] = (top[i] >> s) <= prefix;
+}
+
+__global__ void __launch_bounds__(256) order_gather_kernel(const u64 *__restrict__ src, const i64 *__restrict__ pos, i64 n, u64 *__restrict__ dst) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) dst[i] = src[pos[i]];
+}
+
+__global__ void __launch_bounds__(256) order_iota_kernel(i64 *__restrict__ out, i64 n) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) out[i] = i;
+}
+
+namespace {
+struct VecScope {      // temporaries of one op, released (stream-ordered) when it returns
+  vdl_ctx *ctx;
+  std::vector<vdl_vec> v;
+  ~VecScope() { for (vdl_vec h : v) vdl_vec_free(ctx, h); }
+};
+}  // namespace
+
+// Stable LSD sort of positions 0..n-1 by packed words (word w of position i at words[w * n + i], w = 0 least significant,
+// wbits[w] bits used): *out = the positions in order, a new vector of length n.
+static int order_lsd(vdl_ctx *ctx, const u64 *words, int nwords, const int *wbits, i64 n, vdl_vec *out) {
+  const i64 nb = (n + RDX_TILE - 1) / RDX_TILE;
+  vdl_vec tk[2], ti[2];
+  VecScope tmp{ctx, {}};
+  for (int k = 0; k < 2; k++) {
+    VDL_TRY(vec_new(ctx, VDL_I64, n, &tk[k])); tmp.v.push_back(tk[k]);
+    VDL_TRY(vec_new(ctx, VDL_I64, n, &ti[k])); tmp.v.push_back(ti[k]);
+  }
+  int cur = 0;
+  VDL_TRY(scratch_reserve(ctx, scan_elems(256 * nb) * 8));
+  i64 *hist = (i64 *)ctx->scratch;
+  u64 *key[2] = {(u64 *)ctx->vecs[tk[0]].ptr, (u64 *)ctx->vecs[tk[1]].ptr};
+  i64 *idx[2] = {(i64 *)ctx->vecs[ti[0]].ptr, (i64 *)ctx->vecs[ti[1]].ptr};
+  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
+  order_iota_kernel<<<grid, 256, 0, ctx->stream>>>(idx[0], n);
+  ctx->launches++;
+  for (int w = 0; w < nwords; w++) {
+    const u64 *kin = words + (i64)w * n;
+    if (w > 0) {          // the next more significant word, in the order reached so far
+      order_gather_kernel<<<grid, 256, 0, ctx->stream>>>(kin, idx[cur], n, key[cur]);
+      ctx->launches++;
+      kin = key[cur];
+    }
+    for (int shift = 0; shift < wbits[w]; shift += 8) {
+      radix_hist_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, n, shift, nb, hist);
+      device_exclusive_scan(ctx, hist, 256 * nb);
+      radix_scatter_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, idx[cur], n, shift, nb, hist, key[cur ^ 1], idx[cur ^ 1]);
+      ctx->launches += 2;
+      cur ^= 1;
+      kin = key[cur];
+    }
+  }
+  VDL_CUDA(ctx, cudaGetLastError());
+  tmp.v.erase(std::find(tmp.v.begin(), tmp.v.end(), ti[cur]));
+  *out = ti[cur];
+  return VDL_OK;
+}
+
+extern "C" int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const int *descending, int64_t limit, vdl_vec *out) {
+  if (!ctx || !out || (nkeys > 0 && !keys)) return VDL_EINVAL;
+  if (nkeys < 0 || nkeys > VDL_MAX_ORDER_KEYS) return vdl_fail(ctx, VDL_EINVAL, "Order: %d keys (at most %d)", nkeys, VDL_MAX_ORDER_KEYS);
+  if (nkeys == 0) {
+    if (limit < 0) return vdl_fail(ctx, VDL_EINVAL, "Order: neither keys nor a limit");
+    return vec_new_range(ctx, 0, 1, limit, out);
+  }
+  OrderArgs a;
+  memset(&a, 0, sizeof a);
+  i64 n = -1;
+  for (int k = 0; k < VDL_MAX_ORDER_KEYS; k++) a.word[k] = -1;
+  for (int k = 0; k < nkeys; k++) {
+    Vec *v = vec_get(ctx, keys[k]);
+    if (!v) return VDL_EINVAL;
+    if (n >= 0 && v->len != n) return vdl_fail(ctx, VDL_EINVAL, "Order: key %d has %lld rows, key 0 has %lld", k, (long long)v->len, (long long)n);
+    n = v->len;
+    a.key[k] = operand_of(*v);
+    a.desc[k] = descending && descending[k] ? 1 : 0;
+  }
+  a.nkeys = nkeys;
+  const i64 m = limit < 0 || limit > n ? n : limit;
+  if (m == 0) {
+    VDL_TRY(vec_new(ctx, VDL_I64, 0, out));
+    ctx->vecs[*out].domain = n;
+    return VDL_OK;
+  }
+  VDL_CUDA(ctx, cudaSetDevice(ctx->device));
+  VecScope tmp{ctx, {}};
+  // minimum and maximum of every key in one pass ([min, max] per key, then the 256 top-digit counters of the select)
+  vdl_vec mmv;
+  VDL_TRY(vec_new(ctx, VDL_I64, 2 * VDL_MAX_ORDER_KEYS + 256, &mmv));
+  tmp.v.push_back(mmv);
+  i64 *mm = (i64 *)ctx->vecs[mmv].ptr;
+  unsigned long long *hist = (unsigned long long *)(mm + 2 * VDL_MAX_ORDER_KEYS);
+  i64 hmm[2 * VDL_MAX_ORDER_KEYS];
+  for (int k = 0; k < VDL_MAX_ORDER_KEYS; k++) { hmm[2 * k] = INT64_MAX; hmm[2 * k + 1] = INT64_MIN; }
+  VDL_CUDA(ctx, cudaMemcpyAsync(mm, hmm, sizeof hmm, cudaMemcpyHostToDevice, ctx->stream));
+  VDL_CUDA(ctx, cudaMemsetAsync(hist, 0, 256 * sizeof(unsigned long long), ctx->stream));
+  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 8));
+  order_minmax_kernel<<<grid, 256, 0, ctx->stream>>>(a, n, mm);
+  ctx->launches++;
+  VDL_TRY(read_scalar(ctx, mm, hmm, 64));
+  if (nkeys > 4) VDL_TRY(read_scalar(ctx, mm + 8, hmm + 8, 64));
+  // packing, least significant key first: a key takes bits(max - min) bits, a word holds what fits in 64
+  int wbits[VDL_MAX_ORDER_KEYS] = {0}, nwords = 0;
+  for (int k = nkeys - 1; k >= 0; k--) {
+    const u64 span = (u64)hmm[2 * k + 1] - (u64)hmm[2 * k];
+    const int width = span ? 64 - __builtin_clzll(span) : 0;
+    a.base[k] = (u64)hmm[2 * k + a.desc[k]];
+    if (!width) continue;
+    if (nwords == 0 || wbits[nwords - 1] + width > 64) nwords++;
+    a.word[k] = nwords - 1;
+    a.shift[k] = wbits[nwords - 1];
+    wbits[nwords - 1] += width;
+  }
+  a.nwords = nwords;
+  if (nwords == 0) {       // every key constant: row order
+    VDL_TRY(vec_new_range(ctx, 0, 1, m, out));
+    ctx->vecs[*out].domain = n;
+    return VDL_OK;
+  }
+  const int W = nwords - 1;
+  a.top_shift = wbits[W] > 8 ? wbits[W] - 8 : 0;
+  const bool select = m < n;
+  vdl_vec wv;
+  VDL_TRY(vec_new(ctx, VDL_I64, (i64)nwords * n, &wv));
+  tmp.v.push_back(wv);
+  u64 *words = (u64 *)ctx->vecs[wv].ptr;
+  const int pgrid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
+  if (select) order_pack_kernel<true><<<pgrid, 256, 0, ctx->stream>>>(a, n, words, hist);
+  else order_pack_kernel<false><<<pgrid, 256, 0, ctx->stream>>>(a, n, words, hist);
+  ctx->launches++;
+  VDL_CUDA(ctx, cudaGetLastError());
+  if (!select) {
+    VDL_TRY(order_lsd(ctx, words, nwords, wbits, n, out));
+    ctx->vecs[*out].domain = n;
+    ctx->vecs[*out].is_perm = true;
+    return VDL_OK;
+  }
+  // radix select on the most significant word: `prefix` (its bits from s up) such that the first m rows in order are among
+  // the rows whose bits from s up are <= prefix
+  const u64 *top = words + (i64)W * n;
+  int s_hi = wbits[W], s = a.top_shift;
+  u64 hi = 0, prefix = 0;
+  i64 cands = 0;
+  i64 below = 0;                                   // rows whose bits from s_hi up are < hi: all of them come first
+  const i64 enough = std::max<i64>(2 * m, 4096);
+  unsigned long long hh[256];
+  for (;;) {
+    VDL_CUDA(ctx, cudaMemcpyAsync(hh, hist, sizeof hh, cudaMemcpyDeviceToHost, ctx->stream));
+    VDL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    int t = 0;
+    i64 run = below;
+    while (t < 255 && run + (i64)hh[t] < m) run += (i64)hh[t++];
+    prefix = (hi << (s_hi - s)) | (u64)t;
+    below = run;
+    cands = run + (i64)hh[t];
+    if (cands <= enough || s == 0) break;
+    hi = prefix;
+    s_hi = s;
+    s = s > 8 ? s - 8 : 0;
+    VDL_CUDA(ctx, cudaMemsetAsync(hist, 0, 256 * sizeof(unsigned long long), ctx->stream));
+    order_refine_hist_kernel<<<pgrid, 256, 0, ctx->stream>>>(top, n, s_hi, hi, s, hist);
+    ctx->launches++;
+  }
+  vdl_vec fv, cand, cw, sorted;
+  VDL_TRY(vec_new(ctx, VDL_I32, n, &fv));
+  tmp.v.push_back(fv);
+  order_candidate_kernel<<<pgrid, 256, 0, ctx->stream>>>(top, n, s, prefix, (int *)ctx->vecs[fv].ptr);
+  ctx->launches++;
+  VDL_TRY(vdl_op_fold_select(ctx, fv, &cand));      // candidate positions in row order
+  tmp.v.push_back(cand);
+  const i64 c = ctx->vecs[cand].len;
+  if (c != cands) return vdl_fail(ctx, VDL_ECUDA, "Order: %lld candidates compacted, %lld counted", (long long)c, (long long)cands);
+  VDL_TRY(vec_new(ctx, VDL_I64, (i64)nwords * c, &cw));
+  tmp.v.push_back(cw);
+  u64 *cwords = (u64 *)ctx->vecs[cw].ptr;
+  const i64 *cpos = (const i64 *)ctx->vecs[cand].ptr;
+  const int cgrid = (int)std::max<i64>(1, std::min<i64>((c + 255) / 256, (i64)ctx->sm_count * 16));
+  for (int w = 0; w < nwords; w++) order_gather_kernel<<<cgrid, 256, 0, ctx->stream>>>(words + (i64)w * n, cpos, c, cwords + (i64)w * c);
+  ctx->launches += nwords;
+  VDL_TRY(order_lsd(ctx, cwords, nwords, wbits, c, &sorted));
+  tmp.v.push_back(sorted);
+  ctx->vecs[sorted].len = m;                        // the first m candidates in order, mapped back to row positions
+  return vdl_op_gather(ctx, cand, sorted, out);
+}
+
 // ---------------------------------------------------------------------------------- Fold by runs
 #include "vdl_fold_kernel.cuh"
 

@@ -119,6 +119,9 @@ struct vdl_plan {
   bool tail_ok = false, tail_on = false;
   int tail_groups = -1, tail_partition = -1;     // groups node; its Partition (-1: constant groups)
   i64 tail_rec[4] = {0, 0, 0, 0};                // of the last run: sorted, runs, first key, last key
+  // ORDER BY / LIMIT (vdl_plan_set_order): output indices of the keys, their DESC flags; limit < 0: none
+  std::vector<int> order_key, order_desc;
+  i64 order_limit = -1;
   // run state
   std::vector<vdl_vec> val;
   std::vector<vdl_vec> temps;
@@ -1375,6 +1378,16 @@ int capture_tail_boundary(vdl_plan *p) {
   return VDL_OK;
 }
 
+// the output's own pinned host buffer, grown to hold len values (pinned, so a copy into it is one DMA at PCIe rate)
+int reserve_pinned(vdl_ctx *ctx, Output &o, i64 len) {
+  if (o.pinned) cudaFreeHost(o.pinned);
+  o.pinned = nullptr; o.cap = 0;
+  size_t want = (size_t)len + (size_t)len / 4 + 16;
+  if (cudaHostAlloc(&o.pinned, want * sizeof(i64), cudaHostAllocDefault) != cudaSuccess) return vdl_fail(ctx, VDL_ENOMEM, "output buffer of %lld values", (long long)len);
+  o.cap = want;
+  return VDL_OK;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------- ABI
@@ -1700,7 +1713,44 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
       VDL_TRY(vdl_probe_finalize(p->pgroups[gi]->probe, all_partials ? all_partials[p->groups.size() + gi] : nullptr, nranks));
   }
   bool ran_ops = false, copies_pending = false;
-  for (auto &o : p->outputs) {
+  const bool ordered = !p->order_key.empty() || p->order_limit >= 0;
+  std::vector<vdl_vec> dev(p->outputs.size(), 0);    // ordered: the device value of every op-at-a-time output
+  // the device -> host copy of op-at-a-time output o, whose value is v
+  auto deliver = [&](Output &o, vdl_vec v) -> int {
+    i64 len;
+    VDL_TRY(vdl_vec_len(ctx, v, &len));
+    if ((size_t)len > o.cap) {              // pinned, so the copy is one DMA at PCIe rate
+      int rc = reserve_pinned(ctx, o, len);
+      if (rc) { free_temps(p); return rc; }
+    }
+    Vec *vv = vec_get(ctx, v);
+    o.dtype = 8;
+    if (p->typed_outputs && vv && !vv->is_range && vv->dtype == VDL_I64 && vv->narrow32 && len > 0) {
+      // every value is a value of a 4-byte column: half the bytes over PCIe (a narrowing kernel, then the same async copy)
+      vdl_vec nv;
+      int rc = vec_narrow_copy(ctx, v, &nv);
+      if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
+      p->temps.push_back(nv);
+      VDL_CUDA(ctx, cudaEventRecord(ctx->copy_event, ctx->stream));
+      VDL_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_event, 0));
+      VDL_CUDA(ctx, cudaMemcpyAsync(o.pinned, vec_get(ctx, nv)->ptr, (size_t)len * 4, cudaMemcpyDeviceToHost, ctx->copy_stream));
+      copies_pending = true;
+      o.dtype = 4;
+    } else if (vv && !vv->is_range && vv->dtype == VDL_I64 && len > 0) {
+      // the copy runs on its own stream behind an event, so the next output's kernels overlap it; one wait at the end
+      VDL_CUDA(ctx, cudaEventRecord(ctx->copy_event, ctx->stream));
+      VDL_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_event, 0));
+      VDL_CUDA(ctx, cudaMemcpyAsync(o.pinned, vv->ptr, (size_t)len * 8, cudaMemcpyDeviceToHost, ctx->copy_stream));
+      copies_pending = true;
+    } else {
+      int rc = vdl_vec_download(ctx, v, o.pinned, len);
+      if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
+    }
+    o.data = o.pinned; o.len = len;
+    return VDL_OK;
+  };
+  for (size_t oi = 0; oi < p->outputs.size(); oi++) {
+    Output &o = p->outputs[oi];
     int gi = p->group_of_node[o.node];
     if (p->pgroup_of_node[o.node] >= 0) {   // a Fold over a joined space: the probe's result buffer is already on its way
       ProbeFoldGroup &g = *p->pgroups[p->pgroup_of_node[o.node]];
@@ -1721,39 +1771,67 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
     vdl_vec v;
     int rc = eval(p, o.node, &v);
     if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
-    i64 len;
-    VDL_TRY(vdl_vec_len(ctx, v, &len));
-    if ((size_t)len > o.cap) {              // pinned, so the copy is one DMA at PCIe rate
-      if (o.pinned) cudaFreeHost(o.pinned);
-      o.pinned = nullptr; o.cap = 0;
-      size_t want = (size_t)len + (size_t)len / 4 + 16;
-      if (cudaHostAlloc(&o.pinned, want * sizeof(i64), cudaHostAllocDefault) != cudaSuccess) { free_temps(p); return vdl_fail(ctx, VDL_ENOMEM, "output buffer of %lld values", (long long)len); }
-      o.cap = want;
+    if (ordered) { dev[oi] = v; continue; }
+    VDL_TRY(deliver(o, v));
+  }
+  if (ordered) {
+    // ORDER BY / LIMIT: one permutation of the rows, computed over the key outputs, applied to every output before its copy
+    int rc = VDL_OK;
+    const size_t no = p->outputs.size();
+    std::vector<i64> len(no, 0);
+    for (size_t i = 0; i < no && !rc; i++) {
+      if (dev[i]) rc = vdl_vec_len(ctx, dev[i], &len[i]);
+      else len[i] = p->outputs[i].len;
+      if (!rc && len[i] != len[0])
+        rc = vdl_fail(ctx, VDL_EINVAL, "ORDER BY / LIMIT needs outputs of one length: %s has %lld rows, %s has %lld", p->outputs[0].name.c_str(),
+                      (long long)len[0], p->outputs[i].name.c_str(), (long long)len[i]);
     }
-    Vec *vv = vec_get(ctx, v);
-    o.dtype = 8;
-    if (p->typed_outputs && vv && !vv->is_range && vv->dtype == VDL_I64 && vv->narrow32 && len > 0) {
-      // every value is a value of a 4-byte column: half the bytes over PCIe (a narrowing kernel, then the same async copy)
-      vdl_vec nv;
-      rc = vec_narrow_copy(ctx, v, &nv);
-      if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
-      p->temps.push_back(nv);
-      VDL_CUDA(ctx, cudaEventRecord(ctx->copy_event, ctx->stream));
-      VDL_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_event, 0));
-      VDL_CUDA(ctx, cudaMemcpyAsync(o.pinned, vec_get(ctx, nv)->ptr, (size_t)len * 4, cudaMemcpyDeviceToHost, ctx->copy_stream));
-      copies_pending = true;
-      o.dtype = 4;
-    } else if (vv && !vv->is_range && vv->dtype == VDL_I64 && len > 0) {
-      // the copy runs on its own stream behind an event, so the next output's kernels overlap it; one wait at the end
-      VDL_CUDA(ctx, cudaEventRecord(ctx->copy_event, ctx->stream));
-      VDL_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_event, 0));
-      VDL_CUDA(ctx, cudaMemcpyAsync(o.pinned, vv->ptr, (size_t)len * 8, cudaMemcpyDeviceToHost, ctx->copy_stream));
-      copies_pending = true;
-    } else {
-      rc = vdl_vec_download(ctx, v, o.pinned, len);
-      if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
+    const i64 n = no ? len[0] : 0;
+    std::vector<vdl_vec> keys(p->order_key.size(), 0);
+    for (size_t k = 0; k < keys.size() && !rc; k++) {
+      const int i = p->order_key[k];
+      if (dev[i]) { keys[k] = dev[i]; continue; }
+      // a host-resident result (fused scan, probe fold): its key values go back to the device for the order; the result
+      // buffer itself is shared by the scan's / probe's outputs and stays as it is
+      rc = vec_new(ctx, VDL_I64, n, &keys[k]);
+      if (rc) break;
+      p->temps.push_back(keys[k]);
+      if (n > 0) {
+        const cudaError_t e = cudaMemcpyAsync(ctx->vecs[keys[k]].ptr, p->outputs[i].data, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) rc = vdl_cuda_fail(ctx, e, "ORDER BY key upload");
+      }
     }
-    o.data = o.pinned; o.len = len;
+    vdl_vec perm = 0;
+    if (!rc) {
+      const i64 limit = keys.empty() ? std::min<i64>(p->order_limit, n) : p->order_limit;
+      rc = vdl_op_order(ctx, (int)keys.size(), keys.data(), p->order_desc.data(), limit, &perm);
+      if (!rc) p->temps.push_back(perm);
+    }
+    i64 m = 0;
+    if (!rc) rc = vdl_vec_len(ctx, perm, &m);
+    std::vector<i64> hperm;                 // the permutation on the host, for host-resident results
+    for (size_t i = 0; i < no && !rc; i++) {
+      Output &o = p->outputs[i];
+      if (dev[i]) {
+        vdl_vec g;
+        rc = vdl_op_gather(ctx, dev[i], perm, &g);     // (keeps narrow32: typed outputs still travel as int32)
+        if (rc) break;
+        p->temps.push_back(g);
+        rc = deliver(o, g);
+        if (rc) return rc;
+        continue;
+      }
+      if (keys.empty()) { o.len = m; continue; }          // LIMIT alone: the first m rows, in place
+      if (hperm.empty() && m > 0) {
+        hperm.resize((size_t)m);
+        rc = vdl_vec_download(ctx, perm, hperm.data(), m);
+        if (rc) break;
+      }
+      if ((size_t)m > o.cap && (rc = reserve_pinned(ctx, o, m))) break;
+      for (i64 j = 0; j < m; j++) o.pinned[j] = o.data[hperm[j]];
+      o.data = o.pinned; o.len = m; o.dtype = 8;
+    }
+    if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
   }
   if (copies_pending) VDL_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));     // before the temporaries are released
   int rc = ran_ops ? check_errflag(ctx, "plan") : VDL_OK;
@@ -1775,7 +1853,23 @@ extern "C" int vdl_plan_tail_info(vdl_plan *p, int *mergeable, int *fold_ops, in
 extern "C" int vdl_plan_tail_enable(vdl_plan *p, int on) {
   if (!p) return VDL_EINVAL;
   if (on && !p->tail_ok) return vdl_fail(p->ctx, VDL_EUNSUPPORTED, "the plan's outputs are not Folds by runs of one groups vector");
+  if (on && (!p->order_key.empty() || p->order_limit >= 0))
+    return vdl_fail(p->ctx, VDL_EUNSUPPORTED, "the sharded tail leaves each rank a slice of the result, which an ORDER BY / LIMIT cannot be applied to");
   p->tail_on = on != 0;
+  return VDL_OK;
+}
+extern "C" int vdl_plan_set_order(vdl_plan *p, int nkeys, const int *key_output, const int *descending, int64_t limit) {
+  if (!p || nkeys < 0 || (nkeys > 0 && !key_output)) return VDL_EINVAL;
+  if (nkeys > VDL_MAX_ORDER_KEYS) return vdl_fail(p->ctx, VDL_EINVAL, "ORDER BY: %d keys (at most %d)", nkeys, VDL_MAX_ORDER_KEYS);
+  for (int k = 0; k < nkeys; k++)
+    if (key_output[k] < 0 || key_output[k] >= (int)p->outputs.size())
+      return vdl_fail(p->ctx, VDL_EINVAL, "ORDER BY key %d: output %d out of range (the plan has %d outputs)", k, key_output[k], (int)p->outputs.size());
+  if ((nkeys > 0 || limit >= 0) && p->tail_on)
+    return vdl_fail(p->ctx, VDL_EUNSUPPORTED, "the sharded tail leaves each rank a slice of the result, which an ORDER BY / LIMIT cannot be applied to");
+  p->order_key.assign(key_output, key_output + nkeys);
+  p->order_desc.assign(nkeys, 0);
+  for (int k = 0; k < nkeys && descending; k++) p->order_desc[k] = descending[k] ? 1 : 0;
+  p->order_limit = limit < 0 ? -1 : limit;
   return VDL_OK;
 }
 extern "C" int vdl_plan_tail_boundary(vdl_plan *p, int64_t *rec, int cap) {

@@ -170,6 +170,14 @@ class Context:
     def op_fold(self, op: str, groups: int, data: int) -> int:
         return self._out(self.L.vdl_op_fold, _lib.FOLD_OPS.index(op), groups, data)
 
+    def op_order(self, keys, descending=None, limit: int | None = None) -> int:
+        """Positions that order the rows of the key vectors (vdl_op_order): lexicographic over `keys`, signed int64, key i
+        descending when descending[i]; ties keep row order; the first `limit` of them (None: all)."""
+        k = len(keys)
+        ks = (C.c_int32 * max(1, k))(*keys)
+        ds = (C.c_int * max(1, k))(*[int(bool(d)) for d in (descending or [0] * k)])
+        return self._out(self.L.vdl_op_order, k, ks, ds, -1 if limit is None else limit)
+
     # ---- peer-addressable buffers (multi-GPU combine without a collective library) ------------
     def ipc_alloc(self, nbytes: int) -> int:
         p = C.c_void_p()
@@ -206,6 +214,24 @@ class Context:
 
     def plan(self, text: str, fuse: bool = True) -> "Plan":
         return Plan(self, text, fuse)
+
+
+def order_keys(names, keys) -> tuple:
+    """(output indices, descending flags) of ORDER BY `keys` over outputs `names`.  A key is a name or (name, descending); a
+    name is a full output name or its alias, the part before the first '__' (``o_orderdate`` for
+    ``o_orderdate__orders__o_orderdate``).  Raises KeyError for a name that matches no output or more than one."""
+    idx, desc = [], []
+    for key in keys:
+        name, d = (key, False) if isinstance(key, str) else (key[0], bool(key[1]))
+        hits = [i for i, n in enumerate(names) if n == name]
+        if not hits:
+            hits = [i for i, n in enumerate(names) if n.split("__", 1)[0] == name]
+        if len(hits) != 1:
+            raise KeyError(f"ORDER BY {name!r}: {'no output' if not hits else 'more than one output'} of "
+                           f"{list(names)} has that name or alias")
+        idx.append(hits[0])
+        desc.append(d)
+    return idx, desc
 
 
 def explain(text: str, fuse: bool = True) -> dict:
@@ -378,6 +404,27 @@ class Plan:
         """Result columns whose values provably fit travel as int32 (vdl_plan_set_typed_outputs); outputs() then returns
         int32 arrays for them."""
         self.ctx.check(self.L.vdl_plan_set_typed_outputs(self.h, int(on)))
+
+    def output_names(self) -> list:
+        """The output names in MaterializeCompact order (known from loading: no run needed)."""
+        names = []
+        for i in range(self.L.vdl_plan_num_outputs(self.h)):
+            name = C.c_char_p()
+            self.ctx.check(self.L.vdl_plan_output_typed(self.h, i, C.byref(name), None, None, None))
+            names.append(name.value.decode())
+        return names
+
+    def set_order(self, keys, limit: int | None = None):
+        """ORDER BY `keys` LIMIT `limit`, applied on the device to every later run before the results are copied
+        (vdl_plan_set_order).  keys: [name or (name, descending)], names as `order_keys` resolves them; ([], None) turns
+        the order off.  An unknown or ambiguous name raises before anything is set."""
+        idx, desc = order_keys(self.output_names(), keys)
+        self._set_order(idx, desc, -1 if limit is None else limit)
+
+    def _set_order(self, idx, desc, limit: int):
+        k = len(idx)
+        self.ctx.check(self.L.vdl_plan_set_order(self.h, k, (C.c_int * max(1, k))(*idx),
+                                                 (C.c_int * max(1, k))(*[int(d) for d in desc]), limit))
 
     def outputs(self, copy: bool = True) -> dict:
         """{output name: int64 (or, with typed outputs, int32) array}.  copy=False returns views of the library's pinned host

@@ -17,6 +17,7 @@ BINARY_OPS = ["LogicalAnd", "LogicalOr", "BitwiseAnd", "BitwiseOr", "BitShift", 
 FOLD_OPS = ["FoldSum", "FoldMin", "FoldMax", "FoldChoose", "FoldCount"]
 VDL_MAX_COLS, VDL_MAX_PREDS, VDL_MAX_KEYS, VDL_MAX_AGGS, VDL_MAX_FACTORS, VDL_MAX_POSTS = 12, 8, 4, 8, 3, 8
 VDL_POST_FOLD, VDL_POST_POST, VDL_POST_CONST = 0, 1, 2
+VDL_MAX_ORDER_KEYS = 8
 
 
 class VdlError(RuntimeError):
@@ -141,6 +142,7 @@ SYMBOLS = [
     ("vdl_op_scatter", _I, [_P, C.c_int32, C.c_int32, _L, C.POINTER(C.c_int32)]),
     ("vdl_op_partition", _I, [_P, C.c_int32, _L, _L, _L, C.POINTER(C.c_int32)]),
     ("vdl_op_fold", _I, [_P, _I, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
+    ("vdl_op_order", _I, [_P, _I, C.POINTER(C.c_int32), C.POINTER(_I), _L, C.POINTER(C.c_int32)]),
     ("vdl_fused_prepare", _I, [_P, C.POINTER(FusedDesc), C.POINTER(_P)]),
     ("vdl_fused_launch", _I, [_P]),
     ("vdl_fused_partials", _I, [_P, C.POINTER(_P), C.POINTER(_L)]),
@@ -213,6 +215,7 @@ SYMBOLS = [
     ("vdl_plan_output", _I, [_P, _I, C.POINTER(C.c_char_p), C.POINTER(C.POINTER(_L)), C.POINTER(_L)]),
     ("vdl_plan_set_typed_outputs", _I, [_P, _I]),
     ("vdl_plan_output_typed", _I, [_P, _I, C.POINTER(C.c_char_p), C.POINTER(_P), C.POINTER(_L), C.POINTER(_I)]),
+    ("vdl_plan_set_order", _I, [_P, _I, C.POINTER(_I), C.POINTER(_I), _L]),
     ("vdl_plan_destroy", _I, [_P]),
 ]
 

@@ -27,6 +27,12 @@ def plan_columns(text: str) -> list:
     return seen
 
 
+def plan_outputs(text: str) -> list:
+    """Output names of a plan in MaterializeCompact order: the Project each `MaterializeCompact,Id n` names (Vdl.hs:278-292)."""
+    project = dict(re.findall(r"^(\d+),Project,([^,\s]+),", text, re.M))
+    return [project[i] for i in re.findall(r"^\d+,MaterializeCompact,Id (\d+)", text, re.M)]
+
+
 def shard_range(rows: int, rank: int, world: int) -> tuple:
     """(first global row, row count) of `rank`'s contiguous shard of a `rows`-row fact table."""
     per = -(-rows // world)

@@ -113,3 +113,15 @@ def q05(catalog):
 
 
 QUERIES = {"q06": lambda cat: q06(), "q01": lambda cat: q01(), "q03": q03, "q05": q05}
+
+# TPC-H's ORDER BY / LIMIT of the checked-in plans whose sort keys are all numeric outputs, which the fixtures
+# (tpch10noorder) drop and the executor applies on request (Plan.set_order, --tpch-order): plan -> (keys, limit), keys as
+# (output name or alias, descending).  The other plans order by a string-coded output (n_name, l_returnflag, ...): their
+# values are heap offsets or dictionary codes, not a collation order.
+ORDER = {
+    "q03": ([("revenue", True), ("o_orderdate__orders__o_orderdate", False)], 10),
+    "q05": ([("revenue", True)], None),
+    "q10": ([("revenue", True)], 20),
+    "q11": ([("value", True)], None),
+    "q18": ([("o_totalprice__orders__o_totalprice", True), ("o_orderdate__orders__o_orderdate", False)], 100),
+}
