@@ -31,37 +31,17 @@
 
 #include "vdl_fused_kernel.cuh"
 
-__global__ void __launch_bounds__(256, 1) fused_finalize_kernel(const __grid_constant__ FinDesc f) {
-  __shared__ int warp_cnt[8];
-  __shared__ i64 running;
-  finalize_block<256>(f, f.parts, f.nranks, threadIdx.x, warp_cnt, &running);
-}
-
-// A rank with nothing to scan still takes part in the exchange: its (identity) table, then the common finalize.
-__global__ void __launch_bounds__(256, 1) fused_exchange_kernel(const __grid_constant__ KDesc d, const __grid_constant__ FinDesc f, const __grid_constant__ XDesc x) {
-  __shared__ int warp_cnt[8];
-  __shared__ i64 running;
-  const i64 *parts = exchange_block<256>(x, d.table, d.errflag, threadIdx.x);
-  finalize_block<256>(f, parts, x.world, threadIdx.x, warp_cnt, &running);
-}
-
 // ------------------------------------------------------------------------------ host side
 typedef void (*scan_kernel_fn)(const KDesc, const FinDesc, const XDesc);
 struct vdl_fused {
   vdl_ctx *ctx = nullptr;
   KDesc kd;
-  FinDesc fd;
+  FoldCombine cb;                 // the finalize's descriptor, the peer exchange, the results (views: out[])
   vdl_vec table = 0;
   vdl_vec out[VDL_MAX_AGGS] = {0};
   int nout = 0;
-  i64 *d_outbuf = nullptr;       // [nout][domain] fold results, then [ngroups, errflag]: fetched with ONE copy
-  i64 *h_outbuf = nullptr;       // pinned mirror
-  i64 ngroups = -1;
-  bool finalized = false, always_false = false, rs = false;
-  bool table_clean = false;       // the partial table holds the fold identities (init kernel or a finalize that reset it)
+  bool always_false = false, rs = false;
   unsigned int *d_done = nullptr; // ticket counter of the scan kernel's last-CTA epilogue
-  i64 *h_mapped = nullptr;        // device address of h_outbuf (mapped pinned memory)
-  XDesc xd;                       // peer exchange (world == 0: not configured)
   // register slots: kernels by slot count; the launch picks the smallest count that covers the groups the previous
   // run of this scan produced (more slots = more predicated work per row; too few = keys on the slow global path)
   scan_kernel_fn rs_kernel[9] = {nullptr};
@@ -71,10 +51,7 @@ struct vdl_fused {
   int grid = 1, nc = 256, r = 4;
   scan_kernel_fn kernel = nullptr;
   const char *shape = "generic";
-  // event pairs around the dominant kernel of the last VDL_EVENT_RING launches: durations are read AFTER a timed loop
-  cudaEvent_t ev0[VDL_EVENT_RING] = {nullptr}, ev1[VDL_EVENT_RING] = {nullptr};
-  long nlaunch = 0;
-  bool timed = false;
+  KernelTimer timer;
   // run-time specialised kernels (vdl_jit_kernel): the shape-traits class generated from THIS descriptor
   bool jit = false;
   std::string jit_struct, jit_name;     // the generated `struct ShapeJit {...}` text; "jit:<hash>"
@@ -274,8 +251,8 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
   f->ctx = ctx;
   KDesc &k = f->kd;
   memset(&k, 0, sizeof k);
-  memset(&f->fd, 0, sizeof f->fd);
-  memset(&f->xd, 0, sizeof f->xd);
+  FinDesc &fd = f->cb.fd;
+  memset(&fd, 0, sizeof fd);
   k.rows = desc->rows;
   k.row_base = desc->row_base;
   k.key_mask = desc->key_mask;
@@ -317,17 +294,17 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     for (int t = 0; t < s.nfactors; t++) a.fac[t] = to_k(s.factor[t]);
     if (s.op == VDL_FOLD_SUM || s.op == VDL_FOLD_MIN || s.op == VDL_FOLD_MAX) {
       a.op = s.op == VDL_FOLD_SUM ? 0 : (s.op == VDL_FOLD_MIN ? 1 : 2);
-      f->fd.out_kind[i] = 0;
-      f->fd.out_idx[i] = k.nacc;
+      fd.out_kind[i] = 0;
+      fd.out_idx[i] = k.nacc;
       k.acc[k.nacc++] = a;
     } else if (s.op == VDL_FOLD_CHOOSE) {
       if (k.nchoose == K_MAX_CHOOSE) { delete f; return vdl_fail(ctx, VDL_EUNSUPPORTED, "fused scan: more than %d FoldChoose", K_MAX_CHOOSE); }
-      f->fd.out_kind[i] = 1;
-      f->fd.out_idx[i] = k.nchoose;
+      fd.out_kind[i] = 1;
+      fd.out_idx[i] = k.nchoose;
       k.choose[k.nchoose++] = a;
     } else if (s.op == VDL_FOLD_COUNT) {
-      f->fd.out_kind[i] = 0;
-      f->fd.out_idx[i] = -1;   // patched to cnt_idx below
+      fd.out_kind[i] = 0;
+      fd.out_idx[i] = -1;   // patched to cnt_idx below
     } else { delete f; return vdl_fail(ctx, VDL_EINVAL, "fused scan: fold op %d", s.op); }
   }
   KAcc cnt;
@@ -345,7 +322,7 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     k.acc[k.nacc++] = first;
   }
   for (int i = 0; i < desc->nfolds; i++)
-    if (f->fd.out_kind[i] == 0 && f->fd.out_idx[i] < 0) f->fd.out_idx[i] = k.cnt_idx;
+    if (fd.out_kind[i] == 0 && fd.out_idx[i] < 0) fd.out_idx[i] = k.cnt_idx;
 
   // geometry: consumer threads NC, rows per thread and tile R, ring depth, lane-private tables (or none: register slots)
   const int smem_max = ctx->smem_optin > 0 ? ctx->smem_optin : 232448;
@@ -596,50 +573,38 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
   int rc = vec_new(ctx, VDL_I64, (i64)(k.nacc + k.nchoose) * k.domain, &f->table);
   if (rc) { delete f; return rc; }
   k.table = (i64 *)ctx->vecs[f->table].ptr;
-  {
-    size_t nb = ((size_t)(f->nout + desc->nposts) * k.domain + 3) * sizeof(i64);
-    if (cudaMalloc(&f->d_outbuf, nb) != cudaSuccess || cudaHostAlloc(&f->h_outbuf, nb, cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer(&f->h_mapped, f->h_outbuf, 0) != cudaSuccess || cudaMalloc(&f->d_done, sizeof(unsigned int)) != cudaSuccess ||
-        cudaMemsetAsync(f->d_done, 0, sizeof(unsigned int), ctx->stream) != cudaSuccess) {
-      vdl_fused_destroy(f);
-      return vdl_fail(ctx, VDL_ENOMEM, "fused scan: result buffers");
-    }
-    k.done = f->d_done;
-    memset(f->h_outbuf, 0, nb);        // (the publication word must not start out looking like a finished step)
+  fd.nacc = k.nacc;
+  fd.nchoose = k.nchoose;
+  fd.cnt_idx = k.cnt_idx;
+  fd.first_idx = k.first_idx;
+  for (int j = 0; j < k.nacc; j++) fd.acc_op[j] = k.acc[j].op;
+  for (int q = 0; q < desc->nposts; q++) fd.post[q] = desc->post[q];
+  fd.reset_table = k.table;      // a finalize is the last reader of the table: it leaves the identities for the next launch
+  static const FoldTexts texts = {"finalize: nranks %d without gathered partials",
+                                  "fused scan: peer exchange requested before vdl_fused_set_peers", "fused scan not finalized",
+                                  "fused scan: a peer GPU never delivered its partial table (exchange timed out)",
+                                  "fused scan: %lld rows produced a group key outside the key domain"};
+  if (f->cb.allocate(ctx, &texts, k.table, (i64)(k.nacc + k.nchoose) * k.domain, k.domain, f->nout, desc->nposts) ||
+      cudaMalloc(&f->d_done, sizeof(unsigned int)) != cudaSuccess || cudaMemsetAsync(f->d_done, 0, sizeof(unsigned int), ctx->stream) != cudaSuccess) {
+    vdl_fused_destroy(f);
+    return vdl_fail(ctx, VDL_ENOMEM, "fused scan: result buffers");
   }
+  k.done = f->d_done;
   for (int i = 0; i < f->nout; i++) {   // the fold results are views into the one result buffer
     rc = vec_new_range(ctx, 0, 0, 0, &f->out[i]);
     if (rc) { vdl_fused_destroy(f); return rc; }
     Vec &v = ctx->vecs[f->out[i]];
     v.is_range = false;
-    v.ptr = f->d_outbuf + (size_t)i * k.domain;
+    v.ptr = fd.out[i];
     v.dtype = VDL_I64;
     v.cap_rows = k.domain;
     v.domain = -1;
-    f->fd.out[i] = (i64 *)v.ptr;
   }
-  for (int i = 0; i < VDL_EVENT_RING; i++) { cudaEventCreate(&f->ev0[i]); cudaEventCreate(&f->ev1[i]); }
-  f->fd.domain = k.domain;
-  f->fd.nacc = k.nacc;
-  f->fd.nchoose = k.nchoose;
-  f->fd.cnt_idx = k.cnt_idx;
-  f->fd.first_idx = k.first_idx;
-  f->fd.nout = f->nout;
-  f->fd.part_stride = (i64)(k.nacc + k.nchoose) * k.domain;
-  f->fd.npost = desc->nposts;
-  for (int q = 0; q < desc->nposts; q++) {
-    f->fd.post[q] = desc->post[q];
-    f->fd.post_out[q] = f->d_outbuf + (size_t)(f->nout + q) * k.domain;
-  }
-  f->fd.ngroups = f->d_outbuf + (size_t)(f->nout + desc->nposts) * k.domain;
-  f->fd.errflag = ctx->d_errflag;
-  f->fd.hmirror = f->h_mapped;
-  for (int j = 0; j < k.nacc; j++) f->fd.acc_op[j] = k.acc[j].op;
+  f->timer.create();
 
-  {   // load every kernel a step may launch now, not lazily behind a peer's spinning exchange (see vdl_probe_prepare)
+  {   // load every kernel a step may launch now, not lazily behind a peer's spinning exchange (see FoldCombine::allocate)
     cudaFuncAttributes fa;
-    cudaFuncGetAttributes(&fa, fused_init_kernel); cudaFuncGetAttributes(&fa, fused_choose_kernel); cudaFuncGetAttributes(&fa, fused_finalize_kernel);
-    cudaFuncGetAttributes(&fa, fused_exchange_kernel);
+    cudaFuncGetAttributes(&fa, fused_init_kernel); cudaFuncGetAttributes(&fa, fused_choose_kernel);
     cudaGetLastError();
   }
   cudaError_t e = cudaFuncSetAttribute(f->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -663,15 +628,15 @@ extern "C" int vdl_fused_launch_ex(vdl_fused *f, int self_finalize) {
   VDL_CUDA(ctx, cudaSetDevice(ctx->device));
   if (!vdl_fused_current(f))
     return vdl_fail(ctx, VDL_ESTALE, "fused scan: a column was rewritten or dropped after vdl_fused_prepare (its statistics proofs no longer hold): prepare again");
-  f->finalized = false;
-  f->ngroups = -1;
-  if (!f->table_clean) {
+  f->cb.finalized = false;
+  f->cb.ngroups = -1;
+  if (!f->cb.table_clean) {
     int nb = (int)std::min<i64>(ctx->sm_count, ((i64)(f->kd.nacc + f->kd.nchoose) * f->kd.domain + 255) / 256);
     fused_init_kernel<<<std::max(nb, 1), 256, 0, ctx->stream>>>(f->kd);
     ctx->launches++;
-    f->table_clean = true;
+    f->cb.table_clean = true;
   }
-  VDL_CUDA(ctx, cudaEventRecord(f->ev0[f->nlaunch % VDL_EVENT_RING], ctx->stream));
+  VDL_TRY(f->timer.begin(ctx));
   cudaKernel_t jit_launch = f->jit ? f->jit_kernel : nullptr;
   if (f->rs) {
     int g = f->rs_gmax;
@@ -690,132 +655,69 @@ extern "C" int vdl_fused_launch_ex(vdl_fused *f, int self_finalize) {
     f->kd.gmax = g;
   }
   const bool scan = f->kd.rows > 0 && !f->always_false;
-  if (self_finalize == 2) {
-    if (f->xd.world < 1) return vdl_fail(ctx, VDL_EINVAL, "fused scan: peer exchange requested before vdl_fused_set_peers");
-    f->xd.epoch++;
-  }
-  f->fd.parts = f->kd.table;
-  f->fd.nranks = 1;
-  f->fd.reset_table = f->kd.table;
-  if (self_finalize) f->fd.seq++;
+  FoldCombine &cb = f->cb;
+  if (self_finalize == 2) VDL_TRY(cb.next_epoch());
   if (scan) {
+    cb.fd.parts = f->kd.table;           // the epilogue's single-rank finalize
+    if (self_finalize) cb.fd.seq++;
     f->kd.epilogue = self_finalize == 2 ? 3 : (self_finalize ? 2 : 1);
     if (jit_launch) {
-      void *args[] = {(void *)&f->kd, (void *)&f->fd, (void *)&f->xd};
+      void *args[] = {(void *)&f->kd, (void *)&cb.fd, (void *)&cb.xd};
       VDL_CUDA(ctx, cudaLaunchKernel((const void *)jit_launch, dim3(f->grid), dim3(f->nc + 32), args, f->smem_bytes, ctx->stream));
     } else {
-      f->kernel<<<f->grid, f->nc + 32, f->smem_bytes, ctx->stream>>>(f->kd, f->fd, f->xd);
+      f->kernel<<<f->grid, f->nc + 32, f->smem_bytes, ctx->stream>>>(f->kd, cb.fd, cb.xd);
     }
     ctx->launches++;
-    f->table_clean = self_finalize != 0;
+    f->cb.table_clean = self_finalize != 0;
   } else if (self_finalize == 2) {       // nothing to scan here, but the other ranks wait for this rank's table
-    fused_exchange_kernel<<<1, 256, 0, ctx->stream>>>(f->kd, f->fd, f->xd);
-    ctx->launches++;
+    VDL_TRY(cb.exchange());
   } else if (self_finalize) {            // nothing to scan: the (identity) table finalizes to zero groups
-    fused_finalize_kernel<<<1, 256, 0, ctx->stream>>>(f->fd);
-    ctx->launches++;
+    VDL_TRY(cb.finalize(nullptr, 1));
   }
-  VDL_CUDA(ctx, cudaEventRecord(f->ev1[f->nlaunch % VDL_EVENT_RING], ctx->stream));
-  f->nlaunch++;
-  f->timed = true;
+  VDL_TRY(f->timer.end(ctx));
   VDL_CUDA(ctx, cudaGetLastError());
-  if (self_finalize) f->finalized = true;
+  if (self_finalize) cb.finalized = true;
   return VDL_OK;
 }
 
-// step counter of the peer exchange; the plan carries it over when a scan is re-prepared on the same buffers
-u64 vdl_fused_epoch(vdl_fused *f) { return f->xd.epoch; }
-void vdl_fused_set_epoch(vdl_fused *f, u64 e) { f->xd.epoch = e; }
+FoldCombine *vdl_fused_combine(vdl_fused *f) { return &f->cb; }
 
-extern "C" int vdl_fused_exchange_bytes(vdl_fused *f, int world, int64_t *bytes) {
-  if (!f || !bytes || world < 1 || world > VDL_MAX_RANKS) return VDL_EINVAL;
-  *bytes = ((int64_t)2 * world * f->fd.part_stride + 2 * world) * (int64_t)sizeof(i64);
-  return VDL_OK;
-}
+extern "C" int vdl_fused_exchange_bytes(vdl_fused *f, int world, int64_t *bytes) { return f ? f->cb.exchange_bytes(world, bytes) : VDL_EINVAL; }
 
-extern "C" int vdl_fused_set_peers(vdl_fused *f, int rank, int world, void *const *peer_buffers) {
-  if (!f || !peer_buffers || world < 1 || world > VDL_MAX_RANKS || rank < 0 || rank >= world) return VDL_EINVAL;
-  memset(&f->xd, 0, sizeof f->xd);
-  f->xd.rank = rank;
-  f->xd.world = world;
-  f->xd.stride = f->fd.part_stride;
-  f->xd.timeout_ns = 10000000000ull;                     // 10 s; VDL_PEER_TIMEOUT_MS overrides (tests)
-  if (const char *e = getenv("VDL_PEER_TIMEOUT_MS")) f->xd.timeout_ns = (u64)atoll(e) * 1000000ull;
-  for (int r = 0; r < world; r++) {
-    if (!peer_buffers[r]) return vdl_fail(f->ctx, VDL_EINVAL, "set_peers: buffer of rank %d is null", r);
-    f->xd.peer[r] = (i64 *)peer_buffers[r];
-  }
-  return VDL_OK;
-}
+extern "C" int vdl_fused_set_peers(vdl_fused *f, int rank, int world, void *const *peer_buffers) { return f ? f->cb.set_peers(rank, world, peer_buffers) : VDL_EINVAL; }
 
 extern "C" int vdl_fused_launch(vdl_fused *f) { return vdl_fused_launch_ex(f, 0); }
 
-extern "C" int vdl_fused_partials(vdl_fused *f, void **device_ptr, int64_t *n_int64) {
-  if (!f || !device_ptr || !n_int64) return VDL_EINVAL;
-  *device_ptr = f->kd.table;
-  *n_int64 = f->fd.part_stride;
-  return VDL_OK;
-}
+extern "C" int vdl_fused_partials(vdl_fused *f, void **device_ptr, int64_t *n_int64) { return f ? f->cb.partials(device_ptr, n_int64) : VDL_EINVAL; }
 
-extern "C" int vdl_fused_finalize(vdl_fused *f, const void *all_partials, int nranks) {
-  if (!f) return VDL_EINVAL;
-  vdl_ctx *ctx = f->ctx;
-  if (nranks < 1 || (nranks > 1 && !all_partials)) return vdl_fail(ctx, VDL_EINVAL, "finalize: nranks %d without gathered partials", nranks);
-  VDL_CUDA(ctx, cudaSetDevice(ctx->device));
-  f->fd.parts = all_partials ? (const i64 *)all_partials : f->kd.table;
-  f->fd.nranks = nranks;
-  f->fd.reset_table = f->kd.table;      // the gathered copies (or this one launch) are the last readers of the table
-  f->fd.seq++;
-  fused_finalize_kernel<<<1, 256, 0, ctx->stream>>>(f->fd);
-  ctx->launches++;
-  VDL_CUDA(ctx, cudaGetLastError());
-  f->table_clean = true;
-  f->finalized = true;
-  f->ngroups = -1;
-  return VDL_OK;
-}
+extern "C" int vdl_fused_finalize(vdl_fused *f, const void *all_partials, int nranks) { return f ? f->cb.finalize(all_partials, nranks) : VDL_EINVAL; }
 
-// One device->host copy brings the group count, the error counter and every fold result.
+// The group count, the error counter and every result, published by the finalize into mapped pinned memory.
 static int fused_fetch(vdl_fused *f) {
-  vdl_ctx *ctx = f->ctx;
-  if (!f->finalized) return vdl_fail(ctx, VDL_EINVAL, "fused scan not finalized");
-  if (f->ngroups >= 0) return VDL_OK;
-  size_t n = (size_t)(f->nout + f->fd.npost) * f->kd.domain + 2;
-  VDL_TRY(wait_published(ctx, f->h_outbuf + n, f->fd.seq));   // the finalize wrote the results straight into h_outbuf (mapped)
-  i64 ng = f->h_outbuf[n - 2], err = f->h_outbuf[n - 1];
-  if (err) {
-    cudaMemsetAsync(ctx->d_errflag, 0, sizeof(int), ctx->stream);
-    if (err >= (1 << 20)) return vdl_fail(ctx, VDL_ECUDA, "fused scan: a peer GPU never delivered its partial table (exchange timed out)");
-    return vdl_fail(ctx, VDL_ERANGE, "fused scan: %lld rows produced a group key outside the key domain", (long long)err);
-  }
-  f->ngroups = ng;
-  f->groups_seen = ng;
-  for (int i = 0; i < f->nout; i++) ctx->vecs[f->out[i]].len = ng;
+  VDL_TRY(f->cb.fetch());
+  f->groups_seen = f->cb.ngroups;
+  for (int i = 0; i < f->nout; i++) f->ctx->vecs[f->out[i]].len = f->cb.ngroups;
   return VDL_OK;
 }
 
 extern "C" int vdl_fused_num_groups(vdl_fused *f, int64_t *ngroups) {
   if (!f || !ngroups) return VDL_EINVAL;
   VDL_TRY(fused_fetch(f));
-  *ngroups = f->ngroups;
+  *ngroups = f->cb.ngroups;
   return VDL_OK;
 }
 
 // Host copy of fold `fold_index`'s result (valid until the next launch); no device work beyond the one fetch.
 extern "C" int vdl_fused_result_host(vdl_fused *f, int fold_index, const int64_t **data, int64_t *len) {
-  if (!f || !data || !len || fold_index < 0 || fold_index >= f->nout) return VDL_EINVAL;
+  if (!f || fold_index < 0 || fold_index >= f->nout) return VDL_EINVAL;
   VDL_TRY(fused_fetch(f));
-  *data = f->h_outbuf + (size_t)fold_index * f->kd.domain;
-  *len = f->ngroups;
-  return VDL_OK;
+  return f->cb.result_host(fold_index, data, len);
 }
 
 extern "C" int vdl_fused_post_host(vdl_fused *f, int post_index, const int64_t **data, int64_t *len) {
-  if (!f || !data || !len || post_index < 0 || post_index >= f->fd.npost) return VDL_EINVAL;
+  if (!f || post_index < 0 || post_index >= f->cb.fd.npost) return VDL_EINVAL;
   VDL_TRY(fused_fetch(f));
-  *data = f->h_outbuf + (size_t)(f->nout + post_index) * f->kd.domain;
-  *len = f->ngroups;
-  return VDL_OK;
+  return f->cb.result_host(f->nout + post_index, data, len);
 }
 
 extern "C" int vdl_fused_result(vdl_fused *f, int fold_index, vdl_vec *out) {
@@ -828,32 +730,16 @@ extern "C" int vdl_fused_result(vdl_fused *f, int fold_index, vdl_vec *out) {
 
 extern "C" int vdl_fused_last_kernel_ms(vdl_fused *f, float *ms) {
   if (!f || !ms) return VDL_EINVAL;
-  if (!f->timed) return vdl_fail(f->ctx, VDL_EINVAL, "fused scan not launched yet");
-  const int i = (int)((f->nlaunch - 1) % VDL_EVENT_RING);
-  VDL_CUDA(f->ctx, cudaEventSynchronize(f->ev1[i]));
-  VDL_CUDA(f->ctx, cudaEventElapsedTime(ms, f->ev0[i], f->ev1[i]));
-  return VDL_OK;
+  if (!f->timer.n) return vdl_fail(f->ctx, VDL_EINVAL, "fused scan not launched yet");
+  return f->timer.last_ms(f->ctx, ms);
 }
 
 // Mean / minimum duration of the scan kernel over the last `n` launches (n <= VDL_EVENT_RING), from event pairs recorded
 // around each launch: a timed loop reads them afterwards instead of synchronising on an event every step.
 extern "C" int vdl_fused_kernel_ms_stats(vdl_fused *f, int n, float *mean_ms, float *min_ms) {
   if (!f || n < 1) return VDL_EINVAL;
-  if (!f->timed) return vdl_fail(f->ctx, VDL_EINVAL, "fused scan not launched yet");
-  n = (int)std::min<long>(std::min<long>(n, VDL_EVENT_RING), f->nlaunch);
-  double sum = 0;
-  float mn = 1e30f;
-  for (int k = 1; k <= n; k++) {
-    const int i = (int)((f->nlaunch - k) % VDL_EVENT_RING);
-    float ms = 0;
-    VDL_CUDA(f->ctx, cudaEventSynchronize(f->ev1[i]));
-    VDL_CUDA(f->ctx, cudaEventElapsedTime(&ms, f->ev0[i], f->ev1[i]));
-    sum += ms;
-    mn = std::min(mn, ms);
-  }
-  if (mean_ms) *mean_ms = (float)(sum / n);
-  if (min_ms) *min_ms = mn;
-  return VDL_OK;
+  if (!f->timer.n) return vdl_fail(f->ctx, VDL_EINVAL, "fused scan not launched yet");
+  return f->timer.stats(f->ctx, n, mean_ms, min_ms);
 }
 
 extern "C" const char *vdl_fused_shape_name(vdl_fused *f) { return f ? f->shape : ""; }
@@ -866,10 +752,9 @@ extern "C" int vdl_fused_destroy(vdl_fused *f) {
   if (f->table) vdl_vec_free(ctx, f->table);
   for (int i = 0; i < f->nout; i++)
     if (f->out[i]) vdl_vec_free(ctx, f->out[i]);
-  if (f->d_outbuf) cudaFree(f->d_outbuf);
+  f->cb.release();
   if (f->d_done) cudaFree(f->d_done);
-  if (f->h_outbuf) cudaFreeHost(f->h_outbuf);
-  for (int i = 0; i < VDL_EVENT_RING; i++) { if (f->ev0[i]) cudaEventDestroy(f->ev0[i]); if (f->ev1[i]) cudaEventDestroy(f->ev1[i]); }
+  f->timer.destroy();
   delete f;
   return VDL_OK;
 }

@@ -5,7 +5,6 @@
 
 #include "vdl_device.cuh"
 
-#define K_MAX_ACC 10
 #define K_MAX_CHOOSE 6
 
 // soff / w4 are derived by the host from col: byte offset of the column inside a staged tile, 4-byte flag.
@@ -33,23 +32,6 @@ struct KDesc {
   // is the only launch of a step), 3 the same with the peer-memory exchange of the tables before the finalize.
   unsigned int *done;
   int32_t epilogue, pad1;
-};
-
-struct FinDesc {
-  const i64 *parts;              // nranks tables back to back, each part_stride int64
-  i64 part_stride, domain;
-  int32_t nranks, nacc, nchoose, cnt_idx, first_idx, nout;
-  int32_t acc_op[K_MAX_ACC];
-  int32_t out_kind[VDL_MAX_AGGS], out_idx[VDL_MAX_AGGS];   // kind 0: accumulator, 1: choose
-  i64 *out[VDL_MAX_AGGS];
-  int32_t npost, pad;
-  vdl_post_op post[VDL_MAX_POSTS];
-  i64 *post_out[VDL_MAX_POSTS];
-  i64 *ngroups;                  // [0] number of groups, [1] snapshot of the context's error counter, [2] (host mirror only) seq
-  i64 seq;                       // number of this finalize: the last word the kernel publishes to the host mirror
-  const int *errflag;
-  i64 *hmirror;                  // mapped pinned host copy of the whole result buffer (same layout as out[0]...), or null
-  i64 *reset_table;              // this rank's partial table, re-initialised for the next launch after the merge, or null
 };
 
 // ------------------------------------------------------------------------------ PTX helpers
@@ -92,10 +74,6 @@ __device__ __forceinline__ uint64_t policy_evict_first() {
 template <int NC>
 __device__ __forceinline__ void consumer_barrier() { asm volatile("bar.sync 1, %0;" ::"n"(NC) : "memory"); }
 
-__device__ __forceinline__ i64 acc_identity(int op) { return op == 0 ? 0 : (op == 1 ? INT64_MAX : INT64_MIN); }
-__device__ __forceinline__ i64 acc_combine(int op, i64 a, i64 v) {
-  return op == 0 ? (i64)((u64)a + (u64)v) : (op == 1 ? (v < a ? v : a) : (v > a ? v : a));
-}
 __device__ __forceinline__ void acc_global(int op, i64 *p, i64 v) {
   if (op == 0) atomicAdd((unsigned long long *)p, (unsigned long long)v);
   else if (op == 1) atomicMin((long long *)p, (long long)v);
@@ -559,10 +537,6 @@ __device__ __forceinline__ void select_rows(const KDesc &d, const unsigned char 
 }
 
 __device__ __forceinline__ void choose_keys(const KDesc &d, i64 k0, i64 kstride);
-template <int NT>
-__device__ __forceinline__ void finalize_block(const FinDesc &f, const i64 *parts, int nranks, int tid, int *warp_cnt, i64 *running);
-template <int NT>
-__device__ __forceinline__ const i64 *exchange_block(const XDesc &x, const i64 *table, int *errflag, int tid);
 
 template <class S, int NC, int R, int G>
 __device__ __forceinline__ void fused_scan_fold_body(const KDesc &d, const FinDesc &fd, const XDesc &xd) {
@@ -788,112 +762,3 @@ __global__ void fused_choose_kernel(const __grid_constant__ KDesc d) {
   choose_keys(d, (i64)blockIdx.x * blockDim.x + threadIdx.x, (i64)gridDim.x * blockDim.x);
 }
 #endif
-
-// Merge the per-rank tables, drop empty keys, emit one dense vector per fold in ascending key order, run the post
-// ops, optionally re-initialise this rank's table.  One thread block of NT threads (threads tid 0..NT-1; the
-// barrier is the named barrier 2 so that the scan kernel's consumer warps can run it without the producer warp).
-// Store this rank's table into every rank's exchange buffer, publish the epoch, wait for every rank's epoch.
-// Returns the [world][stride] block of this rank's own buffer that now holds all tables of the step.
-template <int NT>
-__device__ __forceinline__ const i64 *exchange_block(const XDesc &x, const i64 *table, int *errflag, int tid) {
-  auto bar = []() { asm volatile("bar.sync 2, %0;" ::"n"(NT) : "memory"); };
-  const int par = (int)(x.epoch & 1);
-  const size_t slot = ((size_t)par * x.world + x.rank) * x.stride, flags = (size_t)2 * x.world * x.stride;
-  for (int p = 0; p < x.world; p++) {                // NVLink stores (plain st.global to the peer mapping)
-    i64 *dst = x.peer[p] + slot;
-    for (i64 i = tid; i < x.stride; i += NT) dst[i] = __ldcg(&table[i]);
-  }
-  __threadfence_system();
-  bar();
-  if (tid < x.world) {
-    st_release_sys((u64 *)(x.peer[tid] + flags) + (size_t)par * x.world + x.rank, x.epoch);
-    const u64 *mine = (const u64 *)(x.peer[x.rank] + flags) + (size_t)par * x.world + tid;
-    const u64 t0 = global_timer_ns();
-    while (ld_acquire_sys(mine) < x.epoch) {
-      if (global_timer_ns() - t0 > x.timeout_ns) { atomicAdd(errflag, 1 << 20); break; }   // a peer never arrived: fail, do not hang
-      __nanosleep(64);
-    }
-  }
-  bar();
-  return x.peer[x.rank] + (size_t)par * x.world * x.stride;
-}
-
-template <int NT>
-__device__ __forceinline__ void finalize_block(const FinDesc &f, const i64 *parts, int nranks, int tid, int *warp_cnt, i64 *running) {
-  constexpr int NWF = NT / 32;
-  auto bar = []() { asm volatile("bar.sync 2, %0;" ::"n"(NT) : "memory"); };
-  const int lane = tid & 31, warp = tid >> 5;
-  // out[] / post_out[] / ngroups live in one device buffer that starts at out[0]; hmirror has the same layout
-  auto mirror = [&](i64 *dev) { return f.hmirror + (dev - f.out[0]); };
-  if (tid == 0) *running = 0;
-  bar();
-  for (i64 base = 0; base < f.domain; base += NT) {
-    i64 k = base + tid;
-    i64 cnt = 0;
-    if (k < f.domain)
-      for (int r = 0; r < nranks; r++) cnt += __ldcg(&parts[(size_t)r * f.part_stride + (size_t)f.cnt_idx * f.domain + k]);
-    bool exists = cnt > 0;
-    unsigned m = __ballot_sync(0xffffffffu, exists);
-    if (lane == 0) warp_cnt[warp] = __popc(m);
-    bar();
-    int before = 0, total = 0;
-    for (int w = 0; w < NWF; w++) {
-      if (w < warp) before += warp_cnt[w];
-      total += warp_cnt[w];
-    }
-    if (exists) {
-      i64 pos = *running + before + __popc(m & ((1u << lane) - 1));
-      int best = 0;   // rank holding the first row of this key
-      if (f.nchoose > 0) {
-        i64 bf = INT64_MAX;
-        for (int r = 0; r < nranks; r++) {
-          i64 fr = __ldcg(&parts[(size_t)r * f.part_stride + (size_t)f.first_idx * f.domain + k]);
-          if (fr < bf) { bf = fr; best = r; }
-        }
-      }
-      i64 ov[VDL_MAX_AGGS], pv[VDL_MAX_POSTS];
-      for (int o = 0; o < f.nout; o++) {
-        i64 v;
-        if (f.out_kind[o] == 1) {
-          v = __ldcg(&parts[(size_t)best * f.part_stride + (size_t)(f.nacc + f.out_idx[o]) * f.domain + k]);
-        } else {
-          int j = f.out_idx[o], op = f.acc_op[j];
-          v = acc_identity(op);
-          for (int r = 0; r < nranks; r++) v = acc_combine(op, v, __ldcg(&parts[(size_t)r * f.part_stride + (size_t)j * f.domain + k]));
-        }
-        f.out[o][pos] = v;
-        if (f.hmirror) mirror(f.out[o])[pos] = v;
-        ov[o] = v;
-      }
-      // elementwise epilogue over the fold results (AVG's Divide, ...)
-      for (int q = 0; q < f.npost; q++) {
-        const vdl_post_op &P = f.post[q];
-        i64 a = P.a_kind == VDL_POST_CONST ? P.a : (P.a_kind == VDL_POST_FOLD ? ov[P.a] : pv[P.a]);
-        i64 b = P.b_kind == VDL_POST_CONST ? P.b : (P.b_kind == VDL_POST_FOLD ? ov[P.b] : pv[P.b]);
-        pv[q] = binop_apply(P.op, a, b);
-        f.post_out[q][pos] = pv[q];
-        if (f.hmirror) mirror(f.post_out[q])[pos] = pv[q];
-      }
-    }
-    bar();
-    if (tid == 0) *running += total;
-    bar();
-  }
-  if (tid == 0) {
-    const i64 ng = *running, err = *f.errflag;
-    f.ngroups[0] = ng; f.ngroups[1] = err;
-    if (f.hmirror) {
-      mirror(f.ngroups)[0] = ng; mirror(f.ngroups)[1] = err;
-      __threadfence_system();                      // every result store of this block (barriers above) before the publication
-      ((volatile i64 *)mirror(f.ngroups))[2] = f.seq;
-    }
-  }
-  if (f.reset_table) {      // every thread has read what it needed (barriers above): identity-initialise for the next launch
-    const i64 n = (i64)(f.nacc + f.nchoose) * f.domain;
-    for (i64 i = tid; i < n; i += NT) {
-      int j = (int)(i / f.domain);
-      f.reset_table[i] = j < f.nacc ? acc_identity(f.acc_op[j]) : 0;
-    }
-  }
-}
-

@@ -8,7 +8,7 @@
 #include <unordered_map>
 #include <vector>
 
-#include "vdl_device.cuh"      // vdl_cuda.h, i64 / u64, XDesc, the device helpers shared with the run-time compiled kernels
+#include "vdl_device.cuh"      // vdl_cuda.h, i64 / u64, XDesc, FinDesc, the device code shared with the run-time compiled kernels
 
 // A device vector.  Columns are vectors with a name.  Ranges (RangeV/RangeC) are kept virtual:
 // no HBM traffic until a consumer needs the values.
@@ -119,8 +119,57 @@ cudaKernel_t vdl_jit_kernel(vdl_ctx *ctx, const std::string &key, const std::str
 // proofs -- int32 narrowing, 32-bit accumulators, the static shape -- and the device pointers are baked in.)
 bool vdl_fused_current(vdl_fused *f);
 bool vdl_probe_current(vdl_probe *p);
-u64 vdl_probe_epoch(vdl_probe *p);
-void vdl_probe_set_epoch(vdl_probe *p, u64 e);
-u64 vdl_fused_epoch(vdl_fused *f);
-void vdl_fused_set_epoch(vdl_fused *f, u64 e);
+
+// Event pairs around the dominant kernel of the last VDL_EVENT_RING launches: durations are read AFTER a timed loop
+// instead of synchronising on an event every step.
+struct KernelTimer {
+  cudaEvent_t ev0[VDL_EVENT_RING] = {nullptr}, ev1[VDL_EVENT_RING] = {nullptr};
+  long n = 0;                        // launches timed so far
+  void create();
+  void destroy();
+  int begin(vdl_ctx *ctx);
+  int end(vdl_ctx *ctx);
+  int last_ms(vdl_ctx *ctx, float *ms);
+  int stats(vdl_ctx *ctx, int count, float *mean_ms, float *min_ms);   // over the last count (<= VDL_EVENT_RING) launches
+};
+
+// The error messages of a fold family (the fused scan, the probe in fold mode) for its FoldCombine.
+struct FoldTexts {
+  const char *nranks;       // printf format of an nranks without gathered tables
+  const char *no_peers;     // peer exchange before set_peers
+  const char *unfinalized;  // results fetched before a finalize
+  const char *timeout;      // a peer never delivered its table
+  const char *range;        // printf format of the number of rows out of range
+};
+
+// Combine of a fold family's per-rank partial tables [rows][domain] into the fold results: this rank's table, the merge
+// (FinDesc: finalize_block), the peer-memory exchange (XDesc: exchange_block), the result buffer the finalize publishes
+// into mapped pinned memory, and its fetch on the host (vdl_combine.cu).
+struct FoldCombine {
+  vdl_ctx *ctx = nullptr;
+  const FoldTexts *texts = nullptr;
+  i64 *table = nullptr;              // this rank's partial table, fd.part_stride int64
+  FinDesc fd;                        // out / post_out / ngroups point into d_out, hmirror into h_out
+  XDesc xd;                          // world 0: no peer exchange configured
+  i64 *d_out = nullptr;              // [nout + npost][domain] results, then [ngroups, errors]
+  i64 *h_out = nullptr;              // mapped pinned mirror (+ [seq]: the publication word)
+  bool finalized = false;            // the last step published results (else it left its table for an external combine)
+  bool table_clean = false;          // the table holds the fold identities (the family's init, or a finalize that reset it)
+  i64 ngroups = -1;                  // -1 until fetch has read the published results
+
+  // fd's layout fields (nacc, nchoose, cnt_idx, first_idx, out_kind, out_idx, acc_op, post, reset_table) are the
+  // family's; this sets the rest and loads the combine kernels (not lazily behind a peer's spinning exchange).
+  int allocate(vdl_ctx *c, const FoldTexts *t, i64 *tab, i64 part_stride, i64 domain, int nout, int npost);
+  void release();
+  int exchange_bytes(int world, int64_t *bytes) const;
+  int set_peers(int rank, int world, void *const *peer_buffers);
+  int partials(void **device_ptr, int64_t *n_int64) const;
+  int next_epoch();                                     // before a step that exchanges over peer memory
+  int finalize(const void *all_partials, int nranks);   // merge gathered tables (null, 1: this rank's own)
+  int exchange();                                       // this rank's table to the peers, then the merge: one launch
+  int fetch();
+  int result_host(int index, const int64_t **data, int64_t *len);   // index over the nout results, then the npost
+};
+FoldCombine *vdl_fused_combine(vdl_fused *f);
+FoldCombine *vdl_probe_combine(vdl_probe *p);   // fold mode only
 

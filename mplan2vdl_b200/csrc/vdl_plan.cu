@@ -68,6 +68,13 @@ struct MapCluster {
 };
 
 struct FusedFold { int node; vdl_fold_spec spec; };
+// peer-memory combine of a fused scan or a probe fold group (vdl_plan_set_peers): re-applied whenever its scan or probe is
+// re-prepared, with the step counter carried over
+struct PeerState {
+  int rank = -1, world = 0;
+  std::vector<void *> buffers;
+  u64 epoch = 0;
+};
 struct FusedGroup {
   int table, sel, keynode;
   std::vector<int> cols;                // Load node of each column slot
@@ -79,10 +86,7 @@ struct FusedGroup {
   vdl_fused *fused = nullptr;
   std::vector<vdl_vec> bound;           // column handles the prepared scan was built for
   i64 bound_rows = -1, bound_base = -1;
-  // peer-memory combine (vdl_plan_set_peers): re-applied whenever the scan is re-prepared
-  int peer_rank = -1, peer_world = 0;
-  std::vector<void *> peers;
-  u64 epoch = 0;
+  PeerState peer;
 };
 
 }  // namespace
@@ -710,9 +714,7 @@ struct ProbeFoldGroup {
   vdl_probe *probe = nullptr;
   std::vector<vdl_vec> bound;
   i64 bound_rows = -1, bound_base = -1;
-  // peer-memory combine (vdl_plan_set_peers): re-applied whenever the probe is re-prepared
-  int peer_rank = -1, peer_world = 0;
-  std::vector<void *> peers;
+  PeerState peer;
 };
 struct EmitGroup {
   int space = -1;
@@ -1557,6 +1559,14 @@ extern "C" int vdl_plan_set_row_base(vdl_plan *p, int64_t row_base) {
   return VDL_OK;
 }
 
+// A freshly prepared scan or probe takes the peers set on the plan and continues its predecessor's step count.
+static int reapply_peers(PeerState &ps, FoldCombine *cb) {
+  if (ps.world < 1) return VDL_OK;
+  VDL_TRY(cb->set_peers(ps.rank, ps.world, ps.buffers.data()));
+  cb->xd.epoch = ps.epoch;
+  return VDL_OK;
+}
+
 static int plan_run_local(vdl_plan *p, int self_finalize) {
   if (!p) return VDL_EINVAL;
   vdl_ctx *ctx = p->ctx;
@@ -1575,28 +1585,22 @@ static int plan_run_local(vdl_plan *p, int self_finalize) {
     // (re)prepare when the binding changed OR a bound column was written since (new write generation): the scan's
     // int32-narrowing / 32-bit-accumulator / static-shape proofs come from statistics of the data it was prepared on
     if (!g.fused || !vdl_fused_current(g.fused) || h != g.bound || rows != g.bound_rows || p->row_base != g.bound_base) {
-      if (g.fused) { g.epoch = vdl_fused_epoch(g.fused); vdl_fused_destroy(g.fused); g.fused = nullptr; }
+      if (g.fused) { g.peer.epoch = vdl_fused_combine(g.fused)->xd.epoch; vdl_fused_destroy(g.fused); g.fused = nullptr; }
       g.desc.rows = rows;
       g.desc.row_base = p->row_base;
       for (size_t c = 0; c < h.size(); c++) g.desc.column[c] = h[c];
       VDL_TRY(vdl_fused_prepare(ctx, &g.desc, &g.fused));
       g.bound = h; g.bound_rows = rows; g.bound_base = p->row_base;
-      if (g.peer_world > 0) {
-        VDL_TRY(vdl_fused_set_peers(g.fused, g.peer_rank, g.peer_world, g.peers.data()));
-        vdl_fused_set_epoch(g.fused, g.epoch);
-      }
+      VDL_TRY(reapply_peers(g.peer, vdl_fused_combine(g.fused)));
     }
-    VDL_TRY(vdl_fused_launch_ex(g.fused, self_finalize && g.peer_world > 0 ? 2 : self_finalize));
+    VDL_TRY(vdl_fused_launch_ex(g.fused, self_finalize && g.peer.world > 0 ? 2 : self_finalize));
   }
   for (auto *g : p->pgroups) {
     vdl_probe *before = g->probe;
-    const u64 epoch = before ? vdl_probe_epoch(before) : 0;       // (read before a re-prepare destroys the probe)
+    if (before) g->peer.epoch = vdl_probe_combine(before)->xd.epoch;   // (read before a re-prepare destroys the probe)
     VDL_TRY(bind_probe(p, &g->b, &g->probe, &g->bound, &g->bound_rows, &g->bound_base));
-    if (g->probe != before && g->peer_world > 0) {
-      VDL_TRY(vdl_probe_set_peers(g->probe, g->peer_rank, g->peer_world, g->peers.data()));
-      vdl_probe_set_epoch(g->probe, epoch);
-    }
-    VDL_TRY(vdl_probe_run_ex(g->probe, self_finalize && g->peer_world > 0 ? 2 : self_finalize));
+    if (g->probe != before) VDL_TRY(reapply_peers(g->peer, vdl_probe_combine(g->probe)));
+    VDL_TRY(vdl_probe_run_ex(g->probe, self_finalize && g->peer.world > 0 ? 2 : self_finalize));
   }
   if (!self_finalize)        // sharded run: the survivors' vectors are exchanged between ranks before the tail is evaluated
     for (auto *g : p->egroups) VDL_TRY(run_emit_group(p, *g));
@@ -1618,33 +1622,35 @@ extern "C" int vdl_plan_fused(vdl_plan *p, int i, vdl_fused **out) {
   return *out ? VDL_OK : vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
 }
 
-// `index` runs over the plan's partial tables in the order of vdl_plan_partials: fused scans first, then probe fold groups
-extern "C" int vdl_plan_exchange_bytes(vdl_plan *p, int index, int world, int64_t *bytes) {
-  if (!p || index < 0 || index >= (int)(p->groups.size() + p->pgroups.size())) return VDL_EINVAL;
-  if (index < (int)p->groups.size()) {
-    if (!p->groups[index].fused) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
-    return vdl_fused_exchange_bytes(p->groups[index].fused, world, bytes);
+// Partial table i of the plan, in the order of vdl_plan_partials: fused scans first, then probe fold groups.  *cb is the
+// combine of its prepared scan or probe, null before the plan has run.
+static PeerState *plan_partial(vdl_plan *p, int i, FoldCombine **cb) {
+  if (i < (int)p->groups.size()) {
+    FusedGroup &g = p->groups[i];
+    *cb = g.fused ? vdl_fused_combine(g.fused) : nullptr;
+    return &g.peer;
   }
-  ProbeFoldGroup &g = *p->pgroups[index - p->groups.size()];
-  if (!g.probe) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
-  return vdl_probe_exchange_bytes(g.probe, world, bytes);
+  ProbeFoldGroup *g = p->pgroups[i - p->groups.size()];
+  *cb = g->probe ? vdl_probe_combine(g->probe) : nullptr;
+  return &g->peer;
+}
+
+extern "C" int vdl_plan_exchange_bytes(vdl_plan *p, int index, int world, int64_t *bytes) {
+  if (!p || index < 0 || index >= vdl_plan_num_partials(p)) return VDL_EINVAL;
+  FoldCombine *cb;
+  plan_partial(p, index, &cb);
+  if (!cb) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
+  return cb->exchange_bytes(world, bytes);
 }
 
 extern "C" int vdl_plan_set_peers(vdl_plan *p, int index, int rank, int world, void *const *peer_buffers) {
-  if (!p || index < 0 || index >= (int)(p->groups.size() + p->pgroups.size()) || !peer_buffers || world < 1 || world > VDL_MAX_RANKS) return VDL_EINVAL;
-  if (index < (int)p->groups.size()) {
-    FusedGroup &g = p->groups[index];
-    g.peer_rank = rank; g.peer_world = world;
-    g.peers.assign(peer_buffers, peer_buffers + world);
-    g.epoch = 0;
-    if (g.fused) VDL_TRY(vdl_fused_set_peers(g.fused, rank, world, g.peers.data()));
-    return VDL_OK;
-  }
-  ProbeFoldGroup &g = *p->pgroups[index - p->groups.size()];
-  g.peer_rank = rank; g.peer_world = world;
-  g.peers.assign(peer_buffers, peer_buffers + world);
-  if (g.probe) VDL_TRY(vdl_probe_set_peers(g.probe, rank, world, g.peers.data()));
-  return VDL_OK;
+  if (!p || index < 0 || index >= vdl_plan_num_partials(p) || !peer_buffers || world < 1 || world > VDL_MAX_RANKS) return VDL_EINVAL;
+  FoldCombine *cb;
+  PeerState &ps = *plan_partial(p, index, &cb);
+  ps.rank = rank; ps.world = world;
+  ps.buffers.assign(peer_buffers, peer_buffers + world);
+  ps.epoch = 0;
+  return cb ? cb->set_peers(rank, world, ps.buffers.data()) : VDL_OK;
 }
 
 // ---- vectors emitted by probe passes, for the exchange of survivors in a sharded run --------------------------------
@@ -1688,13 +1694,10 @@ extern "C" int vdl_plan_emit_replace(vdl_plan *p, int i, void *device_ptr, int64
 extern "C" int vdl_plan_num_partials(vdl_plan *p) { return p ? (int)(p->groups.size() + p->pgroups.size()) : 0; }
 extern "C" int vdl_plan_partials(vdl_plan *p, int i, void **device_ptr, int64_t *n_int64) {
   if (!p || i < 0 || i >= vdl_plan_num_partials(p)) return VDL_EINVAL;
-  if (i < (int)p->groups.size()) {
-    if (!p->groups[i].fused) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
-    return vdl_fused_partials(p->groups[i].fused, device_ptr, n_int64);
-  }
-  ProbeFoldGroup *g = p->pgroups[i - p->groups.size()];
-  if (!g->probe) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
-  return vdl_probe_partials(g->probe, device_ptr, n_int64);
+  FoldCombine *cb;
+  plan_partial(p, i, &cb);
+  if (!cb) return vdl_fail(p->ctx, VDL_EINVAL, "plan has not run yet");
+  return cb->partials(device_ptr, n_int64);
 }
 
 extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int nranks) {
@@ -1707,10 +1710,12 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
     return vdl_fail(ctx, VDL_EUNSUPPORTED, "a plan without a fused scan or a probe pass cannot be row-sharded");
   i64 l0 = ctx->launches;
   if (!(p->self_finalized && nranks == 1 && !all_partials)) {
-    for (size_t gi = 0; gi < p->groups.size(); gi++)
-      VDL_TRY(vdl_fused_finalize(p->groups[gi].fused, all_partials ? all_partials[gi] : nullptr, nranks));
-    for (size_t gi = 0; gi < p->pgroups.size(); gi++)
-      VDL_TRY(vdl_probe_finalize(p->pgroups[gi]->probe, all_partials ? all_partials[p->groups.size() + gi] : nullptr, nranks));
+    for (int i = 0; i < vdl_plan_num_partials(p); i++) {
+      FoldCombine *cb;
+      plan_partial(p, i, &cb);
+      if (!cb) return vdl_fail(ctx, VDL_EINVAL, "plan has not run yet");
+      VDL_TRY(cb->finalize(all_partials ? all_partials[i] : nullptr, nranks));
+    }
   }
   bool ran_ops = false, copies_pending = false;
   const bool ordered = !p->order_key.empty() || p->order_limit >= 0;

@@ -331,101 +331,18 @@ __global__ void probe_choose_kernel(const __grid_constant__ PDesc d) {
   }
 }
 
-// One dense vector per fold in ascending key order (keys without rows dropped: G14), FoldChoose evaluated at the
-// key's first row, then the post ops; results mirrored into mapped host memory.
-__global__ void __launch_bounds__(256, 1) probe_finalize_kernel(const __grid_constant__ PDesc d, const __grid_constant__ PFin f) {
+// Single GPU: the finalize evaluates FoldChoose itself, at the key's first row (no choose launch).
+struct ChooseAtFirstRow {
+  const PDesc &d;
+  __device__ __forceinline__ i64 operator()(const FinDesc &f, const i64 *, int o, i64, int, i64 first) const {
+    bool ok = true;
+    return prod_value(d, d.fold[o], first - d.row_base, ok);
+  }
+};
+__global__ void __launch_bounds__(256, 1) probe_finalize_kernel(const __grid_constant__ PDesc d, const __grid_constant__ FinDesc f) {
   __shared__ int warp_cnt[8];
   __shared__ i64 running;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) running = 0;
-  __syncthreads();
-  for (i64 base = 0; base < f.domain; base += 256) {
-    const i64 k = base + tid;
-    i64 cnt = 0;
-    if (k < f.domain)
-      for (int r = 0; r < f.nranks; r++) cnt += f.table[(size_t)r * f.stride + (size_t)f.nfolds * f.domain + k];
-    const bool exists = cnt > 0;
-    unsigned m = __ballot_sync(0xffffffffu, exists);
-    if (lane == 0) warp_cnt[warp] = __popc(m);
-    __syncthreads();
-    int before = 0, total = 0;
-    for (int w = 0; w < 8; w++) { if (w < warp) before += warp_cnt[w]; total += warp_cnt[w]; }
-    if (exists) {
-      const i64 pos = running + before + __popc(m & ((1u << lane) - 1));
-      int best = 0;                 // rank that holds the key's first row
-      i64 firstg = INT64_MAX;
-      for (int r = 0; r < f.nranks; r++) {
-        const i64 fr = f.table[(size_t)r * f.stride + (size_t)(f.nfolds + 1) * f.domain + k];
-        if (fr < firstg) { firstg = fr; best = r; }
-      }
-      const i64 first = firstg - d.row_base;
-      i64 ov[VDL_MAX_AGGS], pv[VDL_MAX_POSTS];
-      bool ok = true;
-      for (int j = 0; j < f.nfolds; j++) {
-        const int op = f.fold_op[j];
-        i64 v;
-        if (op == VDL_FOLD_COUNT) v = cnt;
-        else if (op == VDL_FOLD_CHOOSE) v = f.precomputed_choose ? f.table[(size_t)best * f.stride + (size_t)j * f.domain + k] : prod_value(d, d.fold[j], first, ok);
-        else {
-          v = p_identity(op);
-          for (int r = 0; r < f.nranks; r++) {
-            const i64 x = f.table[(size_t)r * f.stride + (size_t)j * f.domain + k];
-            v = op == VDL_FOLD_MIN ? (x < v ? x : v) : (op == VDL_FOLD_MAX ? (x > v ? x : v) : (i64)((u64)v + (u64)x));
-          }
-        }
-        ov[j] = v;
-        f.out[(size_t)j * f.domain + pos] = v;
-        if (f.hmirror) f.hmirror[(size_t)j * f.domain + pos] = v;
-      }
-      for (int q = 0; q < f.npost; q++) {
-        const vdl_post_op &P = f.post[q];
-        i64 a = P.a_kind == VDL_POST_CONST ? P.a : (P.a_kind == VDL_POST_FOLD ? ov[P.a] : pv[P.a]);
-        i64 b = P.b_kind == VDL_POST_CONST ? P.b : (P.b_kind == VDL_POST_FOLD ? ov[P.b] : pv[P.b]);
-        pv[q] = binop_apply(P.op, a, b);
-        f.out[(size_t)(f.nfolds + q) * f.domain + pos] = pv[q];
-        if (f.hmirror) f.hmirror[(size_t)(f.nfolds + q) * f.domain + pos] = pv[q];
-      }
-    }
-    __syncthreads();
-    if (tid == 0) running += total;
-    __syncthreads();
-  }
-  if (tid == 0) {
-    const size_t tail = (size_t)(f.nfolds + f.npost) * f.domain;
-    const i64 ng = running, err = *f.errflag;
-    f.out[tail] = ng; f.out[tail + 1] = err;
-    if (f.hmirror) {
-      f.hmirror[tail] = ng; f.hmirror[tail + 1] = err;
-      __threadfence_system();
-      ((volatile i64 *)f.hmirror)[tail + 2] = f.seq;
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------ host side
-// Multi-GPU combine over peer memory, as in the fused scan (XDesc, vdl_internal.h): one block stores this rank's partial
-// table (FoldChoose values included) into slot [parity][rank] of EVERY rank's exchange buffer over NVLink, publishes the
-// step's epoch and waits for the other ranks' flags; the finalize kernel that follows merges the `world` tables that
-// arrived in this rank's own buffer.  A peer that never arrives: error flag after the timeout, never a hang.
-__global__ void __launch_bounds__(256, 1) probe_exchange_kernel(const __grid_constant__ XDesc x, const i64 *table, int *errflag) {
-  const int tid = threadIdx.x;
-  const int par = (int)(x.epoch & 1);
-  const size_t slot = ((size_t)par * x.world + x.rank) * x.stride, flags = (size_t)2 * x.world * x.stride;
-  for (int p = 0; p < x.world; p++) {
-    i64 *dst = x.peer[p] + slot;
-    for (i64 i = tid; i < x.stride; i += 256) dst[i] = __ldcg(&table[i]);
-  }
-  __threadfence_system();
-  __syncthreads();
-  if (tid < x.world) {
-    st_release_sys((u64 *)(x.peer[tid] + flags) + (size_t)par * x.world + x.rank, x.epoch);
-    const u64 *mine = (const u64 *)(x.peer[x.rank] + flags) + (size_t)par * x.world + tid;
-    const u64 t0 = global_timer_ns();
-    while (ld_acquire_sys(mine) < x.epoch) {
-      if (global_timer_ns() - t0 > x.timeout_ns) { atomicAdd(errflag, 1 << 20); break; }
-      __nanosleep(64);
-    }
-  }
+  finalize_block<256>(f, f.parts, 1, threadIdx.x, warp_cnt, &running, ChooseAtFirstRow{d});
 }
 
 #include <string>
@@ -734,21 +651,18 @@ extern "C" int vdl_probe_jit_selftest(char *log, int log_capacity) {
 struct vdl_probe {
   vdl_ctx *ctx = nullptr;
   PDesc pd;
-  PFin pf;
-  XDesc xd;                            // world 0: no peer exchange configured
-  bool folding = true, ran = false, fetched = false, finalized = false;
+  FoldCombine cb;                      // fold mode: the finalize's descriptor, the peer exchange, the results
+  bool folding = true, ran = false, fetched = false;
   vdl_vec table = 0;
-  i64 *d_out = nullptr, *h_out = nullptr, *h_mapped = nullptr;
+  i64 *h_out = nullptr;                // emit mode: host copy of the survivor count
   i64 *d_total = nullptr;              // [0] survivors (emit mode)
   unsigned int *d_ticket = nullptr;
   unsigned long long *d_state = nullptr;
   vdl_vec emit_vec[VDL_MAX_EMITS] = {0};
-  i64 ngroups = -1, nselected = -1;
+  i64 nselected = -1;
   int grid = 1;
   size_t smem = 0;
-  // event pairs around the dominant kernel of the last VDL_EVENT_RING launches: durations are read AFTER a timed loop
-  cudaEvent_t ev0[VDL_EVENT_RING] = {nullptr}, ev1[VDL_EVENT_RING] = {nullptr};
-  long nlaunch = 0;
+  KernelTimer timer;
   cudaKernel_t jit_kernel = nullptr;   // the descriptor printed as CUDA C and compiled at run time (probe_jit_source)
   // identity of the leaf columns at prepare time (device pointers and lengths are baked into the descriptor)
   int nleaves = 0;
@@ -780,11 +694,11 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
   if (desc->rows < 0) return vdl_fail(ctx, VDL_EINVAL, "probe: negative row count");
   VDL_CUDA(ctx, cudaSetDevice(ctx->device));
   vdl_probe *p = new vdl_probe();
-  memset(&p->xd, 0, sizeof p->xd);
   p->ctx = ctx;
   PDesc &d = p->pd;
   memset(&d, 0, sizeof d);
-  memset(&p->pf, 0, sizeof p->pf);
+  FinDesc &fd = p->cb.fd;
+  memset(&fd, 0, sizeof fd);
   auto fail = [&](int rc) { vdl_probe_destroy(p); return rc; };
   d.rows = desc->rows;
   d.row_base = desc->row_base;
@@ -870,16 +784,25 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
       const vdl_post_op &P = desc->post[q];
       auto okk = [&](int kind, i64 v) { return kind == VDL_POST_CONST || (kind == VDL_POST_FOLD && v >= 0 && v < desc->nfolds) || (kind == VDL_POST_POST && v >= 0 && v < q); };
       if (P.op < 0 || P.op > VDL_MODULO || !okk(P.a_kind, P.a) || !okk(P.b_kind, P.b)) return fail(vdl_fail(ctx, VDL_EINVAL, "probe: bad post op %d", q));
-      p->pf.post[q] = P;
+      fd.post[q] = P;
     }
-    size_t nb = ((size_t)(d.nfolds + desc->nposts) * d.domain + 3) * sizeof(i64);
-    if (cudaMalloc(&p->d_out, nb) != cudaSuccess || cudaHostAlloc(&p->h_out, nb, cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer(&p->h_mapped, p->h_out, 0) != cudaSuccess)
+    // the table's layout for the merge: fold j in row j (a FoldChoose's value too: nacc = 0), count, first row
+    fd.cnt_idx = d.nfolds;
+    fd.first_idx = d.nfolds + 1;
+    fd.acc_op[fd.cnt_idx] = VDL_FOLD_SUM;
+    for (int j = 0; j < d.nfolds; j++) {
+      fd.out_kind[j] = d.fold_op[j] == VDL_FOLD_CHOOSE;
+      fd.out_idx[j] = d.fold_op[j] == VDL_FOLD_COUNT ? fd.cnt_idx : j;
+      fd.acc_op[j] = d.fold_op[j];
+      fd.nchoose += d.fold_op[j] == VDL_FOLD_CHOOSE;
+    }
+    static const FoldTexts texts = {"probe finalize: nranks %d without gathered partials",
+                                    "probe: peer exchange requested before vdl_probe_set_peers",
+                                    "probe ran for an external combine: call vdl_probe_finalize first",
+                                    "probe: a peer GPU never delivered its partial table (exchange timed out)",
+                                    "probe: %lld rows had a lookup index or group key out of range"};
+    if (p->cb.allocate(ctx, &texts, d.table, (i64)(d.nfolds + 2) * d.domain, d.domain, d.nfolds, desc->nposts))
       return fail(vdl_fail(ctx, VDL_ENOMEM, "probe: result buffers"));
-    memset(p->h_out, 0, nb);
-    p->pf.domain = d.domain; p->pf.nfolds = d.nfolds; p->pf.npost = desc->nposts;
-    for (int j = 0; j < d.nfolds; j++) p->pf.fold_op[j] = d.fold_op[j];
-    p->pf.table = d.table; p->pf.nranks = 1; p->pf.stride = (i64)(d.nfolds + 2) * d.domain; p->pf.out = p->d_out; p->pf.hmirror = p->h_mapped; p->pf.errflag = ctx->d_errflag;
   } else {
     for (int e = 0; e < desc->nemits; e++)
       if (!prod(desc->emit[e], &d.emit[e])) return fail(vdl_fail(ctx, VDL_EINVAL, "probe: bad emit %d", e));
@@ -902,16 +825,14 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
     for (int l = 0; l < desc->nleaves; l++)
       if (want[l] && d.leaf[l].ptr) { d.pf_ptr[d.npf] = (const unsigned char *)d.leaf[l].ptr; d.pf_shift[d.npf] = d.leaf[l].w4 ? 2 : 3; d.npf++; }
   }
-  for (int i = 0; i < VDL_EVENT_RING; i++) { cudaEventCreate(&p->ev0[i]); cudaEventCreate(&p->ev1[i]); }
+  p->timer.create();
   int per_sm = P_BLOCKS;
   p->grid = (int)std::max<i64>(1, std::min<i64>((i64)ctx->sm_count * per_sm, d.ntiles));
   if (p->smem > 48 * 1024) cudaFuncSetAttribute(probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem);
-  {   // load every kernel a step may launch NOW (CUDA loads lazily, and loading can wait for running kernels: a first
-      // launch of the finalize kernel behind a peer's spinning exchange kernel would stall the host until the exchange
-      // times out -- seen when one host thread drives several ranks)
+  {   // load every kernel a step may launch now, not lazily behind a peer's spinning exchange (see FoldCombine::allocate)
     cudaFuncAttributes fa;
     cudaFuncGetAttributes(&fa, probe_kernel); cudaFuncGetAttributes(&fa, probe_init_kernel); cudaFuncGetAttributes(&fa, probe_choose_kernel);
-    cudaFuncGetAttributes(&fa, probe_exchange_kernel); cudaFuncGetAttributes(&fa, probe_finalize_kernel);
+    cudaFuncGetAttributes(&fa, probe_finalize_kernel);
     cudaGetLastError();
   }
   {   // run-time specialisation (VDL_PROBE_JIT=0 switches it off; VDL_PROBE_JIT_MIN_ROWS, default 262144)
@@ -928,56 +849,19 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
 
 extern "C" int vdl_probe_run(vdl_probe *p) { return vdl_probe_run_ex(p, 1); }
 
-extern "C" int vdl_probe_exchange_bytes(vdl_probe *p, int world, int64_t *bytes) {
-  if (!p || !bytes || !p->folding || world < 1 || world > VDL_MAX_RANKS) return VDL_EINVAL;
-  const int64_t stride = (int64_t)(p->pd.nfolds + 2) * p->pd.domain;
-  *bytes = ((int64_t)2 * world * stride + 2 * world) * (int64_t)sizeof(i64);
-  return VDL_OK;
-}
+FoldCombine *vdl_probe_combine(vdl_probe *p) { return &p->cb; }
+
+extern "C" int vdl_probe_exchange_bytes(vdl_probe *p, int world, int64_t *bytes) { return p && p->folding ? p->cb.exchange_bytes(world, bytes) : VDL_EINVAL; }
 
 extern "C" int vdl_probe_set_peers(vdl_probe *p, int rank, int world, void *const *peer_buffers) {
-  if (!p || !p->folding || !peer_buffers || world < 1 || world > VDL_MAX_RANKS || rank < 0 || rank >= world) return VDL_EINVAL;
-  memset(&p->xd, 0, sizeof p->xd);
-  p->xd.rank = rank;
-  p->xd.world = world;
-  p->xd.stride = (i64)(p->pd.nfolds + 2) * p->pd.domain;
-  p->xd.timeout_ns = 10000000000ull;                     // 10 s; VDL_PEER_TIMEOUT_MS overrides (tests)
-  if (const char *e = getenv("VDL_PEER_TIMEOUT_MS")) p->xd.timeout_ns = (u64)atoll(e) * 1000000ull;
-  for (int r = 0; r < world; r++) {
-    if (!peer_buffers[r]) return vdl_fail(p->ctx, VDL_EINVAL, "set_peers: buffer of rank %d is null", r);
-    p->xd.peer[r] = (i64 *)peer_buffers[r];
-  }
-  return VDL_OK;
+  return p && p->folding ? p->cb.set_peers(rank, world, peer_buffers) : VDL_EINVAL;
 }
 
-// step counter of the peer exchange; the plan carries it over when a probe is re-prepared on the same buffers
-u64 vdl_probe_epoch(vdl_probe *p) { return p->xd.epoch; }
-void vdl_probe_set_epoch(vdl_probe *p, u64 e) { p->xd.epoch = e; }
-
-extern "C" int vdl_probe_partials(vdl_probe *p, void **device_ptr, int64_t *n_int64) {
-  if (!p || !device_ptr || !n_int64 || !p->folding) return VDL_EINVAL;
-  *device_ptr = p->pd.table;
-  *n_int64 = (int64_t)(p->pd.nfolds + 2) * p->pd.domain;
-  return VDL_OK;
-}
+extern "C" int vdl_probe_partials(vdl_probe *p, void **device_ptr, int64_t *n_int64) { return p && p->folding ? p->cb.partials(device_ptr, n_int64) : VDL_EINVAL; }
 
 // Merge `nranks` partial tables laid out back to back (an all-gather result; NULL and 1: this rank's own) and finalize.
 extern "C" int vdl_probe_finalize(vdl_probe *p, const void *all_partials, int nranks) {
-  if (!p || !p->folding) return VDL_EINVAL;
-  vdl_ctx *ctx = p->ctx;
-  if (nranks < 1 || (nranks > 1 && !all_partials)) return vdl_fail(ctx, VDL_EINVAL, "probe finalize: nranks %d without gathered partials", nranks);
-  VDL_CUDA(ctx, cudaSetDevice(ctx->device));
-  p->pf.table = all_partials ? (const i64 *)all_partials : p->pd.table;
-  p->pf.nranks = nranks;
-  p->pf.stride = (i64)(p->pd.nfolds + 2) * p->pd.domain;
-  p->pf.precomputed_choose = 1;
-  p->pf.seq++;
-  probe_finalize_kernel<<<1, 256, 0, ctx->stream>>>(p->pd, p->pf);
-  ctx->launches++;
-  VDL_CUDA(ctx, cudaGetLastError());
-  p->fetched = false;
-  p->finalized = true;
-  return VDL_OK;
+  return p && p->folding ? p->cb.finalize(all_partials, nranks) : VDL_EINVAL;
 }
 
 // finalize != 0: single GPU, results on their way when this returns.  0 (fold mode): leave the complete partial
@@ -990,7 +874,9 @@ extern "C" int vdl_probe_run_ex(vdl_probe *p, int finalize) {
     return vdl_fail(ctx, VDL_ESTALE, "probe: a column was rewritten or dropped after vdl_probe_prepare: prepare again");
   PDesc &d = p->pd;
   p->fetched = false;
-  p->ngroups = p->nselected = -1;
+  p->nselected = -1;
+  p->cb.finalized = false;
+  p->cb.ngroups = -1;
   VDL_CUDA(ctx, cudaMemsetAsync(p->d_ticket, 0, sizeof(unsigned int), ctx->stream));
   if (p->folding) {
     int nb = (int)std::min<i64>(ctx->sm_count, ((i64)(d.nfolds + 2) * d.domain + 255) / 256);
@@ -1007,7 +893,7 @@ extern "C" int vdl_probe_run_ex(vdl_probe *p, int finalize) {
       d.emit_out[e] = (i64 *)ctx->vecs[p->emit_vec[e]].ptr;
     }
   }
-  VDL_CUDA(ctx, cudaEventRecord(p->ev0[p->nlaunch % VDL_EVENT_RING], ctx->stream));
+  VDL_TRY(p->timer.begin(ctx));
   if (d.rows > 0) {
     if (p->jit_kernel) {
       void *args[] = {(void *)&d};
@@ -1017,70 +903,50 @@ extern "C" int vdl_probe_run_ex(vdl_probe *p, int finalize) {
     }
     ctx->launches++;
   }
-  VDL_CUDA(ctx, cudaEventRecord(p->ev1[p->nlaunch % VDL_EVENT_RING], ctx->stream));
-  p->nlaunch++;
-  p->finalized = !p->folding || finalize != 0;
+  VDL_TRY(p->timer.end(ctx));
   if (p->folding && finalize == 2) {       // peer-memory combine: every rank ends with the global result, no host round trip
-    if (p->xd.world < 1) return vdl_fail(ctx, VDL_EINVAL, "probe: peer exchange requested before vdl_probe_set_peers");
-    p->xd.epoch++;
-    int cb = (int)std::min<i64>(ctx->sm_count, (d.domain + 255) / 256);
-    probe_choose_kernel<<<std::max(cb, 1), 256, 0, ctx->stream>>>(d);
-    probe_exchange_kernel<<<1, 256, 0, ctx->stream>>>(p->xd, d.table, ctx->d_errflag);
-    p->pf.table = p->xd.peer[p->xd.rank] + (size_t)(p->xd.epoch & 1) * p->xd.world * p->xd.stride;
-    p->pf.nranks = p->xd.world; p->pf.stride = p->xd.stride; p->pf.precomputed_choose = 1;
-    p->pf.seq++;
-    probe_finalize_kernel<<<1, 256, 0, ctx->stream>>>(d, p->pf);
-    ctx->launches += 3;
+    VDL_TRY(p->cb.next_epoch());
+    int nb = (int)std::min<i64>(ctx->sm_count, (d.domain + 255) / 256);
+    probe_choose_kernel<<<std::max(nb, 1), 256, 0, ctx->stream>>>(d);
+    ctx->launches++;
+    VDL_TRY(p->cb.exchange());
   } else if (p->folding && finalize) {
-    p->pf.table = d.table; p->pf.nranks = 1; p->pf.stride = (i64)(d.nfolds + 2) * d.domain; p->pf.precomputed_choose = 0;
-    p->pf.seq++;
-    probe_finalize_kernel<<<1, 256, 0, ctx->stream>>>(d, p->pf);
+    p->cb.fd.parts = d.table;
+    p->cb.fd.seq++;
+    probe_finalize_kernel<<<1, 256, 0, ctx->stream>>>(d, p->cb.fd);
     ctx->launches++;
   } else if (p->folding) {
-    int cb = (int)std::min<i64>(ctx->sm_count, (d.domain + 255) / 256);
-    probe_choose_kernel<<<std::max(cb, 1), 256, 0, ctx->stream>>>(d);
+    int nb = (int)std::min<i64>(ctx->sm_count, (d.domain + 255) / 256);
+    probe_choose_kernel<<<std::max(nb, 1), 256, 0, ctx->stream>>>(d);
     ctx->launches++;
   } else {
     VDL_CUDA(ctx, cudaMemcpyAsync(p->h_out, p->d_total, sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
   }
   VDL_CUDA(ctx, cudaGetLastError());
+  p->cb.finalized = p->folding && finalize != 0;
   p->ran = true;
   return VDL_OK;
 }
 
+// Emit mode: the survivor count (the fold mode's results: FoldCombine::fetch).
 static int probe_fetch(vdl_probe *p) {
   vdl_ctx *ctx = p->ctx;
   if (!p->ran) return vdl_fail(ctx, VDL_EINVAL, "probe has not run");
-  if (!p->finalized) return vdl_fail(ctx, VDL_EINVAL, "probe ran for an external combine: call vdl_probe_finalize first");
   if (p->fetched) return VDL_OK;
-  if (p->folding) VDL_TRY(wait_published(ctx, p->h_out + (size_t)(p->pd.nfolds + p->pf.npost) * p->pd.domain + 2, p->pf.seq));
-  else VDL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (p->folding) {
-    size_t tail = (size_t)(p->pd.nfolds + p->pf.npost) * p->pd.domain;
-    i64 err = p->h_out[tail + 1];
-    if (err) {
-      cudaMemsetAsync(ctx->d_errflag, 0, sizeof(int), ctx->stream);
-      if (err >= (1 << 20)) return vdl_fail(ctx, VDL_ECUDA, "probe: a peer GPU never delivered its partial table (exchange timed out)");
-      return vdl_fail(ctx, VDL_ERANGE, "probe: %lld rows had a lookup index or group key out of range", (long long)err);
-    }
-    p->ngroups = p->h_out[tail];
-  } else {
-    p->nselected = p->h_out[0];
-    for (int e = 0; e < p->pd.nemits; e++) {
-      Vec &v = ctx->vecs[p->emit_vec[e]];
-      v.len = p->nselected;
-    }
+  VDL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  p->nselected = p->h_out[0];
+  for (int e = 0; e < p->pd.nemits; e++) {
+    Vec &v = ctx->vecs[p->emit_vec[e]];
+    v.len = p->nselected;
   }
   p->fetched = true;
   return VDL_OK;
 }
 
 extern "C" int vdl_probe_result_host(vdl_probe *p, int index, const int64_t **data, int64_t *len) {
-  if (!p || !data || !len || !p->folding || index < 0 || index >= p->pd.nfolds + p->pf.npost) return VDL_EINVAL;
-  VDL_TRY(probe_fetch(p));
-  *data = p->h_out + (size_t)index * p->pd.domain;
-  *len = p->ngroups;
-  return VDL_OK;
+  if (!p || !p->folding) return VDL_EINVAL;
+  if (!p->ran) return vdl_fail(p->ctx, VDL_EINVAL, "probe has not run");
+  return p->cb.result_host(index, data, len);
 }
 
 // Emit mode: the k-th emitted vector (length = number of surviving rows).  Ownership passes to the caller.
@@ -1093,30 +959,10 @@ extern "C" int vdl_probe_emit_take(vdl_probe *p, int k, vdl_vec *out) {
   return VDL_OK;
 }
 
-extern "C" int vdl_probe_last_kernel_ms(vdl_probe *p, float *ms) {
-  if (!p || !ms || !p->ran) return VDL_EINVAL;
-  const int i = (int)((p->nlaunch - 1) % VDL_EVENT_RING);
-  VDL_CUDA(p->ctx, cudaEventSynchronize(p->ev1[i]));
-  VDL_CUDA(p->ctx, cudaEventElapsedTime(ms, p->ev0[i], p->ev1[i]));
-  return VDL_OK;
-}
+extern "C" int vdl_probe_last_kernel_ms(vdl_probe *p, float *ms) { return p && ms && p->ran ? p->timer.last_ms(p->ctx, ms) : VDL_EINVAL; }
 
 extern "C" int vdl_probe_kernel_ms_stats(vdl_probe *p, int n, float *mean_ms, float *min_ms) {
-  if (!p || n < 1 || !p->ran) return VDL_EINVAL;
-  n = (int)std::min<long>(std::min<long>(n, VDL_EVENT_RING), p->nlaunch);
-  double sum = 0;
-  float mn = 1e30f;
-  for (int k = 1; k <= n; k++) {
-    const int i = (int)((p->nlaunch - k) % VDL_EVENT_RING);
-    float ms = 0;
-    VDL_CUDA(p->ctx, cudaEventSynchronize(p->ev1[i]));
-    VDL_CUDA(p->ctx, cudaEventElapsedTime(&ms, p->ev0[i], p->ev1[i]));
-    sum += ms;
-    mn = std::min(mn, ms);
-  }
-  if (mean_ms) *mean_ms = (float)(sum / n);
-  if (min_ms) *min_ms = mn;
-  return VDL_OK;
+  return p && n >= 1 && p->ran ? p->timer.stats(p->ctx, n, mean_ms, min_ms) : VDL_EINVAL;
 }
 
 extern "C" int vdl_probe_destroy(vdl_probe *p) {
@@ -1127,12 +973,12 @@ extern "C" int vdl_probe_destroy(vdl_probe *p) {
   if (p->table) vdl_vec_free(ctx, p->table);
   for (int e = 0; e < VDL_MAX_EMITS; e++)
     if (p->emit_vec[e]) vdl_vec_free(ctx, p->emit_vec[e]);
-  if (p->d_out) cudaFree(p->d_out);
+  p->cb.release();
   if (p->h_out) cudaFreeHost(p->h_out);
   if (p->d_total) cudaFree(p->d_total);
   if (p->d_ticket) cudaFree(p->d_ticket);
   if (p->d_state) cudaFree(p->d_state);
-  for (int i = 0; i < VDL_EVENT_RING; i++) { if (p->ev0[i]) cudaEventDestroy(p->ev0[i]); if (p->ev1[i]) cudaEventDestroy(p->ev1[i]); }
+  p->timer.destroy();
   delete p;
   return VDL_OK;
 }

@@ -45,20 +45,8 @@ struct PDesc {
   int *errflag;
 };
 
-struct PFin {
-  i64 domain;
-  int32_t nfolds, npost;
-  int32_t fold_op[VDL_MAX_AGGS];
-  vdl_post_op post[VDL_MAX_POSTS];
-  const i64 *table;                 // nranks tables back to back (stride int64 each); one = this rank's own
-  i64 stride;
-  int32_t nranks, precomputed_choose;   // precomputed_choose: FoldChoose values already sit in the tables (multi-rank)
-  i64 *out;                         // [(nfolds + npost)][domain] then [ngroups, errors] (+ [seq] in the host mirror)
-  i64 seq;                          // number of this finalize: the last word published to the host mirror
-  i64 *hmirror;
-  const int *errflag;
-};
-
+// Identity of table_update's op on every fold op code: FoldChoose and COUNT rows start at 0.  (acc_identity, which the
+// merge uses, is defined on SUM / MIN / MAX only.)
 __device__ __forceinline__ i64 p_identity(int op) { return op == VDL_FOLD_MIN ? INT64_MAX : (op == VDL_FOLD_MAX ? INT64_MIN : 0); }
 
 __device__ __forceinline__ void table_update(int op, i64 *p, i64 v) {

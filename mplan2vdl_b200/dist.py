@@ -4,13 +4,15 @@ Two ways to combine the per-rank partial aggregate tables:
 * peer memory (default on GPUs): every rank owns a small exchange buffer that all ranks map (CUDA IPC); the LAST
   thread block of each rank's scan kernel stores its table into every peer's buffer over NVLink, publishes an epoch
   flag, waits for the other ranks' flags, merges and finalizes.  One kernel launch per GPU and step, no collective
-  library on the data path (include/vdl_cuda.h, "multi-GPU combine over peer memory").
+  library on the data path (include/vdl_cuda.h, "multi-GPU combine over peer memory").  A probe pass in fold mode
+  combines with the same code in two more launches: probe_choose_kernel, then the one-block fold_exchange_kernel
+  (exchange, merge, finalize), which also serves a scan rank with an empty shard.
 * all-gather (gloo on CPUs in the tests, NCCL if peer mapping is unavailable or VDL_NO_PEER is set), described next.
 
 The fact table is split by contiguous row range (tpch.shard_range), dimension tables are replicated, every rank
 runs the same plan on its shard (vdl_plan_run_local), the per-rank partial aggregate tables -- [accumulators x key
 domain] int64, a few bytes to a few KB -- are all-gathered (NCCL over NVLink on GPUs), and every rank merges them in
-the finalize kernel (vdl_plan_finish): SUM/MIN/MAX accumulators combine by their op, FoldChoose takes the value
+fold_finalize_kernel (vdl_plan_finish): SUM/MIN/MAX accumulators combine by their op, FoldChoose takes the value
 from the rank that holds the smallest first row, empty groups are dropped after the merge.  There is no other
 data-path collective: the scan itself never leaves the GPU that owns the rows.
 

@@ -185,7 +185,7 @@ def test_peer_exchange_times_out_instead_of_hanging(catalog, monkeypatch):
 @pytest.mark.parametrize("world,sf", [(2, 0.01), (4, 0.01), (4, 0.002)])       # (4, 0.002): the last rank's shard is empty
 def test_probe_fold_plans_combine_over_peer_memory(catalog, q, world, sf):
     """FK-join plans whose Folds run on the probe kernel: each rank's partial table crosses to every rank's exchange
-    buffer inside a kernel (probe_exchange_kernel), the finalize merges them -- vdl_plan_run returns the global result on
+    buffer inside a kernel (fold_exchange_kernel), the finalize merges them -- vdl_plan_run returns the global result on
     every rank, no collective, no host round trip.  Emulated ranks (one context + host thread each), three steps."""
     import threading
     from mplan2vdl_b200 import synth
