@@ -67,6 +67,7 @@ foreign import ccall safe "vdl_op_scatter" c_vdl_op_scatter :: Ptr VdlCtx -> Vdl
 foreign import ccall safe "vdl_op_partition" c_vdl_op_partition :: Ptr VdlCtx -> VdlVec -> Int64 -> Int64 -> Int64 -> Ptr VdlVec -> IO CInt
 foreign import ccall safe "vdl_op_fold" c_vdl_op_fold :: Ptr VdlCtx -> CInt -> VdlVec -> VdlVec -> Ptr VdlVec -> IO CInt
 foreign import ccall safe "vdl_op_order" c_vdl_op_order :: Ptr VdlCtx -> CInt -> Ptr VdlVec -> Ptr CInt -> Int64 -> Ptr VdlVec -> IO CInt
+foreign import ccall safe "vdl_op_collate" c_vdl_op_collate :: Ptr VdlCtx -> VdlVec -> VdlVec -> Int64 -> Ptr VdlVec -> IO CInt
 
 -- whole programs: the text Vdl.vdlFromVexps prints
 foreign import ccall safe "vdl_plan_load" c_vdl_plan_load :: Ptr VdlCtx -> CString -> CInt -> Ptr (Ptr VdlPlan) -> IO CInt
@@ -79,6 +80,7 @@ foreign import ccall safe "vdl_plan_output" c_vdl_plan_output :: Ptr VdlPlan -> 
 foreign import ccall safe "vdl_plan_set_typed_outputs" c_vdl_plan_set_typed_outputs :: Ptr VdlPlan -> CInt -> IO CInt
 foreign import ccall safe "vdl_plan_output_typed" c_vdl_plan_output_typed :: Ptr VdlPlan -> CInt -> Ptr CString -> Ptr (Ptr ()) -> Ptr Int64 -> Ptr CInt -> IO CInt
 foreign import ccall safe "vdl_plan_set_order" c_vdl_plan_set_order :: Ptr VdlPlan -> CInt -> Ptr CInt -> Ptr CInt -> Int64 -> IO CInt
+foreign import ccall safe "vdl_plan_set_order_heap" c_vdl_plan_set_order_heap :: Ptr VdlPlan -> CInt -> VdlVec -> Int64 -> IO CInt
 foreign import ccall safe "vdl_plan_destroy" c_vdl_plan_destroy :: Ptr VdlPlan -> IO CInt
 
 -- multi-GPU combine over peer memory (vdl_cuda.h "multi-GPU combine over peer memory"): after vdl_plan_set_peers,

@@ -49,7 +49,8 @@ enum {
 };
 
 /* storage types (reference Types.hs:66-89: SInt32 4 B; SInt64/SDecimal 8 B); VDL_U8: the bytes of a string heap,
- * `Load,<table>.<col>.heap` (Vdl.hs:244-247) -- such a vector can only be the dictionary argument of vdl_op_like */
+ * `Load,<table>.<col>.heap` (Vdl.hs:244-247) -- such a vector can only be the dictionary argument of vdl_op_like or
+ * vdl_op_collate */
 enum { VDL_U8 = 1, VDL_I32 = 4, VDL_I64 = 8 };
 
 /* binary elementwise ops, in the order of `Voodop` (Vdl.hs:110-123) */
@@ -189,6 +190,14 @@ int vdl_op_fold(vdl_ctx *ctx, int fold_op, vdl_vec groups, vdl_vec data, vdl_vec
  * positions 0..limit-1 (limit >= 0; the caller knows n).  Keys of unequal length: VDL_EINVAL. */
 #define VDL_MAX_ORDER_KEYS 8
 int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const int *descending, int64_t limit, vdl_vec *out);
+/* Collation rank of every row's string: the string of row i starts at heap[data[i] - origin] and ends at its NUL.
+ * out[i] (int64) = number of distinct strings in `data` that sort before it.  Strings compare byte by byte as unsigned
+ * char, and a proper prefix sorts first (C strcmp, MonetDB's byte order for UTF-8).  Equal strings at different offsets
+ * get one rank.  An offset outside [0, heap length), or a string with no NUL before the heap ends, raises the context's
+ * range error (VDL_ERANGE at the next check), as vdl_op_like does.  heap must be VDL_U8; data is int32 or int64.
+ * origin is the value heap byte 0 stands for (0: the offsets of a Load,<t>.<c>.heap column); dictionary codes reach
+ * below zero.  Ranking a string column turns it into a key vdl_op_order sorts in collation order. */
+int vdl_op_collate(vdl_ctx *ctx, vdl_vec data, vdl_vec heap, int64_t origin, vdl_vec *out);
 
 /* ---- fused select -> map -> fold -------------------------------------------------------
  * One launch that scans up to VDL_MAX_COLS columns of one table, applies a conjunction of range
@@ -443,6 +452,11 @@ int vdl_plan_output_typed(vdl_plan *p, int i, const char **name, const void **da
  * limited length.  Excludes the sharded tail (a rank holds only a slice of the result): with vdl_plan_tail_enable(p, 1)
  * in force this fails with VDL_EUNSUPPORTED, and so does that call while an order is set. */
 int vdl_plan_set_order(vdl_plan *p, int nkeys, const int *key_output, const int *descending, int64_t limit);
+/* Key k of the order set by vdl_plan_set_order compares by the strings its output's values point to in `heap`
+ * (vdl_op_collate's contract, with `origin`).  heap = 0 clears it.  A later vdl_plan_set_order clears every heap.  The
+ * outputs keep their values (offsets or codes): only the row order follows the strings.  A key index outside the current
+ * order, or a heap that is not VDL_U8: VDL_EINVAL. */
+int vdl_plan_set_order_heap(vdl_plan *p, int key, vdl_vec heap, int64_t origin);
 int vdl_plan_destroy(vdl_plan *p);
 
 /* ---- several GPUs of one box driven from ONE process (SURVEY.md section 8 b, e) ----------------------------------------

@@ -2,7 +2,8 @@
 reference pipeline (eval_query.sh:18-26): read the Voodoo program mplan2vdl printed (stdin or a file), execute it on
 GPU 0 over synthetic TPC-H-shaped tables generated to the reference's bounds metadata, and print the server's JSON
 (resolve.py:8-32) -- or, with --csv, what `resolve.py dictionary.csv` would print from it.  The translator drops ORDER BY
-and LIMIT; --order-by / --limit / --tpch-order apply them on the GPU before the result is copied."""
+and LIMIT; --order-by / --limit / --tpch-order apply them on the GPU before the result is copied, and --collate orders
+string-coded keys by their strings."""
 from __future__ import annotations
 
 import argparse
@@ -11,8 +12,7 @@ import re
 import sys
 import time
 
-# storage types whose values are string-heap offsets or dictionary codes, not a collation order
-STRING_TYPES = ("char", "varchar")
+from .tpch import STRING_TYPES   # storage types whose values are string-heap offsets or dictionary codes
 
 
 def parse_order_by(spec: str) -> list:
@@ -30,9 +30,10 @@ def parse_order_by(spec: str) -> list:
 
 def order_request(args, text: str, cat) -> tuple:
     """(keys, limit) the arguments ask for, checked against the plan's outputs and the catalogue before any device is
-    opened.  Raises ValueError: an unknown or ambiguous name, a key whose output comes from a char / varchar column."""
+    opened.  Raises ValueError: an unknown or ambiguous name, a key whose output comes from a char / varchar column
+    (with --collate: such a key that has no string heap)."""
     from .executor import order_keys
-    from .tpch_queries import ORDER
+    from .tpch_queries import COLLATED_ORDER, ORDER
     keys, limit = parse_order_by(args.order_by), args.limit
     if limit is not None and limit < 0:
         raise ValueError("--limit must be >= 0")
@@ -40,9 +41,11 @@ def order_request(args, text: str, cat) -> tuple:
         if keys or limit is not None:
             raise ValueError("--tpch-order gives the ORDER BY and LIMIT itself: not with --order-by / --limit")
         q = os.path.basename(args.plan).split(".")[0]
-        if q not in ORDER:
-            raise ValueError(f"--tpch-order: no numeric TPC-H ORDER BY for plan {q!r} (known: {', '.join(sorted(ORDER))})")
-        keys, limit = ORDER[q]
+        known = {**COLLATED_ORDER, **ORDER} if args.collate else ORDER
+        if q not in known:
+            what = "TPC-H ORDER BY" if args.collate else "numeric TPC-H ORDER BY"
+            raise ValueError(f"--tpch-order: no {what} for plan {q!r} (known: {', '.join(sorted(known))})")
+        keys, limit = known[q]
     if not keys:
         return keys, limit
     from .tpch import plan_outputs
@@ -51,6 +54,10 @@ def order_request(args, text: str, cat) -> tuple:
         idx, _ = order_keys(names, keys)
     except KeyError as e:
         raise ValueError(e.args[0]) from None
+    if args.collate:
+        from .tpch import collation_recipes
+        collation_recipes(cat, text, keys)          # every string key has a heap, or ValueError
+        return keys, limit
     for i in idx:
         parts = names[i].split("__")
         if len(parts) == 3:
@@ -74,7 +81,10 @@ def main(argv=None) -> int:
     ap.add_argument("--order-by", default="", help="ORDER BY, applied on the GPU: comma-separated output names or aliases "
                     "(the part before '__'), each optionally :asc or :desc; ties keep the plan's own order")
     ap.add_argument("--limit", type=int, default=None, help="LIMIT: only the first N rows (of the ordered result) are copied")
-    ap.add_argument("--tpch-order", action="store_true", help="TPC-H's own ORDER BY / LIMIT of the plan (qNN.vdl) when its keys are numeric")
+    ap.add_argument("--tpch-order", action="store_true", help="TPC-H's own ORDER BY / LIMIT of the plan (qNN.vdl) when its keys are numeric "
+                    "(with --collate: string keys too)")
+    ap.add_argument("--collate", action="store_true", help="order keys whose output comes from a char / varchar column by their "
+                    "strings (byte order), not by their heap offsets / dictionary codes")
     args = ap.parse_args(argv)
     text = sys.stdin.read() if args.plan == "-" else open(args.plan).read()
     text = re.sub(r" ;;.*", "", text)          # the pipeline strips the --metadata suffix with sed (eval_query.sh:20)
@@ -96,7 +106,8 @@ def main(argv=None) -> int:
     tpch.load_synthetic(ctx, cat, tpch.plan_columns(text), args.sf)
     plan = ctx.plan(text, fuse=not args.no_fuse)
     if order or limit is not None:
-        plan.set_order(order, limit)
+        heaps = tpch.collation_heaps(ctx, cat, text, order) if args.collate else None
+        plan.set_order(order, limit, heaps)
     t0 = time.perf_counter()
     out = plan.run()
     us = 1e6 * (time.perf_counter() - t0)

@@ -1181,6 +1181,242 @@ extern "C" int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const 
   return vdl_op_gather(ctx, cand, sorted, out);
 }
 
+// ---------------------------------------------------------------------------------- Collate (string ranks)
+// A char / varchar value is a heap offset (or a dictionary code, origin != 0), and offset order is not string order.
+// vdl_op_collate turns the offsets into dense collation ranks, which vdl_op_order then sorts like any integer key:
+//  - scan: min, max and OR of the in-range values v = data - origin in one pass; a = trailing zeros of the OR, so every
+//    value is a multiple of 2^a and (v >> a) - (min >> a) indexes a slot table over [min, max] (8-aligned heaps: a = 3);
+//  - the slots that occur are flagged and compacted in ascending offset order by FoldSelect: m distinct strings;
+//  - their lengths, then their bytes as big-endian 8-byte words (zero after the NUL, sign bit flipped, so signed int64
+//    order is unsigned byte order and a proper prefix sorts first), 8 words at a time: the last chunk is sorted first
+//    by vdl_op_order (stable), each earlier chunk is written in the order reached so far and sorted again -- no length
+//    cap and no sort code of its own; a word equal across all strings takes no radix pass (a constant key);
+//  - neighbours in the final order are compared over their full bytes, the "differs" flags scanned to dense ranks,
+//    the ranks scattered into the slot table and gathered per row.
+// The m strings are the heap's distinct entries that occur, not the rows: at TPC-H's result sizes a handful to a few
+// hundred thousand.  The rows are read three times (scan, flag, gather) and written once.  The host waits on the device
+// at least four times: for the scan's min / max, FoldSelect's count, the longest string, and once per chunk inside
+// vdl_op_order (twice when a chunk has more than 4 words), which is why small inputs are expected to cost launches and
+// round trips rather than bytes.
+#define COLLATE_CHUNK 8
+
+__device__ __forceinline__ bool collate_in_range(const Operand &data, i64 i, i64 origin, i64 heap_len, i64 *v) {
+  *v = (i64)((u64)op_ld(data, i) - (u64)origin);
+  return (u64)*v < (u64)heap_len;
+}
+
+__global__ void __launch_bounds__(256) collate_scan_kernel(Operand data, i64 n, i64 origin, i64 heap_len, i64 *mm /* min, max, or */,
+                                                           int *errflag) {
+  i64 lo = INT64_MAX, hi = INT64_MIN;
+  unsigned long long bits = 0;
+  int bad = 0;
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+    i64 v;
+    if (!collate_in_range(data, i, origin, heap_len, &v)) { bad++; continue; }
+    lo = v < lo ? v : lo;
+    hi = v > hi ? v : hi;
+    bits |= (unsigned long long)v;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const i64 x = __shfl_xor_sync(0xffffffffu, lo, o), y = __shfl_xor_sync(0xffffffffu, hi, o);
+    lo = x < lo ? x : lo;
+    hi = y > hi ? y : hi;
+    bits |= __shfl_xor_sync(0xffffffffu, bits, o);
+    bad += __shfl_xor_sync(0xffffffffu, bad, o);
+  }
+  if ((threadIdx.x & 31) == 0) {
+    if (lo <= hi) {
+      atomicMin((long long *)&mm[0], (long long)lo);
+      atomicMax((long long *)&mm[1], (long long)hi);
+      atomicOr((unsigned long long *)&mm[2], bits);
+    }
+    if (bad) atomicAdd(errflag, bad);
+  }
+}
+
+__global__ void __launch_bounds__(256) collate_flag_kernel(Operand data, i64 n, i64 origin, i64 heap_len, int a, i64 slot0, int *__restrict__ flag) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+    i64 v;
+    if (collate_in_range(data, i, origin, heap_len, &v)) flag[(v >> a) - slot0] = 1;
+  }
+}
+
+// len[j] of distinct string j (slot sel[j]); a string the heap ends inside counts as ending there, and as a range error
+__global__ void __launch_bounds__(256) collate_len_kernel(const unsigned char *__restrict__ heap, i64 heap_len, const i64 *__restrict__ sel, i64 m,
+                                                          int a, i64 slot0, i64 *__restrict__ len, i64 *maxlen, int *errflag) {
+  i64 mx = 0;
+  for (i64 j = (i64)blockIdx.x * blockDim.x + threadIdx.x; j < m; j += (i64)gridDim.x * blockDim.x) {
+    const i64 off = (slot0 + sel[j]) << a;
+    i64 k = off;
+    while (k < heap_len && heap[k]) k++;
+    if (k == heap_len) atomicAdd(errflag, 1);
+    len[j] = k - off;
+    mx = k - off > mx ? k - off : mx;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const i64 x = __shfl_xor_sync(0xffffffffu, mx, o);
+    mx = x > mx ? x : mx;
+  }
+  if ((threadIdx.x & 31) == 0 && mx) atomicMax((long long *)maxlen, (long long)mx);
+}
+
+// words w0 .. w0 + nw - 1 of the string at position i of the order reached so far (perm; none: ascending offset order)
+struct CollateWords { i64 *w[COLLATE_CHUNK]; };
+__global__ void __launch_bounds__(256) collate_words_kernel(const unsigned char *__restrict__ heap, const i64 *__restrict__ sel, const i64 *__restrict__ len,
+                                                            Operand perm, bool has_perm, i64 m, int a, i64 slot0, int w0, int nw,
+                                                            const __grid_constant__ CollateWords out) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (i64)gridDim.x * blockDim.x) {
+    const i64 j = has_perm ? op_ld(perm, i) : i;
+    const unsigned char *s = heap + ((slot0 + sel[j]) << a);
+    const i64 l = len[j];
+#pragma unroll
+    for (int w = 0; w < COLLATE_CHUNK; w++) {
+      if (w >= nw) break;
+      u64 x = 0;
+      const i64 b0 = (i64)(w0 + w) * 8;
+#pragma unroll
+      for (int b = 0; b < 8; b++) x |= (b0 + b < l ? (u64)s[b0 + b] : 0ull) << (56 - 8 * b);
+      out.w[w][i] = (i64)(x ^ (1ull << 63));
+    }
+  }
+}
+
+// diff[k] = 1 when the k-th and (k+1)-th strings of the final order differ (the exclusive scan of it is the dense rank)
+__global__ void __launch_bounds__(256) collate_diff_kernel(const unsigned char *__restrict__ heap, const i64 *__restrict__ sel, const i64 *__restrict__ len,
+                                                           Operand perm, i64 m, int a, i64 slot0, i64 *__restrict__ diff) {
+  for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < m; k += (i64)gridDim.x * blockDim.x) {
+    i64 d = 0;
+    if (k + 1 < m) {
+      const i64 x = op_ld(perm, k), y = op_ld(perm, k + 1);
+      const i64 l = len[x];
+      d = l != len[y];
+      const unsigned char *s = heap + ((slot0 + sel[x]) << a), *t = heap + ((slot0 + sel[y]) << a);
+      for (i64 b = 0; !d && b < l; b++) d = s[b] != t[b];
+    }
+    diff[k] = d;
+  }
+}
+
+__global__ void __launch_bounds__(256) collate_scatter_kernel(const i64 *__restrict__ rank, const i64 *__restrict__ sel, Operand perm, i64 m,
+                                                              int *__restrict__ table) {
+  for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < m; k += (i64)gridDim.x * blockDim.x) table[sel[op_ld(perm, k)]] = (int)rank[k];
+}
+
+__global__ void __launch_bounds__(256) collate_gather_kernel(Operand data, i64 n, i64 origin, i64 heap_len, int a, i64 slot0, const int *__restrict__ table,
+                                                             i64 *__restrict__ out) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+    i64 v;
+    out[i] = collate_in_range(data, i, origin, heap_len, &v) ? (i64)table[(v >> a) - slot0] : 0;
+  }
+}
+
+extern "C" int vdl_op_collate(vdl_ctx *ctx, vdl_vec data, vdl_vec heap, int64_t origin, vdl_vec *out) {
+  if (!ctx || !out) return VDL_EINVAL;
+  Vec *vd = vec_get(ctx, data), *vh = vec_get_any(ctx, heap);
+  if (!vd || !vh) return VDL_EINVAL;
+  if (vh->dtype != VDL_U8) return vdl_fail(ctx, VDL_EINVAL, "Collate: the heap must be a string heap (a VDL_U8 vector; Load,<table>.<col>.heap)");
+  const i64 n = vd->len, hl = vh->len;
+  const Operand od = operand_of(*vd);
+  const unsigned char *hp = (const unsigned char *)vh->ptr;
+  VDL_TRY(vec_new(ctx, VDL_I64, n, out));
+  ctx->vecs[*out].narrow32 = true;                  // ranks < m < 2^31
+  if (n == 0) return VDL_OK;
+  VDL_CUDA(ctx, cudaSetDevice(ctx->device));
+  i64 *res = (i64 *)ctx->vecs[*out].ptr;
+  VecScope tmp{ctx, {}};
+  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
+  // scan: [min, max, or] of the in-range values, then the longest string
+  vdl_vec mmv;
+  VDL_TRY(vec_new(ctx, VDL_I64, 4, &mmv));
+  tmp.v.push_back(mmv);
+  i64 *mm = (i64 *)ctx->vecs[mmv].ptr;
+  i64 hmm[4] = {INT64_MAX, INT64_MIN, 0, 0};
+  VDL_CUDA(ctx, cudaMemcpyAsync(mm, hmm, sizeof hmm, cudaMemcpyHostToDevice, ctx->stream));
+  collate_scan_kernel<<<grid, 256, 0, ctx->stream>>>(od, n, origin, hl, mm, ctx->d_errflag);
+  ctx->launches++;
+  VDL_TRY(read_scalar(ctx, mm, hmm, 24));
+  if (hmm[0] > hmm[1]) {                            // no offset inside the heap: every row is a range error, rank 0
+    VDL_CUDA(ctx, cudaMemsetAsync(res, 0, (size_t)n * 8, ctx->stream));
+    return VDL_OK;
+  }
+  const int a = hmm[2] ? __builtin_ctzll((u64)hmm[2]) : 0;
+  const i64 slot0 = hmm[0] >> a, slots = (hmm[1] >> a) - slot0 + 1;
+  if (slots > INT32_MAX) return vdl_fail(ctx, VDL_EUNSUPPORTED, "Collate: %lld string slots (at most %d)", (long long)slots, INT32_MAX);
+  // distinct strings: the slots that occur, in ascending offset order
+  vdl_vec tv, sv;
+  VDL_TRY(vec_new(ctx, VDL_I32, slots, &tv));
+  tmp.v.push_back(tv);
+  int *table = (int *)ctx->vecs[tv].ptr;
+  VDL_CUDA(ctx, cudaMemsetAsync(table, 0, (size_t)slots * 4, ctx->stream));
+  collate_flag_kernel<<<grid, 256, 0, ctx->stream>>>(od, n, origin, hl, a, slot0, table);
+  ctx->launches++;
+  VDL_TRY(vdl_op_fold_select(ctx, tv, &sv));
+  tmp.v.push_back(sv);
+  const i64 m = ctx->vecs[sv].len;
+  const i64 *sel = (const i64 *)ctx->vecs[sv].ptr;
+  const int mgrid = (int)std::max<i64>(1, std::min<i64>((m + 255) / 256, (i64)ctx->sm_count * 16));
+  vdl_vec lv;
+  VDL_TRY(vec_new(ctx, VDL_I64, m, &lv));
+  tmp.v.push_back(lv);
+  const i64 *len = (const i64 *)ctx->vecs[lv].ptr;
+  collate_len_kernel<<<mgrid, 256, 0, ctx->stream>>>(hp, hl, sel, m, a, slot0, (i64 *)len, mm + 3, ctx->d_errflag);
+  ctx->launches++;
+  i64 maxlen = 0;
+  VDL_TRY(read_scalar(ctx, mm + 3, &maxlen, 8));
+  if (maxlen == 0) {                                // every string empty: one rank
+    VDL_CUDA(ctx, cudaMemsetAsync(res, 0, (size_t)n * 8, ctx->stream));
+    return VDL_OK;
+  }
+  // sort the m strings, the last chunk of 8 words first
+  const int nwords = (int)((maxlen + 7) / 8), nchunks = (nwords + COLLATE_CHUNK - 1) / COLLATE_CHUNK;
+  CollateWords cw;
+  vdl_vec wv[COLLATE_CHUNK];
+  const int wk = std::min(nwords, COLLATE_CHUNK);
+  for (int w = 0; w < wk; w++) {
+    VDL_TRY(vec_new(ctx, VDL_I64, m, &wv[w]));
+    tmp.v.push_back(wv[w]);
+    cw.w[w] = (i64 *)ctx->vecs[wv[w]].ptr;
+  }
+  vdl_vec perm = 0;
+  for (int c = nchunks - 1; c >= 0; c--) {
+    const int w0 = c * COLLATE_CHUNK, nw = std::min(COLLATE_CHUNK, nwords - w0);
+    const Operand op = perm ? operand_of(ctx->vecs[perm]) : Operand{nullptr, 0, 0, 0};
+    collate_words_kernel<<<mgrid, 256, 0, ctx->stream>>>(hp, sel, len, op, perm != 0, m, a, slot0, w0, nw, cw);
+    ctx->launches++;
+    VDL_CUDA(ctx, cudaGetLastError());
+    vdl_vec p;
+    VDL_TRY(vdl_op_order(ctx, nw, wv, nullptr, -1, &p));
+    tmp.v.push_back(p);
+    if (perm) {                                     // positions of this pass index the order reached so far
+      vdl_vec q;
+      VDL_TRY(vdl_op_gather(ctx, perm, p, &q));
+      tmp.v.push_back(q);
+      for (vdl_vec done : {perm, p}) {              // only the composed order lives on: O(m) however many chunks
+        tmp.v.erase(std::find(tmp.v.begin(), tmp.v.end(), done));
+        vdl_vec_free(ctx, done);
+      }
+      p = q;
+    }
+    perm = p;
+  }
+  // dense ranks: neighbours compared over their full bytes, the "differs" flags scanned
+  vdl_vec dv;
+  VDL_TRY(vec_new(ctx, VDL_I64, (i64)scan_elems(m), &dv));
+  tmp.v.push_back(dv);
+  i64 *diff = (i64 *)ctx->vecs[dv].ptr;
+  const Operand op = operand_of(ctx->vecs[perm]);
+  collate_diff_kernel<<<mgrid, 256, 0, ctx->stream>>>(hp, sel, len, op, m, a, slot0, diff);
+  ctx->launches++;
+  device_exclusive_scan(ctx, diff, m);
+  collate_scatter_kernel<<<mgrid, 256, 0, ctx->stream>>>(diff, sel, op, m, table);
+  collate_gather_kernel<<<grid, 256, 0, ctx->stream>>>(od, n, origin, hl, a, slot0, table, res);
+  ctx->launches += 2;
+  VDL_CUDA(ctx, cudaGetLastError());
+  return VDL_OK;
+}
+
 // ---------------------------------------------------------------------------------- Fold by runs
 #include "vdl_fold_kernel.cuh"
 

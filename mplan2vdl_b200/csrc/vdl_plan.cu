@@ -126,6 +126,9 @@ struct vdl_plan {
   // ORDER BY / LIMIT (vdl_plan_set_order): output indices of the keys, their DESC flags; limit < 0: none
   std::vector<int> order_key, order_desc;
   i64 order_limit = -1;
+  // per key: the string heap its output's values point into (vdl_plan_set_order_heap; 0: compared as integers), origin
+  std::vector<vdl_vec> order_heap;
+  std::vector<i64> order_origin;
   // run state
   std::vector<vdl_vec> val;
   std::vector<vdl_vec> temps;
@@ -1717,7 +1720,7 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
       VDL_TRY(cb->finalize(all_partials ? all_partials[i] : nullptr, nranks));
     }
   }
-  bool ran_ops = false, copies_pending = false;
+  bool ran_ops = false, copies_pending = false, collated = false;
   const bool ordered = !p->order_key.empty() || p->order_limit >= 0;
   std::vector<vdl_vec> dev(p->outputs.size(), 0);    // ordered: the device value of every op-at-a-time output
   // the device -> host copy of op-at-a-time output o, whose value is v
@@ -1806,6 +1809,17 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
         if (e != cudaSuccess) rc = vdl_cuda_fail(ctx, e, "ORDER BY key upload");
       }
     }
+    for (size_t k = 0; k < keys.size() && !rc; k++) {
+      if (!p->order_heap[k]) continue;
+      // a string key: its values (heap offsets or dictionary codes) are replaced by their collation ranks for the order
+      // only; the output itself keeps them
+      vdl_vec r;
+      rc = vdl_op_collate(ctx, keys[k], p->order_heap[k], p->order_origin[k], &r);
+      if (rc) break;
+      p->temps.push_back(r);
+      keys[k] = r;
+      collated = true;
+    }
     vdl_vec perm = 0;
     if (!rc) {
       const i64 limit = keys.empty() ? std::min<i64>(p->order_limit, n) : p->order_limit;
@@ -1839,7 +1853,7 @@ extern "C" int vdl_plan_finish(vdl_plan *p, const void *const *all_partials, int
     if (rc) { if (copies_pending) cudaStreamSynchronize(ctx->copy_stream); free_temps(p); return rc; }
   }
   if (copies_pending) VDL_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));     // before the temporaries are released
-  int rc = ran_ops ? check_errflag(ctx, "plan") : VDL_OK;
+  int rc = ran_ops || collated ? check_errflag(ctx, "plan") : VDL_OK;
   if (!rc && p->tail_on && p->tail_ok) rc = capture_tail_boundary(p);
   p->launches_last += ctx->launches - l0;
   free_temps(p);
@@ -1875,6 +1889,21 @@ extern "C" int vdl_plan_set_order(vdl_plan *p, int nkeys, const int *key_output,
   p->order_desc.assign(nkeys, 0);
   for (int k = 0; k < nkeys && descending; k++) p->order_desc[k] = descending[k] ? 1 : 0;
   p->order_limit = limit < 0 ? -1 : limit;
+  p->order_heap.assign(nkeys, 0);
+  p->order_origin.assign(nkeys, 0);
+  return VDL_OK;
+}
+extern "C" int vdl_plan_set_order_heap(vdl_plan *p, int key, vdl_vec heap, int64_t origin) {
+  if (!p) return VDL_EINVAL;
+  if (key < 0 || key >= (int)p->order_key.size())
+    return vdl_fail(p->ctx, VDL_EINVAL, "ORDER BY key %d out of range (the order has %d keys)", key, (int)p->order_key.size());
+  if (heap) {
+    Vec *vh = vec_get_any(p->ctx, heap);
+    if (!vh) return VDL_EINVAL;
+    if (vh->dtype != VDL_U8) return vdl_fail(p->ctx, VDL_EINVAL, "ORDER BY key %d: vector %d is not a string heap (VDL_U8)", key, (int)heap);
+  }
+  p->order_heap[key] = heap;
+  p->order_origin[key] = heap ? origin : 0;
   return VDL_OK;
 }
 extern "C" int vdl_plan_tail_boundary(vdl_plan *p, int64_t *rec, int cap) {

@@ -170,6 +170,11 @@ class Context:
     def op_fold(self, op: str, groups: int, data: int) -> int:
         return self._out(self.L.vdl_op_fold, _lib.FOLD_OPS.index(op), groups, data)
 
+    def op_collate(self, data: int, heap: int, origin: int = 0) -> int:
+        """Collation rank of every row's string (vdl_op_collate): the string of row i starts at heap byte data[i] - origin;
+        the rank is the number of distinct strings of `data` that sort before it (unsigned byte order, prefixes first)."""
+        return self._out(self.L.vdl_op_collate, data, heap, origin)
+
     def op_order(self, keys, descending=None, limit: int | None = None) -> int:
         """Positions that order the rows of the key vectors (vdl_op_order): lexicographic over `keys`, signed int64, key i
         descending when descending[i]; ties keep row order; the first `limit` of them (None: all)."""
@@ -414,17 +419,32 @@ class Plan:
             names.append(name.value.decode())
         return names
 
-    def set_order(self, keys, limit: int | None = None):
+    def set_order(self, keys, limit: int | None = None, heaps=None):
         """ORDER BY `keys` LIMIT `limit`, applied on the device to every later run before the results are copied
         (vdl_plan_set_order).  keys: [name or (name, descending)], names as `order_keys` resolves them; ([], None) turns
-        the order off.  An unknown or ambiguous name raises before anything is set."""
-        idx, desc = order_keys(self.output_names(), keys)
+        the order off.  heaps: {key name or alias: heap handle or (heap handle, origin)}: that key compares by the strings
+        its values point to in the heap (vdl_plan_set_order_heap, vdl_op_collate), not by the values themselves.  An
+        unknown or ambiguous name, or a heap name that is not among the keys, raises before anything is set."""
+        names = self.output_names()
+        idx, desc = order_keys(names, keys)
+        by_key = []
+        for name, h in (heaps or {}).items():
+            (i,), _ = order_keys(names, [name])
+            if i not in idx:
+                raise KeyError(f"ORDER BY heap {name!r}: {names[i]} is not among the keys {[names[j] for j in idx]}")
+            h, origin = h if isinstance(h, tuple) else (h, 0)
+            by_key.append((idx.index(i), int(h), int(origin)))
         self._set_order(idx, desc, -1 if limit is None else limit)
+        for k, h, origin in by_key:
+            self._set_order_heap(k, h, origin)
 
     def _set_order(self, idx, desc, limit: int):
         k = len(idx)
         self.ctx.check(self.L.vdl_plan_set_order(self.h, k, (C.c_int * max(1, k))(*idx),
                                                  (C.c_int * max(1, k))(*[int(d) for d in desc]), limit))
+
+    def _set_order_heap(self, key: int, heap: int, origin: int):
+        self.ctx.check(self.L.vdl_plan_set_order_heap(self.h, key, heap, origin))
 
     def outputs(self, copy: bool = True) -> dict:
         """{output name: int64 (or, with typed outputs, int32) array}.  copy=False returns views of the library's pinned host

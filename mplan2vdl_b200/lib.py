@@ -143,6 +143,7 @@ SYMBOLS = [
     ("vdl_op_partition", _I, [_P, C.c_int32, _L, _L, _L, C.POINTER(C.c_int32)]),
     ("vdl_op_fold", _I, [_P, _I, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
     ("vdl_op_order", _I, [_P, _I, C.POINTER(C.c_int32), C.POINTER(_I), _L, C.POINTER(C.c_int32)]),
+    ("vdl_op_collate", _I, [_P, C.c_int32, C.c_int32, _L, C.POINTER(C.c_int32)]),
     ("vdl_fused_prepare", _I, [_P, C.POINTER(FusedDesc), C.POINTER(_P)]),
     ("vdl_fused_launch", _I, [_P]),
     ("vdl_fused_partials", _I, [_P, C.POINTER(_P), C.POINTER(_L)]),
@@ -216,6 +217,7 @@ SYMBOLS = [
     ("vdl_plan_set_typed_outputs", _I, [_P, _I]),
     ("vdl_plan_output_typed", _I, [_P, _I, C.POINTER(C.c_char_p), C.POINTER(_P), C.POINTER(_L), C.POINTER(_I)]),
     ("vdl_plan_set_order", _I, [_P, _I, C.POINTER(_I), C.POINTER(_I), _L]),
+    ("vdl_plan_set_order_heap", _I, [_P, _I, C.c_int32, _L]),
     ("vdl_plan_destroy", _I, [_P]),
 ]
 

@@ -200,3 +200,44 @@ def string_offsets(cat: Catalog, qualified: str, rows: int, row_offset: int, see
         z = z ^ (z >> np.uint64(31))
     idx = ((z >> np.uint64(32)) * np.uint64(len(offs)) >> np.uint64(32)).astype(np.int64)      # mulhi on the high word: uniform enough
     return offs[idx]
+
+
+# ------------------------------------------------------------------------------------------ code heaps
+# A char column that is not Loaded with its heap holds dictionary codes drawn at a fixed stride (UNIFORM / SEQ above:
+# l_returnflag 16, 40, 64; o_orderpriority -128, -120, ..., 104).  To order such a column by its strings the executor
+# needs strings behind the codes: the code heap puts a NUL-terminated string of at most stride - 1 bytes at byte
+# code - origin of every code the recipe can draw, origin being the smallest.  A code dictionary.csv names holds that
+# string (cut to fit: '1-URGENT' at stride 8 is '1-URGEN'); every other code a string of the TPC-H filler words, of a
+# length and content fixed by the column's name and the code.  The column's values are untouched.
+def _sm64_np(x):
+    import numpy as np
+    with np.errstate(over="ignore"):
+        z = x + np.uint64(0x9E3779B97F4A7C15)
+        z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        return z ^ (z >> np.uint64(31))
+
+
+def code_heap(cat: Catalog, qualified: str):
+    """(heap bytes as numpy uint8, origin) of the dictionary codes of char column `qualified`: the string of code c starts
+    at heap byte c - origin.  ValueError for a column whose codes are not drawn at a fixed stride."""
+    import numpy as np
+    col = cat.column(qualified)
+    spec = column_spec(cat, qualified, 10)
+    if spec.kind not in (UNIFORM, SEQ) or spec.stride < 2 or col.mtype not in ("char", "varchar"):
+        raise ValueError(f"{qualified}: no code heap (a {col.mtype} column whose synthetic values are not codes at a fixed stride)")
+    count = spec.p0 if spec.kind == UNIFORM else (col.vmax - spec.vmin) // spec.stride + 1
+    width = spec.stride - 1
+    named = {code: s for s, code in cat.dictionary.get(qualified, {}).items()}
+    h = _sm64_np(np.arange(count, dtype=np.uint64) + np.uint64(_fnv1a(qualified + ".codes")))
+    words = [h]
+    for _ in range(3):
+        words.append(_sm64_np(words[-1]))
+    lens = (1 + (h >> np.uint64(32)) % np.uint64(width)).tolist()
+    idx = [(w % np.uint64(len(_FILLER))).tolist() for w in words[1:]]
+    out = []
+    for k in range(count):
+        s = named.get(spec.vmin + k * spec.stride)
+        b = s.encode() if s is not None else " ".join(_FILLER[ix[k]] for ix in idx).encode()[:lens[k]]
+        out.append(b[:width].ljust(spec.stride, b"\0"))
+    return np.frombuffer(b"".join(out), dtype=np.uint8).copy(), spec.vmin

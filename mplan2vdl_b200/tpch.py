@@ -68,3 +68,57 @@ def load_synthetic(ctx, cat: Catalog, columns, sf: float, rank: int = 0, world: 
         ctx.fill_synthetic(q, spec, n, seed, start)
         rows_here[table] = n
     return {"row_base": row_base, "rows": rows_here}
+
+
+# storage types whose values are string-heap offsets or dictionary codes, not a collation order
+STRING_TYPES = ("char", "varchar")
+# prefix of the name a code heap is uploaded under: no plan Loads it (Load names are [\w.]+), so it never meets a Like heap
+CODE_HEAP_PREFIX = "collate:"
+
+
+def collation_recipes(cat: Catalog, text: str, keys) -> dict:
+    """{key name: ("pool", column) or ("codes", column)} for the ORDER BY `keys` of plan `text` whose output comes from a
+    char / varchar column (keys as Plan.set_order takes them; numeric keys are left out).  "pool": the plan Loads the
+    column's heap, so its values are offsets into synth.string_heap (origin 0); "codes": its values are dictionary codes,
+    ordered through synth.code_heap.  Raises KeyError for an unknown name, ValueError for a string key with neither."""
+    from .executor import order_keys
+    names, loads = plan_outputs(text), plan_columns(text)
+    out = {}
+    for key in keys:
+        name = key if isinstance(key, str) else key[0]
+        (i,), _ = order_keys(names, [name])
+        parts = names[i].split("__")
+        if len(parts) != 3:
+            continue
+        q = f"{parts[1]}.{parts[2]}"
+        try:
+            col = cat.column(q)
+        except KeyError:
+            continue
+        if col.mtype not in STRING_TYPES:
+            continue
+        if q + ".heap" in loads:
+            out[name] = ("pool", q)
+            continue
+        spec = synth.column_spec(cat, q, 10)
+        if spec.kind not in (synth.UNIFORM, synth.SEQ) or spec.stride < 2:
+            raise ValueError(f"ORDER BY {names[i]}: no string heap for {q} (neither Loaded with its heap nor codes at a fixed stride)")
+        out[name] = ("codes", q)
+    return out
+
+
+def collation_heaps(ctx, cat: Catalog, text: str, keys) -> dict:
+    """The `heaps` mapping of Plan.set_order for the string keys among `keys` of plan `text` (collation_recipes): a
+    pool heap the plan Loads is looked up (uploaded when absent), a code heap uploaded once under CODE_HEAP_PREFIX +
+    column.  {} when no key is a string."""
+    from .lib import VdlError
+    out = {}
+    for name, (kind, q) in collation_recipes(cat, text, keys).items():
+        hname = q + ".heap" if kind == "pool" else CODE_HEAP_PREFIX + q
+        origin = 0 if kind == "pool" else synth.column_spec(cat, q, 10).vmin       # code_heap's origin: the smallest code
+        try:
+            h = ctx.lookup(hname)
+        except VdlError:                            # the bytes are built only when the heap is not on the device yet
+            h = ctx.upload_column(hname, synth.string_heap(cat, q)[0] if kind == "pool" else synth.code_heap(cat, q)[0])
+        out[name] = (h, origin)
+    return out

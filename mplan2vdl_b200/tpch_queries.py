@@ -125,3 +125,14 @@ ORDER = {
     "q11": ([("value", True)], None),
     "q18": ([("o_totalprice__orders__o_totalprice", True), ("o_orderdate__orders__o_orderdate", False)], 100),
 }
+
+# TPC-H's ORDER BY of the checked-in plans whose sort keys include a string-coded output, applied with the keys' strings
+# (Plan.set_order's heaps, tpch.collation_heaps, --tpch-order --collate): plan -> (keys, limit) as in ORDER.
+COLLATED_ORDER = {
+    "q01": ([("l_returnflag", False), ("l_linestatus", False)], None),
+    "q04": ([("o_orderpriority", False)], None),
+    "q09": ([("nation", False), ("o_year", True)], None),
+    "q12": ([("l_shipmode", False)], None),
+    "q16": ([("supplier_cnt", True), ("p_brand", False), ("p_type", False), ("p_size", False)], None),
+    "q20": ([("s_name", False)], None),
+}
