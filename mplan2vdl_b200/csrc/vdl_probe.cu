@@ -21,7 +21,7 @@
 // No validity vector, inverse index, position vector or gathered copy is ever materialised.
 //
 // Kernel shape: persistent thread blocks take 4096-row tiles in order from a ticket counter and evaluate the
-// predicates stage by stage, compacting the survivors in row order after each (see "staged evaluation" below; the
+// predicates stage by stage, compacting the survivors after each (probe_body in vdl_probe_kernel.cuh; the
 // fact-column loads of a stage are coalesced, and the lineitem->orders index is clustered, so the first dimension
 // gather is nearly sequential too).  Fold mode accumulates into a shared-memory table per block (flushed with
 // global atomics); emit mode places a tile's survivors with a decoupled look-back across tiles (one 64-bit
@@ -90,20 +90,10 @@ __device__ __forceinline__ i64 prod_value(const PDesc &d, const PProd &p, i64 ro
   for (int f = 0; f < p.nfac; f++) v = (i64)((u64)v * (u64)term_value(d, p.f[f], row, ok));
   return v;
 }
-__device__ __forceinline__ bool row_passes(const PDesc &d, i64 row, bool &ok) {
-  for (int q = 0; q < d.npreds; q++) {
-    if (!pred_holds(d, d.pred[q], row, ok) || !ok) return false;
-  }
-  return true;
-}
 
-// ---- staged evaluation ---------------------------------------------------------------------------------------------
-// A tile goes through the predicates one STAGE at a time; after every stage the surviving rows are compacted (in row
-// order) into a shared-memory queue, so the next stage runs with full warps on survivors only and its lookups are
-// independent loads of different rows (memory-level parallelism instead of divergent lanes waiting on a long
-// dependent chain).  A range predicate on a lookup chain of depth <= 4 -- every predicate the FK-join lowering
-// produces -- runs as straight-line code: the chain (pointers, lengths, widths) is read from the descriptor once per
-// tile and stage, not per row.
+// ---- the interpreter's evaluator (probe_body: vdl_probe_kernel.cuh) -----------------------------------------------------
+// A range predicate on a lookup chain of depth <= 4 -- every predicate the FK-join lowering produces -- runs as
+// straight-line code: the chain (pointers, lengths, widths) is read from the descriptor once per tile and stage, not per row.
 struct StageRegs { const void *ptr[4]; i64 len[4]; int w4mask, shr, depth; i64 a, b, lo; u64 span; };
 
 // S.ptr[0] is the leaf's own column (the LAST load), S.ptr[D-1] the fact column (the first): all indexing static.
@@ -127,194 +117,76 @@ __device__ __forceinline__ bool chain_test(const StageRegs &S, i64 row, i64 row_
 #define P_SUB 4      // rows per thread and round of a stage (8 was best while every round ended in two barriers)
 #endif
 
-__global__ void __launch_bounds__(P_THREADS, P_BLOCKS) probe_kernel(const __grid_constant__ PDesc d) {
-  extern __shared__ __align__(16) unsigned char psm[];
-  __shared__ uint16_t queue[2][P_TILE];
-  __shared__ int s_cnt[3];                        // survivors appended by stage q: s_cnt[(q + 1) % 3]
-  __shared__ unsigned int s_bits[P_TILE / 32];    // emit mode: the tile's survivors as a bitmap, to put them back in row order
-  __shared__ int wsum[P_THREADS / 32];
-  __shared__ i64 s_off;
-  __shared__ unsigned int s_tile;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const bool folding = d.nemits == 0;
-  const int nacc = d.nfolds + 2;
-  i64 *stab = (i64 *)psm;                         // [nacc][domain] when smem_table
-  if (folding && d.smem_table) {
-    for (i64 i = tid; i < (i64)nacc * d.domain; i += P_THREADS) {
-      int j = (int)(i / d.domain);
-      stab[i] = j < d.nfolds ? p_identity(d.fold_op[j]) : (j == d.nfolds ? 0 : INT64_MAX);
-    }
+struct ProbeInterp {
+  static constexpr int SUB = P_SUB;
+  __device__ __forceinline__ static int npreds(const PDesc &d) { return d.npreds; }
+  __device__ __forceinline__ static int nfolds(const PDesc &d) { return d.nfolds; }
+  __device__ __forceinline__ static int nemits(const PDesc &d) { return d.nemits; }
+  template <class F> __device__ __forceinline__ static void stages(const PDesc &d, const int &n_in, F &&run_stage) {
+    for (int q = 0; q < d.npreds && n_in > 0; q++) run_stage(q);
   }
-  __syncthreads();
-  i64 *tab = (folding && d.smem_table) ? stab : d.table;
-
-  for (;;) {
-    if (tid == 0) { s_tile = atomicAdd(d.ticket, 1u); s_cnt[1] = 0; }
-    __syncthreads();
-    const i64 tile = s_tile;
-    if (tile >= d.ntiles) break;
-    const i64 base = tile * P_TILE;
-    if (d.npf) {
-      const i64 b2 = base + (i64)d.pf_dist * P_TILE;
-      const i64 n2 = min((i64)P_TILE, d.rows - b2);
-      for (int c = 0; c < d.npf && n2 > 0; c++) {
-        const unsigned char *p0 = d.pf_ptr[c] + (b2 << d.pf_shift[c]);
-        const i64 bytes = n2 << d.pf_shift[c];
-        for (i64 o = (i64)tid * 128; o < bytes; o += P_THREADS * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(p0 + o));
+  // the chain of stage q's term, if it has the fast form
+  __device__ __forceinline__ static StageRegs stage(const PDesc &d, int q) {
+    const PPred &P = d.pred[q];
+    StageRegs S;
+    S.depth = -1;
+    if (P.kind == 0 && P.nmore == 0 && P.t.leaf != -1) {
+      int l = P.t.leaf, n = 0;
+      S.w4mask = 0;
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        S.ptr[k] = nullptr; S.len[k] = 0;
+        if (l >= 0) {
+          const PLeaf &L = d.leaf[l];
+          S.ptr[k] = L.ptr; S.len[k] = L.len; S.w4mask |= (L.w4 ? 1 : 0) << k;
+          l = L.parent; n = k + 1;
+        }
       }
+      if (l < 0) { S.depth = n; S.shr = P.t.shr; S.a = P.t.a; S.b = P.t.b; S.lo = P.lo; S.span = P.span; if (P.t.a == 0 && P.t.b == 1) S.depth += 8; }   // +8: plain
     }
-    bool ok = true;
-    int n_in = (int)min((i64)P_TILE, d.rows - base);      // stage input: all rows of the tile, then the previous stage's survivors
-    int cur = 0;
-    for (int q = 0; q < d.npreds && n_in > 0; q++) {
-      const PPred &P = d.pred[q];
-      // the chain of this stage's term, if it has the fast form
-      StageRegs S;
-      S.depth = -1;
-      if (P.kind == 0 && P.nmore == 0 && P.t.leaf != -1) {
-        int l = P.t.leaf, n = 0;
-        S.w4mask = 0;
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-          S.ptr[k] = nullptr; S.len[k] = 0;
-          if (l >= 0) {
-            const PLeaf &L = d.leaf[l];
-            S.ptr[k] = L.ptr; S.len[k] = L.len; S.w4mask |= (L.w4 ? 1 : 0) << k;
-            l = L.parent; n = k + 1;
-          }
-        }
-        if (l < 0) { S.depth = n; S.shr = P.t.shr; S.a = P.t.a; S.b = P.t.b; S.lo = P.lo; S.span = P.span; if (P.t.a == 0 && P.t.b == 1) S.depth += 8; }   // +8: plain
-      }
-      for (int j0 = 0; j0 < n_in; j0 += P_SUB * P_THREADS) {
-        bool f[P_SUB];
-        int r[P_SUB];
-#pragma unroll
-        for (int k = 0; k < P_SUB; k++) {
-          const int j = j0 + k * P_THREADS + tid;
-          r[k] = j < n_in ? (q == 0 ? j : (int)queue[cur][j]) : -1;
-        }
+    return S;
+  }
+  __device__ __forceinline__ static void round(const PDesc &d, int q, const StageRegs &S, i64 base, const int (&r)[SUB], bool (&f)[SUB], bool &ok) {
 #define STAGE_CASE(DEPTH, PL)                                                                                                   \
-  _Pragma("unroll") for (int k = 0; k < P_SUB; k++) f[k] = r[k] >= 0 && chain_test<DEPTH, PL>(S, base + r[k], d.row_base, ok)
-        if (S.depth == 8 + 2) { STAGE_CASE(2, true);
-        } else if (S.depth == 8 + 1) { STAGE_CASE(1, true);
-        } else if (S.depth == 8 + 3) { STAGE_CASE(3, true);
-        } else if (S.depth == 8 + 4) { STAGE_CASE(4, true);
-        } else if (S.depth == 1) { STAGE_CASE(1, false);
-        } else if (S.depth == 2) { STAGE_CASE(2, false);
-        } else if (S.depth == 3) { STAGE_CASE(3, false);
-        } else if (S.depth == 4) { STAGE_CASE(4, false);
-        } else if (S.depth == 0 || S.depth == 8) { STAGE_CASE(0, false);
-        } else {      // generic: constants, column-vs-column comparisons, range sets, deeper chains
+  _Pragma("unroll") for (int k = 0; k < SUB; k++) f[k] = r[k] >= 0 && chain_test<DEPTH, PL>(S, base + r[k], d.row_base, ok)
+    if (S.depth == 8 + 2) { STAGE_CASE(2, true);
+    } else if (S.depth == 8 + 1) { STAGE_CASE(1, true);
+    } else if (S.depth == 8 + 3) { STAGE_CASE(3, true);
+    } else if (S.depth == 8 + 4) { STAGE_CASE(4, true);
+    } else if (S.depth == 1) { STAGE_CASE(1, false);
+    } else if (S.depth == 2) { STAGE_CASE(2, false);
+    } else if (S.depth == 3) { STAGE_CASE(3, false);
+    } else if (S.depth == 4) { STAGE_CASE(4, false);
+    } else if (S.depth == 0 || S.depth == 8) { STAGE_CASE(0, false);
+    } else {      // generic: constants, column-vs-column comparisons, range sets, deeper chains
 #pragma unroll 1
-          for (int k = 0; k < P_SUB; k++) f[k] = r[k] >= 0 && pred_holds(d, P, base + r[k], ok);
-        }
-        // append this round's survivors to the next stage's queue.  Queue order is irrelevant to a stage (and to a
-        // fold); emit mode restores row order once, at the end.  One shared atomic per warp and round, no barrier.
-        unsigned m[P_SUB];
-        int wtotal = 0;
-#pragma unroll
-        for (int k = 0; k < P_SUB; k++) { m[k] = __ballot_sync(0xffffffffu, f[k]); wtotal += __popc(m[k]); }
-        if (wtotal) {
-          int at = 0;
-          if (lane == 0) at = atomicAdd(&s_cnt[(q + 1) % 3], wtotal);
-          at = __shfl_sync(0xffffffffu, at, 0);
-#pragma unroll
-          for (int k = 0; k < P_SUB; k++) {
-            if (f[k]) queue[cur ^ 1][at + __popc(m[k] & ((1u << lane) - 1))] = (uint16_t)r[k];
-            at += __popc(m[k]);
-          }
-        }
-      }
-      // the counter two stages ahead is idle: every thread read it (as its n_in) before the previous stage's barrier
-      if (tid == 0) s_cnt[(q + 2) % 3] = 0;
-      __syncthreads();
-      n_in = s_cnt[(q + 1) % 3];
-      cur ^= 1;
-    }
-    const bool implicit = d.npreds == 0;            // no predicate at all: every row of the tile survives
-    // ---- survivors: fold into the table, or emit in order
-    if (folding) {
-      for (int j = tid; j < n_in; j += P_THREADS) {
-        const i64 row = base + (implicit ? j : (int)queue[cur][j]);
-        i64 key = 0;
-        for (int q = 0; q < d.nkeys; q++) key |= (i64)((u64)term_value(d, d.key[q], row, ok) << d.key_shl[q]);
-        key &= d.key_mask;
-        if ((u64)key >= (u64)d.domain) { ok = false; continue; }
-        for (int j2 = 0; j2 < d.nfolds; j2++) {
-          const int op = d.fold_op[j2];
-          if (op == VDL_FOLD_CHOOSE || op == VDL_FOLD_COUNT) continue;     // from the first row / the row count
-          table_update(op, tab + (size_t)j2 * d.domain + key, prod_value(d, d.fold[j2], row, ok));
-        }
-        atomicAdd((unsigned long long *)(tab + (size_t)d.nfolds * d.domain + key), 1ull);
-        atomicMin((long long *)(tab + (size_t)(d.nfolds + 1) * d.domain + key), (long long)(d.row_base + row));
-      }
-    } else {
-      if (!implicit) {
-        // survivors back into row order: bitmap of the tile, one 32-row word per thread, block scan of the word counts
-        static_assert(P_TILE / 32 == P_THREADS, "one bitmap word per thread");
-        s_bits[tid] = 0;
-        __syncthreads();
-        for (int j = tid; j < n_in; j += P_THREADS) { const unsigned rr = queue[cur][j]; atomicOr(&s_bits[rr >> 5], 1u << (rr & 31)); }
-        __syncthreads();
-        unsigned w = s_bits[tid];
-        const int c = __popc(w);
-        int incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int at = incl - c;
-        for (int ww = 0; ww < warp; ww++) at += wsum[ww];
-        while (w) { const int b = __ffs(w) - 1; w &= w - 1; queue[cur ^ 1][at++] = (uint16_t)(tid * 32 + b); }
-        cur ^= 1;
-        __syncthreads();
-      }
-      // tile offset by decoupled look-back over the tiles before this one
-      if (tid == 0) {
-        const unsigned long long T = (unsigned long long)n_in;
-        i64 excl = 0;
-        if (tile == 0) {
-          atomicExch(d.tile_state, (2ull << 62) | T);
-        } else {
-          atomicExch(d.tile_state + tile, (1ull << 62) | T);
-          for (i64 j = tile - 1;; j--) {
-            unsigned long long st;
-            do { st = *((volatile unsigned long long *)(d.tile_state + j)); } while ((st >> 62) == 0);
-            excl += (i64)(st & ((1ull << 62) - 1));
-            if ((st >> 62) == 2) break;
-          }
-          atomicExch(d.tile_state + tile, (2ull << 62) | (unsigned long long)(excl + (i64)T));
-        }
-        s_off = excl;
-        if (tile == d.ntiles - 1) *d.total = excl + (i64)T;
-      }
-      __syncthreads();
-      const i64 off = s_off;
-      for (int j = tid; j < n_in; j += P_THREADS) {
-        const i64 row = base + (implicit ? j : (int)queue[cur][j]);
-        for (int e = 0; e < d.nemits; e++) d.emit_out[e][off + j] = prod_value(d, d.emit[e], row, ok);
-      }
-    }
-    if (!ok) atomicAdd(d.errflag, 1);
-    __syncthreads();
-  }
-  if (folding && d.smem_table) {
-    __syncthreads();
-    for (i64 i = tid; i < (i64)nacc * d.domain; i += P_THREADS) {
-      int j = (int)(i / d.domain);
-      const i64 v = stab[i];
-      if (j < d.nfolds) { if (v != p_identity(d.fold_op[j])) table_update(d.fold_op[j], d.table + i, v); }
-      else if (j == d.nfolds) { if (v) atomicAdd((unsigned long long *)(d.table + i), (unsigned long long)v); }
-      else if (v != INT64_MAX) atomicMin((long long *)(d.table + i), (long long)v);
+      for (int k = 0; k < SUB; k++) f[k] = r[k] >= 0 && pred_holds(d, d.pred[q], base + r[k], ok);
     }
   }
-}
+  __device__ __forceinline__ static void fold_row(const PDesc &d, i64 row, i64 *tab, bool &ok) {
+    i64 key = 0;
+    for (int q = 0; q < d.nkeys; q++) key |= (i64)((u64)term_value(d, d.key[q], row, ok) << d.key_shl[q]);
+    key &= d.key_mask;
+    if ((u64)key >= (u64)d.domain) { ok = false; return; }
+    for (int j = 0; j < d.nfolds; j++) {
+      const int op = d.fold_op[j];
+      if (op == VDL_FOLD_CHOOSE || op == VDL_FOLD_COUNT) continue;     // from the first row / the row count
+      table_update(op, tab + (size_t)j * d.domain + key, prod_value(d, d.fold[j], row, ok));
+    }
+    atomicAdd((unsigned long long *)(tab + (size_t)d.nfolds * d.domain + key), 1ull);
+    atomicMin((long long *)(tab + (size_t)(d.nfolds + 1) * d.domain + key), (long long)(d.row_base + row));
+  }
+  __device__ __forceinline__ static void emit_row(const PDesc &d, i64 row, i64 at, bool &ok) {
+    for (int e = 0; e < d.nemits; e++) d.emit_out[e][at] = prod_value(d, d.emit[e], row, ok);
+  }
+};
+
+__global__ void __launch_bounds__(P_THREADS, P_BLOCKS) probe_kernel(const __grid_constant__ PDesc d) { probe_body<ProbeInterp>(d, threadIdx.x); }
 
 __global__ void probe_init_kernel(const __grid_constant__ PDesc d) {
   const i64 n = (i64)(d.nfolds + 2) * d.domain;
   for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
-    int j = (int)(i / d.domain);
-    d.table[i] = j < d.nfolds ? p_identity(d.fold_op[j]) : (j == d.nfolds ? 0 : INT64_MAX);
+    d.table[i] = table_identity(d, d.nfolds, (int)(i / d.domain));
   }
 }
 
@@ -354,9 +226,10 @@ __global__ void __launch_bounds__(256, 1) probe_finalize_kernel(const __grid_con
 // them loads (profiles/r01e_q05_sf10_dominant_kernel.txt).  For tables of a few hundred thousand rows and up the descriptor
 // is instead PRINTED as CUDA C: one straight-line function per predicate stage (typed loads along the lookup chain, bounds
 // and constants as literals, out-of-range lookups turned into a flag and a clamped index so that no branch separates the
-// loads), one for the fold / emit of a surviving row, and the same tile loop around them.  The P_SUB rows a thread handles
-// per round are independent straight-line chains, so their loads overlap (memory-level parallelism instead of one
-// dependent chain per warp).  Same results as the interpreter (tests/test_gpu_probe.py and the fuzz plans run both).
+// loads), one each for the fold and the emit of a surviving row, and an evaluator struct that hands them to probe_body,
+// the tile loop probe_kernel instantiates too.  The 8 rows a thread handles per round are independent straight-line
+// chains, so their loads overlap (memory-level parallelism instead of one dependent chain per warp).  Same results as the
+// interpreter (tests/test_gpu_probe.py and the fuzz plans run both).
 struct ProbeGen {
   const PDesc &d;
   std::string body;                 // statements of the function being generated
@@ -422,161 +295,43 @@ struct ProbeGen {
   }
 };
 
-static const char *PROBE_JIT_TAIL = R"SKEL(
-#define STAGE_LOOP(Q, FN)                                                                                          \
-  if (n_in > 0) {                                                                                                  \
-    for (int j0 = 0; j0 < n_in; j0 += P_SUB * P_THREADS) {                                                         \
-      bool f[P_SUB];                                                                                               \
-      int r[P_SUB];                                                                                                \
-      _Pragma("unroll") for (int k = 0; k < P_SUB; k++) {                                                          \
-        const int j = j0 + k * P_THREADS + tid;                                                                    \
-        r[k] = j < n_in ? ((Q) == 0 ? j : (int)queue[cur][j]) : -1;                                                \
-      }                                                                                                            \
-      /* every slot evaluates a row (its own, or the tile's row 0 as a stand-in): straight-line, loads overlap */ \
-      _Pragma("unroll") for (int k = 0; k < P_SUB; k++) {                                                          \
-        bool okk = true;                                                                                           \
-        const bool pass = FN(d, base + (r[k] >= 0 ? r[k] : 0), okk);                                               \
-        f[k] = r[k] >= 0 && pass && okk;                                                                           \
-        if (r[k] >= 0 && !okk) ok = false;                                                                         \
-      }                                                                                                            \
-      unsigned m[P_SUB];                                                                                           \
-      int wtotal = 0;                                                                                              \
-      _Pragma("unroll") for (int k = 0; k < P_SUB; k++) { m[k] = __ballot_sync(0xffffffffu, f[k]); wtotal += __popc(m[k]); } \
-      if (wtotal) {                                                                                                \
-        int at = 0;                                                                                                \
-        if (lane == 0) at = atomicAdd(&s_cnt[((Q) + 1) % 3], wtotal);                                              \
-        at = __shfl_sync(0xffffffffu, at, 0);                                                                      \
-        _Pragma("unroll") for (int k = 0; k < P_SUB; k++) {                                                        \
-          if (f[k]) queue[cur ^ 1][at + __popc(m[k] & ((1u << lane) - 1))] = (uint16_t)r[k];                       \
-          at += __popc(m[k]);                                                                                      \
-        }                                                                                                          \
-      }                                                                                                            \
-    }                                                                                                              \
-  }                                                                                                                \
-  if (tid == 0) s_cnt[((Q) + 2) % 3] = 0;                                                                          \
-  __syncthreads();                                                                                                 \
-  n_in = s_cnt[((Q) + 1) % 3];                                                                                     \
-  cur ^= 1;
-
-extern "C" __global__ void __launch_bounds__(P_THREADS, P_JIT_BLOCKS) vdl_probe_jit(const __grid_constant__ PDesc d) {
-  extern __shared__ __align__(16) unsigned char psm[];
-  __shared__ uint16_t queue[2][P_TILE];
-  __shared__ int s_cnt[3];
-  __shared__ unsigned int s_bits[P_TILE / 32];
-  __shared__ int wsum[P_THREADS / 32];
-  __shared__ i64 s_off;
-  __shared__ unsigned int s_tile;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  constexpr bool folding = P_NEMITS == 0;
-  constexpr int nacc = P_NFOLDS + 2;
-  i64 *stab = (i64 *)psm;
-  if (folding && d.smem_table) {
-    for (i64 i = tid; i < (i64)nacc * d.domain; i += P_THREADS) {
-      int j = (int)(i / d.domain);
-      stab[i] = j < P_NFOLDS ? p_identity(d.fold_op[j]) : (j == P_NFOLDS ? 0 : INT64_MAX);
-    }
-  }
-  __syncthreads();
-  i64 *tab = (folding && d.smem_table) ? stab : d.table;
-  for (;;) {
-    if (tid == 0) { s_tile = atomicAdd(d.ticket, 1u); s_cnt[1] = 0; }
-    __syncthreads();
-    const i64 tile = s_tile;
-    if (tile >= d.ntiles) break;
-    const i64 base = tile * P_TILE;
-    if (d.npf) {
-      const i64 b2 = base + (i64)d.pf_dist * P_TILE;
-      const i64 n2 = min((i64)P_TILE, d.rows - b2);
-      for (int c = 0; c < d.npf && n2 > 0; c++) {
-        const unsigned char *p0 = d.pf_ptr[c] + (b2 << d.pf_shift[c]);
-        const i64 bytes = n2 << d.pf_shift[c];
-        for (i64 o = (i64)tid * 128; o < bytes; o += P_THREADS * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(p0 + o));
-      }
-    }
-    bool ok = true;
-    int n_in = (int)min((i64)P_TILE, d.rows - base);
-    int cur = 0;
-    P_STAGES
-    constexpr bool implicit = P_NPREDS == 0;
-    if (folding) {
-      for (int j = tid; j < n_in; j += P_THREADS) probe_fold_row(d, base + (implicit ? j : (int)queue[cur][j]), tab, ok);
-    } else {
-      if (!implicit) {
-        s_bits[tid] = 0;
-        __syncthreads();
-        for (int j = tid; j < n_in; j += P_THREADS) { const unsigned rr = queue[cur][j]; atomicOr(&s_bits[rr >> 5], 1u << (rr & 31)); }
-        __syncthreads();
-        unsigned w = s_bits[tid];
-        const int c = __popc(w);
-        int incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int at = incl - c;
-        for (int ww = 0; ww < warp; ww++) at += wsum[ww];
-        while (w) { const int b = __ffs(w) - 1; w &= w - 1; queue[cur ^ 1][at++] = (uint16_t)(tid * 32 + b); }
-        cur ^= 1;
-        __syncthreads();
-      }
-      if (tid == 0) {
-        const unsigned long long T = (unsigned long long)n_in;
-        i64 excl = 0;
-        if (tile == 0) {
-          atomicExch(d.tile_state, (2ull << 62) | T);
-        } else {
-          atomicExch(d.tile_state + tile, (1ull << 62) | T);
-          for (i64 j = tile - 1;; j--) {
-            unsigned long long st;
-            do { st = *((volatile unsigned long long *)(d.tile_state + j)); } while ((st >> 62) == 0);
-            excl += (i64)(st & ((1ull << 62) - 1));
-            if ((st >> 62) == 2) break;
-          }
-          atomicExch(d.tile_state + tile, (2ull << 62) | (unsigned long long)(excl + (i64)T));
-        }
-        s_off = excl;
-        if (tile == d.ntiles - 1) *d.total = excl + (i64)T;
-      }
-      __syncthreads();
-      const i64 off = s_off;
-      for (int j = tid; j < n_in; j += P_THREADS) probe_emit_row(d, base + (implicit ? j : (int)queue[cur][j]), off + j, ok);
-    }
-    if (!ok) atomicAdd(d.errflag, 1);
-    __syncthreads();
-  }
-  if (folding && d.smem_table) {
-    __syncthreads();
-    for (i64 i = tid; i < (i64)nacc * d.domain; i += P_THREADS) {
-      int j = (int)(i / d.domain);
-      const i64 v = stab[i];
-      if (j < P_NFOLDS) { if (v != p_identity(d.fold_op[j])) table_update(d.fold_op[j], d.table + i, v); }
-      else if (j == P_NFOLDS) { if (v) atomicAdd((unsigned long long *)(d.table + i), (unsigned long long)v); }
-      else if (v != INT64_MAX) atomicMin((long long *)(d.table + i), (long long)v);
-    }
-  }
-}
-)SKEL";
-
 static std::string probe_jit_source(const PDesc &d, int p_sub, int blocks) {
   ProbeGen g(d);
   char b[256];
-  snprintf(b, sizeof b, "#include \"vdl_probe_kernel.cuh\"\n#define P_SUB %d\n#define P_JIT_BLOCKS %d\n#define P_NPREDS %d\n#define P_NFOLDS %d\n#define P_NEMITS %d\n",
-           p_sub, blocks, d.npreds, d.nfolds, d.nemits);
-  std::string s = b, stages;
+  std::string s = "#include \"vdl_probe_kernel.cuh\"\n", stage_of_q, calls;
   for (int q = 0; q < d.npreds; q++) {
     g.reset();
     const std::string e = g.pred(d.pred[q]);
     snprintf(b, sizeof b, "__device__ __forceinline__ bool probe_stage_%d(const PDesc &d, const i64 row, bool &ok) {\n", q);
     s += b + g.body + "  return " + e + ";\n}\n";
-    snprintf(b, sizeof b, "STAGE_LOOP(%d, probe_stage_%d) ", q, q);
-    stages += b;
+    snprintf(b, sizeof b, "q == %d ? probe_stage_%d(d, row, okk) : ", q, q);
+    stage_of_q += b;
+    snprintf(b, sizeof b, " run_stage(%d);", q);
+    calls += b;
   }
+  // probe_body's evaluator.  Every stage is run, with a literal q, also when no row survived an earlier one.
+  snprintf(b, sizeof b, "struct ProbeJit {\n  static constexpr int SUB = %d;\n", p_sub);
+  s += b;
+  snprintf(b, sizeof b, "  __device__ static int npreds(const PDesc &) { return %d; }\n  __device__ static int nfolds(const PDesc &) { return %d; }\n"
+                        "  __device__ static int nemits(const PDesc &) { return %d; }\n", d.npreds, d.nfolds, d.nemits);
+  s += b;
+  s += "  template <class F> __device__ __forceinline__ static void stages(const PDesc &, const int &, F &&run_stage) {" + calls + " }\n"
+       "  __device__ static int stage(const PDesc &, int) { return 0; }\n"
+       "  __device__ __forceinline__ static void round(const PDesc &d, int q, int, i64 base, const int (&r)[SUB], bool (&f)[SUB], bool &ok) {\n"
+       "#pragma unroll\n"
+       "    for (int k = 0; k < SUB; k++) {   // every slot evaluates a row (its own, or the tile's row 0 as a stand-in): straight-line, loads overlap\n"
+       "      bool okk = true;\n"
+       "      const i64 row = base + (r[k] >= 0 ? r[k] : 0);\n"
+       "      const bool pass = " + stage_of_q + "false;\n"
+       "      f[k] = r[k] >= 0 && pass && okk;\n"
+       "      if (r[k] >= 0 && !okk) ok = false;\n"
+       "    }\n"
+       "  }\n";
   // fold of one surviving row (fold mode) / its emitted expressions (emit mode)
   g.reset();
-  s += "__device__ __forceinline__ void probe_fold_row(const PDesc &d, const i64 row, i64 *tab, bool &ok) {\n";
+  s += "  __device__ __forceinline__ static void fold_row(const PDesc &d, const i64 row, i64 *tab, bool &ok) {\n";
   if (d.nemits == 0) {
     std::string keyexpr = "  i64 key = 0;\n";
-    std::string pre;
     for (int q = 0; q < d.nkeys; q++) {
       const std::string t = g.term(d.key[q]);
       keyexpr += "  key |= (i64)((u64)" + t + " << " + std::to_string(d.key_shl[q]) + ");\n";
@@ -592,26 +347,23 @@ static std::string probe_jit_source(const PDesc &d, int p_sub, int blocks) {
              d.nfolds, d.nfolds + 1);
     s += b;
   }
-  s += "}\n";
+  s += "  }\n";
   g.reset();
-  s += "__device__ __forceinline__ void probe_emit_row(const PDesc &d, const i64 row, const i64 at, bool &ok) {\n";
+  s += "  __device__ __forceinline__ static void emit_row(const PDesc &d, const i64 row, const i64 at, bool &ok) {\n";
   {
     std::string st;
     for (int e = 0; e < d.nemits; e++) { snprintf(b, sizeof b, "  d.emit_out[%d][at] = ", e); st += b + g.product(d.emit[e]) + ";\n"; }
     s += g.body + st;
   }
-  s += "}\n#define P_STAGES " + stages + "\n";
-  return s + PROBE_JIT_TAIL;
+  snprintf(b, sizeof b, "  }\n};\nextern \"C\" __global__ void __launch_bounds__(P_THREADS, %d) vdl_probe_jit(const __grid_constant__ PDesc d) { probe_body<ProbeJit>(d, threadIdx.x); }\n", blocks);
+  return s + b;
 }
 
-static cudaKernel_t probe_jit_compile(vdl_ctx *ctx, const PDesc &d, size_t smem, bool *ok, std::string *log) {
-  int p_sub = 8, blocks = 8;       // measured on B200 (Q5 / Q3 / Q12 / Q19 SF10): 8 rows per thread and round, 8 blocks x 64 registers
-  if (const char *e = getenv("VDL_PROBE_JIT_SUB")) p_sub = std::max(1, std::min(16, atoi(e)));
-  if (const char *e = getenv("VDL_PROBE_JIT_BLOCKS")) blocks = std::max(1, std::min(16, atoi(e)));
+static cudaKernel_t probe_jit_compile(vdl_ctx *ctx, const PDesc &d, size_t smem, int p_sub, int blocks, bool *ok, std::string *log) {
   const std::string src = probe_jit_source(d, p_sub, blocks);
   static const char *const headers[] = {EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_probe_kernel_cuh};
   static const char *const names[] = {"vdl_cuda.h", "vdl_device.cuh", "vdl_probe_kernel.cuh"};
-  if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] probe:\n%s\n", src.substr(0, src.find("#define STAGE_LOOP")).c_str());
+  if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] probe:\n%s\n", src.c_str());
   cudaKernel_t kh = vdl_jit_kernel(ctx, "probe|" + src, src, "vdl_probe_jit", 3, headers, names, ok, log);
   if (kh && smem > 48 * 1024 && cudaFuncSetAttribute((const void *)kh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     cudaGetLastError();
@@ -638,12 +390,10 @@ extern "C" int vdl_probe_jit_selftest(char *log, int log_capacity) {
   d.fold_op[2] = VDL_FOLD_COUNT;
   std::string l;
   bool ok1 = false, ok2 = false;
-  vdl_jit_kernel(nullptr, "", probe_jit_source(d, 4, 12), "vdl_probe_jit", 3, (const char *const[]){EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_probe_kernel_cuh},
-                 (const char *const[]){"vdl_cuda.h", "vdl_device.cuh", "vdl_probe_kernel.cuh"}, &ok1, &l);
+  probe_jit_compile(nullptr, d, 0, 4, 12, &ok1, &l);
   if (l == "NVRTC is not installed") return VDL_ENOTFOUND;
   d.nfolds = 0; d.nkeys = 0; d.nemits = 2; d.emit[0] = d.fold[0]; d.emit[1].nfac = 1; d.emit[1].f[0] = PTerm{2, 0, 0, 1};
-  if (ok1) vdl_jit_kernel(nullptr, "", probe_jit_source(d, 4, 12), "vdl_probe_jit", 3, (const char *const[]){EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_probe_kernel_cuh},
-                          (const char *const[]){"vdl_cuda.h", "vdl_device.cuh", "vdl_probe_kernel.cuh"}, &ok2, &l);
+  if (ok1) probe_jit_compile(nullptr, d, 0, 4, 12, &ok2, &l);
   if (log && log_capacity > 1) snprintf(log, (size_t)log_capacity, "%s", l.c_str());
   return ok1 && ok2 ? VDL_OK : VDL_ECUDA;
 }
@@ -841,7 +591,10 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
     if (const char *m = getenv("VDL_PROBE_JIT_MIN_ROWS")) min_rows = atoll(m);
     bool lens_ok = true;             // the generated code clamps a failed lookup to index 0: every looked-up column needs a row
     for (int l = 0; l < d.nleaves; l++) if (d.leaf[l].parent >= 0 && d.leaf[l].len < 1) lens_ok = false;
-    if (!(e && !strcmp(e, "0")) && d.rows >= min_rows && lens_ok) p->jit_kernel = probe_jit_compile(ctx, d, p->smem, nullptr, nullptr);
+    int p_sub = 8, blocks = 8;       // measured on B200 (Q5 / Q3 / Q12 / Q19 SF10): 8 rows per thread and round, 8 blocks x 64 registers
+    if (const char *s = getenv("VDL_PROBE_JIT_SUB")) p_sub = std::max(1, std::min(16, atoi(s)));
+    if (const char *s = getenv("VDL_PROBE_JIT_BLOCKS")) blocks = std::max(1, std::min(16, atoi(s)));
+    if (!(e && !strcmp(e, "0")) && d.rows >= min_rows && lens_ok) p->jit_kernel = probe_jit_compile(ctx, d, p->smem, p_sub, blocks, nullptr, nullptr);
   }
   *out = p;
   return VDL_OK;

@@ -1,5 +1,6 @@
-"""The fused FK-join probe kernel through its C entry points (vdl_probe_*), against a numpy evaluation of the
-same leaf / term / predicate descriptor: fold mode (small key domain) and emit mode (dense ordered output)."""
+"""The fused FK-join probe kernels through their C entry points (vdl_probe_*), against a numpy evaluation of the
+same leaf / term / predicate descriptor: fold mode (small key domain) and emit mode (dense ordered output).  Every case
+runs through both kernels: the interpreter and the kernel compiled at run time for the descriptor."""
 import ctypes as C
 
 import numpy as np
@@ -38,6 +39,30 @@ def tables(n, n1, n2, seed):
     }
 
 
+KERNELS = ["interpreter", "jit"]
+
+
+def use_kernel(kernel, monkeypatch):
+    """VDL_PROBE_JIT=0 keeps the interpreter; VDL_PROBE_JIT_MIN_ROWS=0 compiles the descriptor at every size.  With
+    VDL_DEBUG_JIT the compiled source is printed, which shows that the kernel named by the parameter is the one that ran."""
+    monkeypatch.delenv("VDL_PROBE_JIT", raising=False)
+    monkeypatch.delenv("VDL_PROBE_JIT_MIN_ROWS", raising=False)
+    monkeypatch.setenv("VDL_PROBE_JIT_MIN_ROWS" if kernel == "jit" else "VDL_PROBE_JIT", "0")
+    monkeypatch.setenv("VDL_DEBUG_JIT", "1")
+
+
+def assert_kernel_ran(kernel, capfd):
+    err = capfd.readouterr().err
+    assert ("[vdl jit] probe:" in err) == (kernel == "jit") and "runs instead" not in err, err[-2000:]
+
+
+@pytest.fixture(params=KERNELS)
+def kernel(request, monkeypatch, capfd):
+    use_kernel(request.param, monkeypatch)
+    yield request.param
+    assert_kernel_ran(request.param, capfd)
+
+
 def run_probe(ctx, desc):
     L = ctx.L
     h = C.c_void_p()
@@ -47,7 +72,7 @@ def run_probe(ctx, desc):
 
 
 @pytest.mark.parametrize("n", [1, 1000, 1024, 1025, 300_007])
-def test_probe_fold_matches_numpy(n):
+def test_probe_fold_matches_numpy(n, kernel):
     from mplan2vdl_b200.executor import Context
     ctx = Context(0)
     t = tables(n, max(1, n // 4), 50, n)
@@ -95,7 +120,7 @@ def test_probe_fold_matches_numpy(n):
 
 
 @pytest.mark.parametrize("n", [1, 1024, 5000, 1_000_003])
-def test_probe_emit_is_the_dense_foldselect_order(n):
+def test_probe_emit_is_the_dense_foldselect_order(n, kernel):
     from mplan2vdl_b200.executor import Context
     ctx = Context(0)
     t = tables(n, max(1, n // 3), 20, n + 1)
@@ -125,20 +150,23 @@ def test_probe_emit_is_the_dense_foldselect_order(n):
     ctx.close()
 
 
-def test_probe_reports_lookup_index_out_of_range():
+def test_probe_reports_lookup_index_out_of_range(monkeypatch, capfd):
     from mplan2vdl_b200.executor import Context
     from mplan2vdl_b200.lib import VdlError
-    ctx = Context(0)
-    f = ctx.upload_column("f.fk", np.array([0, 1, 5], dtype=np.int64))
-    dcol = ctx.upload_column("d.a", np.array([1, 2], dtype=np.int64))
-    d = vlib.ProbeDesc()
-    d.rows, d.nleaves = 3, 2
-    d.leaf[0], d.leaf[1] = vlib.Leaf(f, -1), vlib.Leaf(dcol, 0)
-    d.nkeys, d.domain, d.key_mask, d.nfolds = 0, 1, -1, 1
-    d.fold[0] = vlib.ProbeFold(SUM, 0, product(term(1)))
-    h = run_probe(ctx, d)
-    data, ln = C.POINTER(C.c_int64)(), C.c_int64()
-    with pytest.raises(VdlError):
-        ctx.check(ctx.L.vdl_probe_result_host(h, 0, C.byref(data), C.byref(ln)))
-    ctx.L.vdl_probe_destroy(h)
-    ctx.close()
+    for kernel in KERNELS:
+        use_kernel(kernel, monkeypatch)
+        ctx = Context(0)
+        f = ctx.upload_column("f.fk", np.array([0, 1, 5], dtype=np.int64))
+        dcol = ctx.upload_column("d.a", np.array([1, 2], dtype=np.int64))
+        d = vlib.ProbeDesc()
+        d.rows, d.nleaves = 3, 2
+        d.leaf[0], d.leaf[1] = vlib.Leaf(f, -1), vlib.Leaf(dcol, 0)
+        d.nkeys, d.domain, d.key_mask, d.nfolds = 0, 1, -1, 1
+        d.fold[0] = vlib.ProbeFold(SUM, 0, product(term(1)))
+        h = run_probe(ctx, d)
+        data, ln = C.POINTER(C.c_int64)(), C.c_int64()
+        with pytest.raises(VdlError):
+            ctx.check(ctx.L.vdl_probe_result_host(h, 0, C.byref(data), C.byref(ln)))
+        ctx.L.vdl_probe_destroy(h)
+        ctx.close()
+        assert_kernel_ran(kernel, capfd)
