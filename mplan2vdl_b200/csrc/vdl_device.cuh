@@ -1,5 +1,5 @@
-// Declarations shared by the device code of libvdl_cuda, written so that NVRTC can compile them too (the fused scan is
-// specialised at run time: vdl_fused_jit.cu): no host headers, fixed-width types spelled out under __CUDACC_RTC__.
+// Declarations shared by the device code of libvdl_cuda, written so that NVRTC can compile them too (the map, the fused
+// scan and the probe are specialised at run time: vdl_jit.cu): no host headers, fixed-width types spelled out under __CUDACC_RTC__.
 #pragma once
 
 #ifdef __CUDACC_RTC__
@@ -25,6 +25,21 @@ typedef unsigned long uintptr_t;
 
 typedef int64_t i64;
 typedef uint64_t u64;
+
+// Operand as the per-op kernels see it.
+struct Operand {
+  const void *p;
+  int kind;      // 0 = int64 array, 1 = int32 array, 2 = range
+  i64 from, step;
+};
+
+// vdl_op_map's kernel arguments (interpreter in vdl_ops.cu, run-time specialisation in vdl_jit.cu)
+struct MapArgs {
+  Operand in[VDL_MAP_MAX_INPUTS];
+  Operand tab[VDL_MAP_MAX_TABLES];
+  i64 tab_len[VDL_MAP_MAX_TABLES];
+  vdl_map_desc d;
+};
 
 // Peer-memory exchange of the partial tables (one buffer per rank, addressable by all ranks):
 //   data  [2 (epoch parity)][world][stride] int64   rank r's table of the step lands in slot [parity][r] of EVERY buffer
@@ -73,6 +88,19 @@ __device__ __forceinline__ u64 global_timer_ns() {
   u64 t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
+}
+// Element i of an operand whose storage kind is known at compile time (the run-time specialised map prints it as a
+// literal), and of any operand
+template <int KIND>
+__device__ __forceinline__ i64 op_ld_k(const Operand &o, i64 i) {
+  if (KIND == 0) return ((const i64 *)o.p)[i];
+  if (KIND == 1) return (i64)((const int32_t *)o.p)[i];
+  return (i64)((u64)o.from + (u64)i * (u64)o.step);
+}
+__device__ __forceinline__ i64 op_ld(const Operand &o, i64 i) {
+  if (o.kind == 0) return op_ld_k<0>(o, i);
+  if (o.kind == 1) return op_ld_k<1>(o, i);
+  return op_ld_k<2>(o, i);
 }
 // Elementwise op semantics (Vdl.hs:136-157, 209-231).  Comparisons / logicals give 0/1; BitShift: +k arithmetic right,
 // -k left (Vlite.hs:205-208); Divide truncates, x/0 := 0, INT64_MIN/-1 wraps; Modulo is the C remainder, x%0 := 0.

@@ -138,7 +138,6 @@ static bool shape_matches(const KDesc &k) {
 // accumulators may live in registers and how) is printed as a shape-traits class, fused_scan_fold_body is instantiated
 // over it by NVRTC for sm_100a and cached per context.  Every constant stays a run-time descriptor field, exactly as with
 // the static shapes, so one compiled kernel serves every plan of that structure.
-#include "vdl_embedded.inc"      // the three headers the generated source includes, as strings (written by build.py)
 
 static int flags_of(const KAffine &a) {
   if (a.col == -1) return FF_CONST;
@@ -188,22 +187,18 @@ static std::string jit_shape_struct(const KDesc &k, int key32, int rs_g, const i
   return s;
 }
 
-static cudaKernel_t jit_scan_compile(vdl_ctx *ctx, const std::string &shape_struct, int nc, int r, int g, int smem_max, bool *ok, std::string *log) {
+static std::string jit_scan_source(const std::string &shape_struct, int nc, int r, int g) {
   char b[512];
   snprintf(b, sizeof b,
            "extern \"C\" __global__ void __launch_bounds__(%d, 1) vdl_scan_jit(const __grid_constant__ KDesc d, const __grid_constant__ FinDesc fd, "
            "const __grid_constant__ XDesc xd) {\n  fused_scan_fold_body<ShapeJit, %d, %d, %d>(d, fd, xd);\n}\n", nc + 32, nc, r, g);
-  const std::string src = std::string("#include \"vdl_fused_kernel.cuh\"\n") + shape_struct + b;
-  static const char *const headers[] = {EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_fused_kernel_cuh};
-  static const char *const names[] = {"vdl_cuda.h", "vdl_device.cuh", "vdl_fused_kernel.cuh"};
   if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] fused scan nc=%d r=%d g=%d:\n%s\n", nc, r, g, shape_struct.c_str());
-  cudaKernel_t kh = vdl_jit_kernel(ctx, "scan|" + src, src, "vdl_scan_jit", 3, headers, names, ok, log);
-  if (kh && cudaFuncSetAttribute((const void *)kh, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max) != cudaSuccess) {
-    cudaGetLastError();
-    if (ok) *ok = false;
-    return nullptr;
-  }
-  return kh;
+  return std::string("#include \"vdl_fused_kernel.cuh\"\n") + shape_struct + b;
+}
+
+static cudaKernel_t jit_scan_compile(vdl_ctx *ctx, const std::string &shape_struct, int nc, int r, int g, int smem_max) {
+  const std::string src = jit_scan_source(shape_struct, nc, r, g);
+  return vdl_jit_kernel(ctx, "scan|" + src, "vdl_scan_jit", smem_max, [&] { return src; });
 }
 
 // Host-only check (no GPU): generate the shape of a Q1-like descriptor and compile it with NVRTC for sm_100a.
@@ -220,12 +215,10 @@ extern "C" int vdl_scan_jit_selftest(char *log, int log_capacity) {
   k.acc[3].op = 1; k.acc[3].nfac = 1; k.acc[3].fac[0] = KAffine{-2, 0, 0, 1, 0, 0, 0, 0};
   const int rk[K_MAX_ACC] = {RK_N32, RK_MADW, RK_N32, RK_FIRST};
   std::string l;
-  bool ok1 = false, ok2 = false;
-  jit_scan_compile(nullptr, jit_shape_struct(k, 1, 8, rk), 352, 4, 6, 0, &ok1, &l);
-  if (l == "NVRTC is not installed") return VDL_ENOTFOUND;
-  if (ok1) jit_scan_compile(nullptr, jit_shape_struct(k, 0, 0, rk), 512, 4, 0, 0, &ok2, &l);
+  int rc = vdl_jit_compile(jit_scan_source(jit_shape_struct(k, 1, 8, rk), 352, 4, 6), &l);
+  if (rc == VDL_OK) rc = vdl_jit_compile(jit_scan_source(jit_shape_struct(k, 0, 0, rk), 512, 4, 0), &l);
   if (log && log_capacity > 1) snprintf(log, (size_t)log_capacity, "%s", l.c_str());
-  return ok1 && ok2 ? VDL_OK : VDL_ECUDA;
+  return rc;
 }
 
 static bool affine_ok(const vdl_affine &a, int ncols) { return a.column >= -2 && a.column < ncols && a.shr >= 0 && a.shr < 64; }
@@ -481,8 +474,6 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     if (k.rows < min_rows || f->always_false) return 0;
     const int key32 = jit_key32(k);
     int rk[K_MAX_ACC] = {0};
-    bool ok = false;
-    std::string log;
     if (key32 && k.nacc <= 8 && k.domain <= 64 && !getenv("VDL_NO_REGISTER_SLOTS")) {
       int want_nc = 0, want_r = 0;
       if (const char *g = getenv("VDL_RS_GEOMETRY")) sscanf(g, "%d,%d", &want_nc, &want_r);
@@ -494,7 +485,7 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
         for (int j = 0; j < k.nacc; j++)      // cheapest representation whose proof holds
           rk[j] = rs_proof(j, RK_FIRST) ? RK_FIRST : (rs_proof(j, RK_N32) ? RK_N32 : (rs_proof(j, RK_MADW) ? RK_MADW : RK_WIDE));
         f->jit_struct = jit_shape_struct(k, key32, 8, rk);
-        cudaKernel_t kh = jit_scan_compile(ctx, f->jit_struct, geo[0], geo[1], 8, smem_max, &ok, &log);
+        cudaKernel_t kh = jit_scan_compile(ctx, f->jit_struct, geo[0], geo[1], 8, smem_max);
         if (kh) {
           f->jit_rs_kernel[8] = kh; f->jit_rs_tried[8] = true;
           f->rs = true; f->rs_gmax = 8; f->jit = true;
@@ -507,7 +498,7 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
       if (rc2) return -rc2;
     }
     f->jit_struct = jit_shape_struct(k, key32, 0, rk);
-    f->jit_kernel = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, 0, smem_max, &ok, &log);
+    f->jit_kernel = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, 0, smem_max);
     if (!f->jit_kernel) return 0;
     f->jit = true;
     return 1;
@@ -646,7 +637,7 @@ extern "C" int vdl_fused_launch_ex(vdl_fused *f, int self_finalize) {
           if (f->jit && !f->jit_rs_tried[c]) {        // the variant with fewer register slots: compiled on first use
             f->jit_rs_tried[c] = true;
             const int smem_max = ctx->smem_optin > 0 ? ctx->smem_optin : 232448;
-            f->jit_rs_kernel[c] = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, c, smem_max, nullptr, nullptr);
+            f->jit_rs_kernel[c] = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, c, smem_max);
           }
           if (f->jit ? f->jit_rs_kernel[c] != nullptr : f->rs_kernel[c] != nullptr) g = c;
         }

@@ -1,6 +1,6 @@
 // Device code of the fused select -> map -> fold scan (see vdl_fused.cu for what it replaces in the emitted graph and for
-// the host side).  Kept in a header that NVRTC can compile as well: vdl_fused_jit.cu generates the shape-traits class of a
-// prepared descriptor at run time and instantiates fused_scan_fold_body over it.
+// the host side).  Kept in a header that NVRTC can compile as well: vdl_fused.cu generates the shape-traits class of a
+// prepared descriptor at run time and instantiates fused_scan_fold_body over it (compiled by vdl_jit.cu).
 #pragma once
 
 #include "vdl_device.cuh"
@@ -716,7 +716,7 @@ __device__ __forceinline__ void fused_scan_fold_body(const KDesc &d, const FinDe
 }
 
 // The precompiled instantiations (GenericShape and the static shapes of vdl_shapes.cuh); a shape generated at run time
-// from a prepared descriptor gets its own `extern "C"` wrapper around fused_scan_fold_body (vdl_fused_jit.cu).
+// from a prepared descriptor gets its own `extern "C"` wrapper around fused_scan_fold_body (jit_scan_source, vdl_fused.cu).
 template <class S, int NC, int R, int G>
 __global__ void __launch_bounds__(NC + 32, 1) fused_scan_fold_kernel(const __grid_constant__ KDesc d, const __grid_constant__ FinDesc fd, const __grid_constant__ XDesc xd) {
   fused_scan_fold_body<S, NC, R, G>(d, fd, xd);

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <functional>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -55,7 +56,7 @@ struct vdl_ctx {
   void *scratch = nullptr;  // reusable scratch for scans / histograms
   size_t scratch_bytes = 0;
   void *h_mail = nullptr, *d_mail = nullptr;   // 64 B of mapped pinned memory: scalars the host waits for (read_scalar)
-  void *jit = nullptr;      // vdl_jit.cu: specialised vdl_op_map kernels
+  void *jit = nullptr;      // vdl_jit.cu: the run-time compiled map, scan and probe kernels
   u64 gen_counter = 0;      // source of Vec::gen
 };
 
@@ -93,27 +94,19 @@ int vec_narrow_copy(vdl_ctx *ctx, vdl_vec src, vdl_vec *out);   // vdl_ops.cu: i
 // 0.3 ms step on 8 GPUs.  Falls back to synchronising the stream (errors surface there) after ~20 ms.
 int wait_published(vdl_ctx *ctx, const volatile i64 *word, i64 seq);
 
-// Operand as the per-op kernels see it.
-struct Operand {
-  const void *p;
-  int kind;      // 0 = int64 array, 1 = int32 array, 2 = range
-  i64 from, step;
-};
 Operand operand_of(const Vec &v);
 inline bool vec_is_narrow(const Vec &v) { return v.narrow32 || (v.dtype == VDL_I32 && !v.is_range); }
 
-// vdl_op_map's kernel arguments (interpreter in vdl_ops.cu, run-time specialisation in vdl_jit.cu)
-struct MapArgs {
-  Operand in[VDL_MAP_MAX_INPUTS];
-  Operand tab[VDL_MAP_MAX_TABLES];
-  i64 tab_len[VDL_MAP_MAX_TABLES];
-  vdl_map_desc d;
-};
 int vdl_jit_map_launch(vdl_ctx *ctx, const MapArgs &m, i64 *out, i64 n, int blocks);   // 1 launched, 0 use the interpreter, <0 error
 void vdl_jit_destroy(vdl_ctx *ctx);
-// NVRTC compile + load of one kernel, cached per context under `key` (vdl_jit.cu); ctx == nullptr: compile only
-cudaKernel_t vdl_jit_kernel(vdl_ctx *ctx, const std::string &key, const std::string &src, const char *kernel_name, int nheaders,
-                            const char *const *headers, const char *const *header_names, bool *ok, std::string *log);
+// vdl_jit.cu: NVRTC compile of `src` for sm_100a against the headers embedded in the library.  VDL_OK (the image in
+// *cubin, if given), VDL_ENOTFOUND when NVRTC is not installed, VDL_ECUDA when it rejected the source (NVRTC's log in
+// *log, its status in *status, if given).  Needs no GPU.
+int vdl_jit_compile(const std::string &src, std::string *log, std::vector<char> *cubin = nullptr, int *status = nullptr);
+// The kernel `name` of the source `source()` returns, compiled and loaded once per context and cached under `key`;
+// `source` is called on a miss only.  Takes `smem` bytes of dynamic shared memory when that is over the default 48 KB.
+// nullptr: NVRTC is missing, compilation or loading failed (also cached: no retry), or the attribute could not be set.
+cudaKernel_t vdl_jit_kernel(vdl_ctx *ctx, const std::string &key, const char *name, size_t smem, const std::function<std::string()> &source);
 
 // Do the columns a prepared scan / probe was built from still hold what they held at prepare time?  (The statistics
 // proofs -- int32 narrowing, 32-bit accumulators, the static shape -- and the device pointers are baked in.)

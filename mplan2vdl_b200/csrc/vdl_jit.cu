@@ -1,10 +1,11 @@
-// Run-time specialisation of vdl_op_map: for long vectors the register program is turned into straight-line CUDA C,
-// compiled for sm_100a with NVRTC (dlopen'ed: the library has no link-time dependency on it) and loaded through the
-// runtime's library API.  The interpreter in vdl_ops.cu spends ~15 issue slots per instruction and row on decoding and
-// on its local-memory register file; the specialised kernel keeps every value in a register and is bound by the HBM
-// reads of its inputs.  Kernels are cached per context, keyed by the program and the operands' storage kinds.
-// Semantics per instruction: the same expressions as binop_apply (vdl_internal.h) / map_kernel (vdl_ops.cu); the parity
-// tests run every binary op through both.
+// Run-time compiled kernels: a generated source is compiled for sm_100a with NVRTC (dlopen'ed: the library has no
+// link-time dependency on it) against the headers embedded in the library, loaded through the runtime's library API and
+// cached per context.  The fused scan (vdl_fused.cu) and the FK-join probe (vdl_probe.cu) generate theirs; the one of
+// vdl_op_map is generated here.
+// vdl_op_map: for long vectors the register program is turned into straight-line CUDA C.  The interpreter in vdl_ops.cu
+// spends ~15 issue slots per instruction and row on decoding and on its local-memory register file; the specialised kernel
+// keeps every value in a register and is bound by the HBM reads of its inputs.  Both take MapArgs, op_ld and binop_apply
+// from vdl_device.cuh: the generated source only spells the operands' storage kinds and the ops as literals.
 #include <dlfcn.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -15,6 +16,7 @@
 #include <vector>
 
 #include "vdl_internal.h"
+#include "vdl_embedded.inc"      // the headers a generated source may include, as strings (written by build.py)
 
 namespace {
 
@@ -58,78 +60,32 @@ struct JitCache {
   std::vector<cudaLibrary_t> libs;
 };
 
-// One C expression per binary op, over int64 operands A and B (binop_apply's cases).
-std::string binop_expr(int op, const std::string &A, const std::string &B) {
-  switch (op) {
-    case VDL_LOGICAL_AND: return "(i64)((" + A + " != 0) && (" + B + " != 0))";
-    case VDL_LOGICAL_OR: return "(i64)((" + A + " != 0) || (" + B + " != 0))";
-    case VDL_BITWISE_AND: return "(" + A + " & " + B + ")";
-    case VDL_BITWISE_OR: return "(" + A + " | " + B + ")";
-    case VDL_BITSHIFT: return "shift(" + A + ", " + B + ")";
-    case VDL_EQUALS: return "(i64)(" + A + " == " + B + ")";
-    case VDL_ADD: return "(i64)((u64)" + A + " + (u64)" + B + ")";
-    case VDL_SUBTRACT: return "(i64)((u64)" + A + " - (u64)" + B + ")";
-    case VDL_GREATER: return "(i64)(" + A + " > " + B + ")";
-    case VDL_MULTIPLY: return "(i64)((u64)" + A + " * (u64)" + B + ")";
-    case VDL_DIVIDE: return "divide(" + A + ", " + B + ")";
-    case VDL_MODULO: return "modulo(" + A + ", " + B + ")";
-  }
-  return "0";
-}
-
-std::string load_expr(const char *arr, int k, int kind, const std::string &idx) {
-  char b[256];
-  if (kind == 0) snprintf(b, sizeof b, "((const i64 *)m.%s[%d].p)[%s]", arr, k, idx.c_str());
-  else if (kind == 1) snprintf(b, sizeof b, "(i64)((const int *)m.%s[%d].p)[%s]", arr, k, idx.c_str());
-  else snprintf(b, sizeof b, "(i64)((u64)m.%s[%d].from + (u64)(%s) * (u64)m.%s[%d].step)", arr, k, idx.c_str(), arr, k);
-  return b;
-}
-
 std::string generate(const MapArgs &m) {
   const vdl_map_desc &d = m.d;
-  std::string s;
+  std::string s = "#include \"vdl_device.cuh\"\n__device__ __forceinline__ i64 row(const MapArgs &m, const i64 i, int *err) {\n";
   char b[512];
-  snprintf(b, sizeof b,
-           "typedef long long i64;\ntypedef unsigned long long u64;\n"
-           "struct Operand { const void *p; int kind; i64 from, step; };\n"
-           "struct Instr { short op, dst, a, b; };\n"
-           "struct Desc { int ninputs, ntables, ninstrs, nimms; Instr instr[%d]; i64 imm[%d]; };\n"
-           "struct Args { Operand in[%d]; Operand tab[%d]; i64 tab_len[%d]; Desc d; };\n",
-           VDL_MAP_MAX_INSTRS, VDL_MAP_MAX_IMMS, VDL_MAP_MAX_INPUTS, VDL_MAP_MAX_TABLES, VDL_MAP_MAX_TABLES);
-  s += b;
-  s += "__device__ __forceinline__ i64 shift(i64 a, i64 b) {\n"
-       "  if (b >= 0) return b >= 64 ? (a < 0 ? -1 : 0) : (a >> b);\n"
-       "  return b <= -64 ? 0 : (i64)((u64)a << (-b));\n}\n"
-       "__device__ __forceinline__ i64 divide(i64 a, i64 b) {\n"
-       "  if (b == 0) return 0;\n  if (b == -1) return (i64)(0 - (u64)a);\n  return a / b;\n}\n"
-       "__device__ __forceinline__ i64 modulo(i64 a, i64 b) {\n"
-       "  if (b == 0 || b == -1) return 0;\n  return a % b;\n}\n";
-  s += "__device__ __forceinline__ i64 row(const Args &m, const i64 i, int *err) {\n";
   // SSA over the register program: reg -> name of the value it currently holds
   std::vector<std::string> cur(VDL_MAP_MAX_REGS);
   for (int t = 0; t < d.ninstrs; t++) {
     const vdl_map_instr &ins = d.instr[t];
-    std::string v = "v" + std::to_string(t), e;
+    const std::string v = "v" + std::to_string(t);
     if (ins.op == VDL_MAP_LOAD) {
-      e = load_expr("in", ins.b, m.in[ins.b].kind, "i");
+      snprintf(b, sizeof b, "  const i64 %s = op_ld_k<%d>(m.in[%d], i);\n", v.c_str(), m.in[ins.b].kind, ins.b);
     } else if (ins.op == VDL_MAP_RANGE) {
-      snprintf(b, sizeof b, "(i64)(%lluull + (u64)i * %lluull)", (unsigned long long)d.imm[ins.a], (unsigned long long)d.imm[ins.b]);
-      e = b;
+      snprintf(b, sizeof b, "  const i64 %s = (i64)(%lluull + (u64)i * %lluull);\n", v.c_str(), (unsigned long long)d.imm[ins.a],
+               (unsigned long long)d.imm[ins.b]);
     } else if (ins.op == VDL_MAP_GATHER) {
-      const std::string &a = cur[ins.a];
-      snprintf(b, sizeof b, "  i64 %s = 0;\n  if ((u64)%s >= (u64)m.tab_len[%d]) atomicAdd(err, 1); else %s = ", v.c_str(), a.c_str(), ins.b, v.c_str());
-      s += b;
-      s += load_expr("tab", ins.b, m.tab[ins.b].kind, a) + ";\n";
-      cur[ins.dst] = v;
-      continue;
+      const char *a = cur[ins.a].c_str();
+      snprintf(b, sizeof b, "  i64 %s = 0;\n  if ((u64)%s >= (u64)m.tab_len[%d]) atomicAdd(err, 1); else %s = op_ld_k<%d>(m.tab[%d], %s);\n",
+               v.c_str(), a, ins.b, v.c_str(), m.tab[ins.b].kind, ins.b, a);
     } else {
-      e = binop_expr(ins.op, cur[ins.a], cur[ins.b]);
+      snprintf(b, sizeof b, "  const i64 %s = binop_apply(%d, %s, %s);\n", v.c_str(), ins.op, cur[ins.a].c_str(), cur[ins.b].c_str());
     }
-    s += "  const i64 " + v + " = " + e + ";\n";
+    s += b;
     cur[ins.dst] = v;
   }
   s += "  return " + cur[d.instr[d.ninstrs - 1].dst] + ";\n}\n";
-  s += "extern \"C\" __global__ void __launch_bounds__(256) vdl_map_jit(const __grid_constant__ Args m, i64 *__restrict__ out, const i64 n, int *err) {\n"
+  s += "extern \"C\" __global__ void __launch_bounds__(256) vdl_map_jit(const __grid_constant__ MapArgs m, i64 *__restrict__ out, const i64 n, int *err) {\n"
        "  const i64 stride = (i64)gridDim.x * 256;\n"
        "  i64 i = (i64)blockIdx.x * 256 + threadIdx.x;\n"
        "  for (; i + stride < n; i += 2 * stride) {\n"
@@ -139,99 +95,96 @@ std::string generate(const MapArgs &m) {
   return s;
 }
 
-cudaKernel_t compile(vdl_ctx *ctx, JitCache *jc, const std::string &src, const char *kernel_name = "vdl_map_jit", int nheaders = 0,
-                     const char *const *headers = nullptr, const char *const *header_names = nullptr, std::string *log_out = nullptr) {
-  Nvrtc &N = g_nvrtc;
-  void *prog = nullptr;
-  if (N.create(&prog, src.c_str(), "vdl_jit.cu", nheaders, headers, header_names) != 0) return nullptr;
-  // -default-device: the public header's (unannotated) function declarations are only declarations here
-  const char *opts[] = {"--gpu-architecture=sm_100a", "--std=c++17", "-lineinfo", "-default-device"};
-  int rc = N.compile(prog, 4, opts);
-  if (rc != 0) {
-    size_t ls = 0;
-    N.log_size(prog, &ls);
-    std::string log(ls + 1, '\0');
-    if (ls) N.log(prog, &log[0]);
-    if (log_out) *log_out = log;
-    fprintf(stderr, "[vdl jit] NVRTC failed (%d) for %s; the precompiled kernel runs instead.\n%s\n", rc, kernel_name, log.c_str());
+// Compile `src` and load its kernel `name`.  nullptr, after a message on stderr, when either fails.
+cudaKernel_t compile_and_load(JitCache *jc, const std::string &src, const char *name) {
+  std::string log;
+  std::vector<char> cubin;
+  int status = 0;
+  if (vdl_jit_compile(src, &log, &cubin, &status) != VDL_OK) {
+    fprintf(stderr, "[vdl jit] NVRTC failed (%d) for %s; the precompiled kernel runs instead.\n%s\n", status, name, log.c_str());
     if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "%s\n", src.c_str());
-    N.destroy(&prog);
     return nullptr;
   }
-  size_t cs = 0;
-  N.cubin_size(prog, &cs);
-  std::vector<char> cubin(cs);
-  N.cubin(prog, cubin.data());
-  N.destroy(&prog);
   cudaLibrary_t lib = nullptr;
   cudaKernel_t k = nullptr;
   if (cudaLibraryLoadData(&lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0) != cudaSuccess ||
-      cudaLibraryGetKernel(&k, lib, kernel_name) != cudaSuccess) {
+      cudaLibraryGetKernel(&k, lib, name) != cudaSuccess) {
     fprintf(stderr, "[vdl jit] loading the compiled kernel failed (%s); the interpreter runs instead.\n", cudaGetErrorString(cudaGetLastError()));
     if (lib) cudaLibraryUnload(lib);
     return nullptr;
   }
   jc->libs.push_back(lib);
-  (void)ctx;
   return k;
 }
 
 }  // namespace
 
+int vdl_jit_compile(const std::string &src, std::string *log, std::vector<char> *cubin, int *status) {
+  log->clear();
+  if (!nvrtc_load()) return VDL_ENOTFOUND;
+  // NVRTC reads only the headers the source includes
+  static const char *const headers[] = {EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_fused_kernel_cuh, EMB_vdl_probe_kernel_cuh};
+  static const char *const names[] = {"vdl_cuda.h", "vdl_device.cuh", "vdl_fused_kernel.cuh", "vdl_probe_kernel.cuh"};
+  Nvrtc &N = g_nvrtc;
+  void *prog = nullptr;
+  int rc = N.create(&prog, src.c_str(), "vdl_jit.cu", 4, headers, names);
+  if (status) *status = rc;
+  if (rc != 0) return VDL_ECUDA;
+  // -default-device: the public header's (unannotated) function declarations are only declarations here
+  const char *opts[] = {"--gpu-architecture=sm_100a", "--std=c++17", "-lineinfo", "-default-device"};
+  rc = N.compile(prog, 4, opts);
+  if (status) *status = rc;
+  size_t ls = 0, cs = 0;
+  N.log_size(prog, &ls);
+  if (ls > 1) {
+    log->resize(ls);
+    N.log(prog, &(*log)[0]);
+    log->resize(ls - 1);                           // without the terminating NUL
+  }
+  if (rc == 0) N.cubin_size(prog, &cs);
+  if (cubin && cs > 0) {
+    cubin->resize(cs);
+    N.cubin(prog, cubin->data());
+  }
+  N.destroy(&prog);
+  return rc == 0 && cs > 0 ? VDL_OK : VDL_ECUDA;
+}
+
+cudaKernel_t vdl_jit_kernel(vdl_ctx *ctx, const std::string &key, const char *name, size_t smem, const std::function<std::string()> &source) {
+  if (!nvrtc_load()) return nullptr;
+  if (!ctx->jit) ctx->jit = new JitCache();
+  JitCache *jc = (JitCache *)ctx->jit;
+  auto it = jc->kernels.find(key);
+  if (it == jc->kernels.end()) it = jc->kernels.emplace(key, compile_and_load(jc, source(), name)).first;
+  if (it->second && smem > 48 * 1024 &&
+      cudaFuncSetAttribute((const void *)it->second, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    cudaGetLastError();
+    return nullptr;
+  }
+  return it->second;
+}
+
 // Launches the specialised kernel for `m` on the context's stream.  Returns 1 when it did, 0 when the caller should run
 // the interpreter (NVRTC missing, compilation failed, VDL_NO_JIT), negative on a launch error.
 int vdl_jit_map_launch(vdl_ctx *ctx, const MapArgs &m, i64 *out, i64 n, int blocks) {
-  const bool off = getenv("VDL_NO_JIT") != nullptr;
-  if (off || !nvrtc_load()) return 0;
-  if (!ctx->jit) ctx->jit = new JitCache();
-  JitCache *jc = (JitCache *)ctx->jit;
+  if (getenv("VDL_NO_JIT")) return 0;
   // key: everything the generated source depends on (the program, its immediates, the operands' storage kinds)
-  std::string key;
+  std::string key = "map|";
   key.append((const char *)&m.d, 4 * sizeof(int32_t));
   key.append((const char *)m.d.instr, (size_t)m.d.ninstrs * sizeof(vdl_map_instr));
   key.append((const char *)m.d.imm, (size_t)m.d.nimms * sizeof(int64_t));
   for (int k = 0; k < m.d.ninputs; k++) key.push_back((char)m.in[k].kind);
   for (int k = 0; k < m.d.ntables; k++) key.push_back((char)m.tab[k].kind);
-  auto it = jc->kernels.find(key);
-  if (it == jc->kernels.end()) {
+  cudaKernel_t kh = vdl_jit_kernel(ctx, key, "vdl_map_jit", 0, [&] {
     if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] compiling a %d-instruction map program\n", m.d.ninstrs);
-    it = jc->kernels.emplace(key, compile(ctx, jc, generate(m))).first;
-  }
-  if (!it->second) return 0;
+    return generate(m);
+  });
+  if (!kh) return 0;
   int *err = ctx->d_errflag;
   void *args[] = {(void *)&m, (void *)&out, (void *)&n, (void *)&err};
-  cudaError_t e = cudaLaunchKernel((const void *)it->second, dim3(blocks), dim3(256), args, 0, ctx->stream);
+  cudaError_t e = cudaLaunchKernel((const void *)kh, dim3(blocks), dim3(256), args, 0, ctx->stream);
   if (e != cudaSuccess) { vdl_cuda_fail(ctx, e, "launch of a specialised map kernel"); return -1; }
   return 1;
-}
-
-// Compile `src` (which may #include the in-memory `headers`) for sm_100a and return the kernel `kernel_name`, cached per
-// context under `key`.  nullptr: NVRTC is missing or rejected the source (also cached: no retry).  With `ctx == nullptr`
-// only the compilation is attempted (host-only check: the cubin is not loaded); *ok tells whether it succeeded.
-cudaKernel_t vdl_jit_kernel(vdl_ctx *ctx, const std::string &key, const std::string &src, const char *kernel_name, int nheaders,
-                            const char *const *headers, const char *const *header_names, bool *ok, std::string *log) {
-  if (ok) *ok = false;
-  if (!nvrtc_load()) { if (log) *log = "NVRTC is not installed"; return nullptr; }
-  if (!ctx) {
-    Nvrtc &N = g_nvrtc;
-    void *prog = nullptr;
-    if (N.create(&prog, src.c_str(), "vdl_jit.cu", nheaders, headers, header_names) != 0) return nullptr;
-    const char *opts[] = {"--gpu-architecture=sm_100a", "--std=c++17", "-lineinfo", "-default-device"};
-    const int rc = N.compile(prog, 4, opts);
-    size_t ls = 0, cs = 0;
-    N.log_size(prog, &ls);
-    if (log && ls > 1) { log->assign(ls + 1, '\0'); N.log(prog, &(*log)[0]); }
-    if (rc == 0) N.cubin_size(prog, &cs);
-    N.destroy(&prog);
-    if (ok) *ok = rc == 0 && cs > 0;
-    return nullptr;
-  }
-  if (!ctx->jit) ctx->jit = new JitCache();
-  JitCache *jc = (JitCache *)ctx->jit;
-  auto it = jc->kernels.find(key);
-  if (it == jc->kernels.end()) it = jc->kernels.emplace(key, compile(ctx, jc, src, kernel_name, nheaders, headers, header_names, log)).first;
-  if (ok) *ok = it->second != nullptr;
-  return it->second;
 }
 
 // Host-only self-test (no GPU needed): print a program that uses every instruction kind and storage kind as CUDA C and
@@ -254,23 +207,10 @@ extern "C" int vdl_jit_selftest(char *log, int log_capacity) {
   d.instr[t++] = vdl_map_instr{VDL_MAP_GATHER, 7, 5, 1};
   d.instr[t++] = vdl_map_instr{VDL_ADD, 6, 6, 7};
   d.ninstrs = t;
-  if (!nvrtc_load()) return VDL_ENOTFOUND;
-  Nvrtc &N = g_nvrtc;
-  const std::string src = generate(m);
-  void *prog = nullptr;
-  if (N.create(&prog, src.c_str(), "vdl_map_jit.cu", 0, nullptr, nullptr) != 0) return VDL_ECUDA;
-  const char *opts[] = {"--gpu-architecture=sm_100a", "--std=c++17", "-lineinfo"};
-  const int rc = N.compile(prog, 3, opts);
-  size_t ls = 0, cs = 0;
-  N.log_size(prog, &ls);
-  if (log && log_capacity > 1 && ls > 1) {
-    std::string l(ls + 1, '\0');
-    N.log(prog, &l[0]);
-    snprintf(log, (size_t)log_capacity, "%s", l.c_str());
-  }
-  if (rc == 0) N.cubin_size(prog, &cs);
-  N.destroy(&prog);
-  return rc == 0 && cs > 0 ? VDL_OK : VDL_ECUDA;
+  std::string l;
+  const int rc = vdl_jit_compile(generate(m), &l);
+  if (log && log_capacity > 1) snprintf(log, (size_t)log_capacity, "%s", l.c_str());
+  return rc;
 }
 
 void vdl_jit_destroy(vdl_ctx *ctx) {

@@ -10,12 +10,6 @@
 #include "vdl_internal.h"
 #include <type_traits>
 
-__device__ __forceinline__ i64 op_ld(const Operand &o, i64 i) {
-  if (o.kind == 0) return ((const i64 *)o.p)[i];
-  if (o.kind == 1) return (i64)((const int32_t *)o.p)[i];
-  return (i64)((u64)o.from + (u64)i * (u64)o.step);
-}
-
 // ---------------------------------------------------------------------------------- RangeV / RangeC
 extern "C" int vdl_op_range(vdl_ctx *ctx, int64_t from, int64_t step, int64_t len, vdl_vec *out) {
   if (!ctx || !out) return VDL_EINVAL;
@@ -23,7 +17,7 @@ extern "C" int vdl_op_range(vdl_ctx *ctx, int64_t from, int64_t step, int64_t le
 }
 
 // ---------------------------------------------------------------------------------- elementwise
-// op semantics: binop_apply in vdl_internal.h
+// op semantics: binop_apply in vdl_device.cuh
 template <int OP>
 __global__ void __launch_bounds__(256) binary_kernel(Operand a, Operand b, i64 *__restrict__ out, i64 n) {
   // two elements per thread and step: 16-byte stores, 2 x (8 or 4)-byte loads per operand in flight

@@ -218,7 +218,6 @@ __global__ void __launch_bounds__(256, 1) probe_finalize_kernel(const __grid_con
 }
 
 #include <string>
-#include "vdl_embedded.inc"
 
 // ---- run-time specialisation of the probe (NVRTC) ---------------------------------------------------------------------
 // probe_kernel above INTERPRETS the descriptor: per row and stage it walks parent chains through the leaf table, dispatches
@@ -356,20 +355,9 @@ static std::string probe_jit_source(const PDesc &d, int p_sub, int blocks) {
     s += g.body + st;
   }
   snprintf(b, sizeof b, "  }\n};\nextern \"C\" __global__ void __launch_bounds__(P_THREADS, %d) vdl_probe_jit(const __grid_constant__ PDesc d) { probe_body<ProbeJit>(d, threadIdx.x); }\n", blocks);
-  return s + b;
-}
-
-static cudaKernel_t probe_jit_compile(vdl_ctx *ctx, const PDesc &d, size_t smem, int p_sub, int blocks, bool *ok, std::string *log) {
-  const std::string src = probe_jit_source(d, p_sub, blocks);
-  static const char *const headers[] = {EMB_vdl_cuda_h, EMB_vdl_device_cuh, EMB_vdl_probe_kernel_cuh};
-  static const char *const names[] = {"vdl_cuda.h", "vdl_device.cuh", "vdl_probe_kernel.cuh"};
-  if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] probe:\n%s\n", src.c_str());
-  cudaKernel_t kh = vdl_jit_kernel(ctx, "probe|" + src, src, "vdl_probe_jit", 3, headers, names, ok, log);
-  if (kh && smem > 48 * 1024 && cudaFuncSetAttribute((const void *)kh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
-  return kh;
+  s += b;
+  if (getenv("VDL_DEBUG_JIT")) fprintf(stderr, "[vdl jit] probe:\n%s\n", s.c_str());
+  return s;
 }
 
 // Host-only check (no GPU): print a two-stage descriptor with a lookup chain, a range set, a column comparison, an
@@ -389,13 +377,11 @@ extern "C" int vdl_probe_jit_selftest(char *log, int log_capacity) {
   d.fold_op[1] = VDL_FOLD_MIN; d.fold[1].nfac = 1; d.fold[1].f[0] = PTerm{-2, 0, 0, 1};
   d.fold_op[2] = VDL_FOLD_COUNT;
   std::string l;
-  bool ok1 = false, ok2 = false;
-  probe_jit_compile(nullptr, d, 0, 4, 12, &ok1, &l);
-  if (l == "NVRTC is not installed") return VDL_ENOTFOUND;
+  int rc = vdl_jit_compile(probe_jit_source(d, 4, 12), &l);
   d.nfolds = 0; d.nkeys = 0; d.nemits = 2; d.emit[0] = d.fold[0]; d.emit[1].nfac = 1; d.emit[1].f[0] = PTerm{2, 0, 0, 1};
-  if (ok1) probe_jit_compile(nullptr, d, 0, 4, 12, &ok2, &l);
+  if (rc == VDL_OK) rc = vdl_jit_compile(probe_jit_source(d, 4, 12), &l);
   if (log && log_capacity > 1) snprintf(log, (size_t)log_capacity, "%s", l.c_str());
-  return ok1 && ok2 ? VDL_OK : VDL_ECUDA;
+  return rc;
 }
 
 struct vdl_probe {
@@ -594,7 +580,10 @@ extern "C" int vdl_probe_prepare(vdl_ctx *ctx, const vdl_probe_desc *desc, vdl_p
     int p_sub = 8, blocks = 8;       // measured on B200 (Q5 / Q3 / Q12 / Q19 SF10): 8 rows per thread and round, 8 blocks x 64 registers
     if (const char *s = getenv("VDL_PROBE_JIT_SUB")) p_sub = std::max(1, std::min(16, atoi(s)));
     if (const char *s = getenv("VDL_PROBE_JIT_BLOCKS")) blocks = std::max(1, std::min(16, atoi(s)));
-    if (!(e && !strcmp(e, "0")) && d.rows >= min_rows && lens_ok) p->jit_kernel = probe_jit_compile(ctx, d, p->smem, p_sub, blocks, nullptr, nullptr);
+    if (!(e && !strcmp(e, "0")) && d.rows >= min_rows && lens_ok) {
+      const std::string src = probe_jit_source(d, p_sub, blocks);
+      p->jit_kernel = vdl_jit_kernel(ctx, "probe|" + src, "vdl_probe_jit", p->smem, [&] { return src; });
+    }
   }
   *out = p;
   return VDL_OK;
