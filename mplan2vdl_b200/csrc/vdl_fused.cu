@@ -32,7 +32,6 @@
 #include "vdl_fused_kernel.cuh"
 
 // ------------------------------------------------------------------------------ host side
-typedef void (*scan_kernel_fn)(const KDesc, const FinDesc, const XDesc);
 struct vdl_fused {
   vdl_ctx *ctx = nullptr;
   KDesc kd;
@@ -42,22 +41,22 @@ struct vdl_fused {
   int nout = 0;
   bool always_false = false, rs = false;
   unsigned int *d_done = nullptr; // ticket counter of the scan kernel's last-CTA epilogue
-  // register slots: kernels by slot count; the launch picks the smallest count that covers the groups the previous
-  // run of this scan produced (more slots = more predicated work per row; too few = keys on the slow global path)
-  scan_kernel_fn rs_kernel[9] = {nullptr};
-  int rs_gmax = 0;
+  // Precompiled instantiations or vdl_jit_kernel's cudaKernel_t (cudaLaunchKernel takes both): `kernel` with shared-memory
+  // tables, or `rs_kernel` by register-slot count.  The launch picks the smallest count that covers the groups the previous
+  // run produced (more slots = more predicated work per row; too few = keys on the slow global path).  Static variants are
+  // filled at prepare, run-time compiled ones with fewer slots compiled on first use (rs_tried).
+  const void *kernel = nullptr;
+  const void *rs_kernel[9] = {nullptr};
+  bool rs_tried[9] = {false};
   i64 groups_seen = -1;
   size_t smem_bytes = 0;
+  int smem_max = 0;               // the dynamic shared memory every scan kernel is allowed
   int grid = 1, nc = 256, r = 4;
-  scan_kernel_fn kernel = nullptr;
   const char *shape = "generic";
   KernelTimer timer;
   // run-time specialised kernels (vdl_jit_kernel): the shape-traits class generated from THIS descriptor
   bool jit = false;
   std::string jit_struct, jit_name;     // the generated `struct ShapeJit {...}` text; "jit:<hash>"
-  cudaKernel_t jit_kernel = nullptr;    // shared-memory tables (G = 0)
-  cudaKernel_t jit_rs_kernel[9] = {nullptr};
-  bool jit_rs_tried[9] = {false};
   // identity of the columns at prepare time (the proofs above hold for exactly this data)
   int ncols = 0;
   vdl_vec col_handle[VDL_MAX_COLS] = {0};
@@ -74,55 +73,68 @@ bool vdl_fused_current(vdl_fused *f) {
 
 #include "vdl_shapes.cuh"
 
-template <class S>
-static scan_kernel_fn scan_kernel_for(int nc, int r) {
-  if (nc == 512) return r == 4 ? fused_scan_fold_kernel<S, 512, 4, 0> : (r == 2 ? fused_scan_fold_kernel<S, 512, 2, 0> : fused_scan_fold_kernel<S, 512, 1, 0>);
-  return r == 4 ? fused_scan_fold_kernel<S, 256, 4, 0> : (r == 2 ? fused_scan_fold_kernel<S, 256, 2, 0> : fused_scan_fold_kernel<S, 256, 1, 0>);
-}
-// register-slot instantiations (geometries: rs_geometries) for g of the shape's RS_G slots in registers
-template <class S, int G>
-static scan_kernel_fn rs_kernel_for_g(int nc, int r) {
-  // consumer warps + the producer warp are dealt round-robin to the 4 SM sub-partitions (16 K registers each):
-  // 11 + 1 warps -> 3 per sub-partition -> 168 registers per thread; 15 + 1 -> 4 -> 128; 7 + 1 -> 2 -> 255
-  if (nc == 352 && r == 4) return fused_scan_fold_kernel<S, 352, 4, G>;
-  if (nc == 352 && r == 2) return fused_scan_fold_kernel<S, 352, 2, G>;
-  if (nc == 480 && r == 2) return fused_scan_fold_kernel<S, 480, 2, G>;
-  return nullptr;
-}
-template <class S>
-static scan_kernel_fn rs_kernel_for(int nc, int r, int g) {
-  if constexpr (S::RS_G > 0) {
-    static_assert(S::RS_G == 8, "instantiate the slot counts this shape allows");
-    if (g == 8) return rs_kernel_for_g<S, 8>(nc, r);
-    if (g == 6) return rs_kernel_for_g<S, 6>(nc, r);
-    if (g == 4) return rs_kernel_for_g<S, 4>(nc, r);
-  }
-  return nullptr;
-}
+// register slots: the slot counts of every register-slot kernel, and the launch geometries {nc, r} tried in this order.
+// Consumer warps + the producer warp are dealt round-robin to the 4 SM sub-partitions (16 K registers each):
+// 11 + 1 warps -> 3 per sub-partition -> 168 registers per thread; 15 + 1 -> 4 -> 128; 7 + 1 -> 2 -> 255
 static const int rs_slot_counts[] = {4, 6, 8};
 static const int rs_geometries[][2] = {{352, 4}, {352, 2}, {480, 2}};
 
-// does the prepared descriptor satisfy every assumption static shape S compiles in?
+// The precompiled instantiation of shape S for nc consumer threads, r rows per thread and g register slots, or nullptr:
+// g = 0 (shared-memory tables) for every geometry default_geometry picks, g = 4 / 6 / 8 for rs_geometries when S has
+// register slots.
+template <class S>
+static const void *static_kernel(int nc, int r, int g) {
+#define VDL_SCAN_KERNEL(NC, R, G) \
+  if (nc == NC && r == R && g == G) return (const void *)fused_scan_fold_kernel<S, NC, R, G>
+  VDL_SCAN_KERNEL(512, 4, 0); VDL_SCAN_KERNEL(512, 2, 0); VDL_SCAN_KERNEL(512, 1, 0);
+  VDL_SCAN_KERNEL(256, 4, 0); VDL_SCAN_KERNEL(256, 2, 0); VDL_SCAN_KERNEL(256, 1, 0);
+  if constexpr (S::RS_G > 0) {
+    static_assert(S::RS_G == 8, "instantiate the slot counts this shape allows");
+    VDL_SCAN_KERNEL(352, 4, 8); VDL_SCAN_KERNEL(352, 2, 8); VDL_SCAN_KERNEL(480, 2, 8);
+    VDL_SCAN_KERNEL(352, 4, 6); VDL_SCAN_KERNEL(352, 2, 6); VDL_SCAN_KERNEL(480, 2, 6);
+    VDL_SCAN_KERNEL(352, 4, 4); VDL_SCAN_KERNEL(352, 2, 4); VDL_SCAN_KERNEL(480, 2, 4);
+  }
+#undef VDL_SCAN_KERNEL
+  return nullptr;
+}
+
+// The structure of one affine term as FF_* flags: what a shape may assume about it.
+static int flags_of(const KAffine &a) {
+  if (a.col == -1) return FF_CONST;
+  int fl = 0;
+  if (a.col == -2) fl |= FF_ROWID;
+  else if (a.w4) fl |= FF_W4;
+  if (a.shr == 0) fl |= FF_SHR0;
+  if (a.b == 1) fl |= FF_B1;
+  else if (a.b == -1) fl |= FF_BM1;
+  if (a.a == 0) fl |= FF_A0;
+  if (a.col >= 0 && a.narrow) fl |= FF_NARROW;
+  return fl;
+}
+// a static shape's flags fl hold for the term: the same kind of term and width, and every trivial part it assumes
 static bool flags_ok(int fl, const KAffine &a) {
-  if (((fl & FF_CONST) != 0) != (a.col == -1) || ((fl & FF_ROWID) != 0) != (a.col == -2)) return false;
-  if (a.col >= 0 && ((fl & FF_W4) != 0) != (a.w4 != 0)) return false;
-  if ((fl & FF_SHR0) && a.shr != 0) return false;
-  if ((fl & FF_B1) && a.b != 1) return false;
-  if ((fl & FF_BM1) && a.b != -1) return false;
-  if ((fl & FF_A0) && a.a != 0) return false;
-  if ((fl & FF_NARROW) && !a.narrow) return false;
+  const int f = flags_of(a);
+  return ((fl ^ f) & (FF_CONST | FF_ROWID | FF_W4)) == 0 && (fl & ~f) == 0;
+}
+
+// Can the key be computed in 32 bits?  Every part is narrow (its low 32 bits are exact; OR / AND / << are bitwise) and
+// the mask is below the domain.
+static bool jit_key32(const KDesc &k) {
+  if (k.nkeys == 0 || k.key_mask < 0 || k.key_mask > INT32_MAX || k.key_mask >= k.domain) return false;
+  for (int i = 0; i < k.nkeys; i++)
+    if (!(k.key[i].e.col >= 0 && k.key[i].e.narrow)) return false;
   return true;
 }
+
+// does the prepared descriptor satisfy every assumption static shape S compiles in?
 template <class S>
 static bool shape_matches(const KDesc &k) {
   if (k.npreds != S::NPREDS || k.nkeys != S::NKEYS || k.nacc != S::NACC) return false;
   for (int i = 0; i < k.npreds; i++)
     if (k.pred[i].w4 != S::PRED_MODE[i] || (S::PRED_SHR0[i] && k.pred[i].shr != 0)) return false;
-  for (int i = 0; i < k.nkeys; i++) {
+  for (int i = 0; i < k.nkeys; i++)
     if (!flags_ok(S::KEY_FLAGS[i], k.key[i].e) || (S::KEY_SHL0[i] && k.key[i].shl != 0)) return false;
-    if (S::KEY32 && !k.key[i].e.narrow) return false;
-  }
-  if (S::KEY32 && (k.key_mask < 0 || k.key_mask > INT32_MAX || k.key_mask >= k.domain)) return false;
+  if (S::KEY32 && !jit_key32(k)) return false;
   for (int j = 0; j < k.nacc; j++) {
     if (k.acc[j].op != S::ACC_OP[j] || k.acc[j].chain != S::ACC_CHAIN[j] || k.acc[j].nfac != S::ACC_NFAC[j]) return false;
     for (int t = 0; t < k.acc[j].nfac; t++)
@@ -138,26 +150,6 @@ static bool shape_matches(const KDesc &k) {
 // accumulators may live in registers and how) is printed as a shape-traits class, fused_scan_fold_body is instantiated
 // over it by NVRTC for sm_100a and cached per context.  Every constant stays a run-time descriptor field, exactly as with
 // the static shapes, so one compiled kernel serves every plan of that structure.
-
-static int flags_of(const KAffine &a) {
-  if (a.col == -1) return FF_CONST;
-  int fl = 0;
-  if (a.col == -2) fl |= FF_ROWID;
-  else if (a.w4) fl |= FF_W4;
-  if (a.shr == 0) fl |= FF_SHR0;
-  if (a.b == 1) fl |= FF_B1;
-  else if (a.b == -1) fl |= FF_BM1;
-  if (a.a == 0) fl |= FF_A0;
-  if (a.col >= 0 && a.narrow) fl |= FF_NARROW;
-  return fl;
-}
-
-static bool jit_key32(const KDesc &k) {
-  if (k.nkeys == 0 || k.key_mask < 0 || k.key_mask > INT32_MAX || k.key_mask >= k.domain) return false;
-  for (int i = 0; i < k.nkeys; i++)
-    if (!(k.key[i].e.col >= 0 && k.key[i].e.narrow)) return false;     // low 32 bits of every part are exact; OR / AND / << are bitwise
-  return true;
-}
 
 static std::string jit_shape_struct(const KDesc &k, int key32, int rs_g, const int *rk) {
   std::string s = "struct ShapeJit {\n  static constexpr bool kStatic = true;\n";
@@ -196,9 +188,10 @@ static std::string jit_scan_source(const std::string &shape_struct, int nc, int 
   return std::string("#include \"vdl_fused_kernel.cuh\"\n") + shape_struct + b;
 }
 
-static cudaKernel_t jit_scan_compile(vdl_ctx *ctx, const std::string &shape_struct, int nc, int r, int g, int smem_max) {
-  const std::string src = jit_scan_source(shape_struct, nc, r, g);
-  return vdl_jit_kernel(ctx, "scan|" + src, "vdl_scan_jit", smem_max, [&] { return src; });
+// f's generated shape with g register slots (0: shared-memory tables) at f's current geometry
+static const void *jit_scan_compile(vdl_fused *f, int g) {
+  const std::string src = jit_scan_source(f->jit_struct, f->nc, f->r, g);
+  return (const void *)vdl_jit_kernel(f->ctx, "scan|" + src, "vdl_scan_jit", f->smem_max, [&] { return src; });
 }
 
 // Host-only check (no GPU): generate the shape of a Q1-like descriptor and compile it with NVRTC for sm_100a.
@@ -318,14 +311,14 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     if (fd.out_kind[i] == 0 && fd.out_idx[i] < 0) fd.out_idx[i] = k.cnt_idx;
 
   // geometry: consumer threads NC, rows per thread and tile R, ring depth, lane-private tables (or none: register slots)
-  const int smem_max = ctx->smem_optin > 0 ? ctx->smem_optin : 232448;
+  f->smem_max = ctx->smem_optin > 0 ? ctx->smem_optin : 232448;
   if ((size_t)desc->domain * 4 > 64 * 1024) { delete f; return vdl_fail(ctx, VDL_EUNSUPPORTED, "fused scan: key domain %lld too large for the shared-memory slot map", (long long)desc->domain); }
   auto set_geometry = [&](int nc, int r, int gmax, bool tables, int min_stages) -> bool {
     int tile_rows = nc * r, off = 0;
     size_t fixed = (tables ? (size_t)gmax * k.nacc * nc * 8 : 0) + (size_t)desc->domain * 4 + (size_t)gmax * 4 + 16 + 256;
     size_t per_stage = 3 * 8 + 4 + 4 + 2 * (size_t)tile_rows;   // barriers, queue count, queue
     for (int c = 0; c < k.ncols; c++) { k.soff[c] = off; off += ((tile_rows * k.width[c] + 127) / 128) * 128; }
-    int stages = (int)(((long)smem_max - (long)fixed) / (long)(off + per_stage));
+    int stages = (int)(((long)f->smem_max - (long)fixed) / (long)(off + per_stage));
     if (stages < min_stages) return false;
     k.tile_rows = tile_rows; k.stage_bytes = off; k.stage_tx = tile_rows * rowbytes; k.stages = std::min(stages, 12);
     k.gmax = gmax; f->nc = nc; f->r = r;
@@ -457,15 +450,33 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     if (rk == RK_FIRST && (k.acc[j].op != 1 || j != k.first_idx || (__int128)tiles_per_cta * k.tile_rows >= INT32_MAX)) return false;
     return true;
   };
-  auto rs_proofs_hold = [&](const int *rk) -> bool {
-    for (int j = 0; j < k.nacc; j++) if (!rs_proof(j, rk[j])) return false;
-    return true;
+  auto table_geometry = [&]() -> int { default_geometry(); return derive(); };
+  // The register-slot geometry search of both specialised paths: the first geometry of rs_geometries (only the one
+  // VDL_RS_GEOMETRY names, when set) that fits shared memory and for which rep(j) gives every accumulator j a
+  // representation (an RK_*; negative: refused) stays applied, the representations in rk: 1.  Otherwise the tables: 0.
+  // Negative: derive's error.
+  auto rs_search = [&](int *rk, auto rep) -> int {
+    if (getenv("VDL_NO_REGISTER_SLOTS")) return 0;
+    int want_nc = 0, want_r = 0;
+    if (const char *e = getenv("VDL_RS_GEOMETRY")) sscanf(e, "%d,%d", &want_nc, &want_r);
+    for (auto &geo : rs_geometries) {
+      if (want_nc && (geo[0] != want_nc || geo[1] != want_r)) continue;
+      if (!set_geometry(geo[0], geo[1], 8, false, 3)) continue;
+      if (int rc2 = derive()) return -rc2;
+      int j = 0;
+      while (j < k.nacc && (rk[j] = rep(j)) >= 0) j++;
+      if (j == k.nacc) return 1;
+    }
+    int rc2 = table_geometry();
+    return rc2 ? -rc2 : 0;
   };
 
   // Run-time specialisation first: the shape of THIS descriptor, compiled by NVRTC (cached per context).  Worth it for
   // tables of a few million rows and up (VDL_SCAN_JIT_MIN_ROWS; VDL_SCAN_JIT=0 switches it off); without NVRTC, or for
   // small tables, the precompiled instantiations below run: a static shape of vdl_shapes.cuh when one matches, else the
   // generic kernel.  Identical results whichever runs (tests/test_gpu_fuzz.py runs every random plan through both).
+  // Register slots when the key is 32 bits and its domain small: the first geometry that fits, every accumulator in the
+  // cheapest representation proved for it.
   auto try_jit = [&]() -> int {
     const char *e = getenv("VDL_SCAN_JIT");
     if (e && !strcmp(e, "0")) return 0;
@@ -474,65 +485,46 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     if (k.rows < min_rows || f->always_false) return 0;
     const int key32 = jit_key32(k);
     int rk[K_MAX_ACC] = {0};
-    if (key32 && k.nacc <= 8 && k.domain <= 64 && !getenv("VDL_NO_REGISTER_SLOTS")) {
-      int want_nc = 0, want_r = 0;
-      if (const char *g = getenv("VDL_RS_GEOMETRY")) sscanf(g, "%d,%d", &want_nc, &want_r);
-      for (auto &geo : rs_geometries) {
-        if (want_nc && (geo[0] != want_nc || geo[1] != want_r)) continue;
-        if (!set_geometry(geo[0], geo[1], 8, false, 3)) continue;
-        int rc2 = derive();
-        if (rc2) return -rc2;
-        for (int j = 0; j < k.nacc; j++)      // cheapest representation whose proof holds
-          rk[j] = rs_proof(j, RK_FIRST) ? RK_FIRST : (rs_proof(j, RK_N32) ? RK_N32 : (rs_proof(j, RK_MADW) ? RK_MADW : RK_WIDE));
+    if (key32 && k.nacc <= 8 && k.domain <= 64) {
+      int m = rs_search(rk, [&](int j) {
+        return rs_proof(j, RK_FIRST) ? RK_FIRST : (rs_proof(j, RK_N32) ? RK_N32 : (rs_proof(j, RK_MADW) ? RK_MADW : RK_WIDE));
+      });
+      if (m < 0) return m;
+      if (m > 0) {
         f->jit_struct = jit_shape_struct(k, key32, 8, rk);
-        cudaKernel_t kh = jit_scan_compile(ctx, f->jit_struct, geo[0], geo[1], 8, smem_max);
-        if (kh) {
-          f->jit_rs_kernel[8] = kh; f->jit_rs_tried[8] = true;
-          f->rs = true; f->rs_gmax = 8; f->jit = true;
+        if ((f->rs_kernel[8] = jit_scan_compile(f, 8))) {
+          f->rs_tried[8] = f->rs = f->jit = true;
           return 1;
         }
-        break;
+        if (int rc2 = table_geometry()) return -rc2;
       }
-      default_geometry();
-      int rc2 = derive();
-      if (rc2) return -rc2;
     }
     f->jit_struct = jit_shape_struct(k, key32, 0, rk);
-    f->jit_kernel = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, 0, smem_max);
-    if (!f->jit_kernel) return 0;
-    f->jit = true;
-    return 1;
+    f->kernel = jit_scan_compile(f, 0);
+    f->jit = f->kernel != nullptr;
+    return f->jit;
   };
 
-  // pick the kernel: a static shape whose assumptions all hold, else the generic one; a shape with register slots
-  // runs in that mode when the key domain's slots and the 32-bit proofs allow it
-  f->kernel = scan_kernel_for<GenericShape>(f->nc, f->r);
+  // Else a static shape whose assumptions all hold, else the generic kernel.  A static shape with register slots runs
+  // in that mode in the first geometry where the assumptions still hold and its ACC_RK representations are proved.
   auto try_shape = [&](auto shape_tag) -> int {
     using S = decltype(shape_tag);
     if (!shape_matches<S>(k)) return 0;
-    f->kernel = scan_kernel_for<S>(f->nc, f->r);
     f->shape = S::kName;
     if constexpr (S::RS_G > 0) {
-      if (getenv("VDL_NO_REGISTER_SLOTS")) return 1;
-      int want_nc = 0, want_r = 0;
-      if (const char *e = getenv("VDL_RS_GEOMETRY")) sscanf(e, "%d,%d", &want_nc, &want_r);
-      for (auto &geo : rs_geometries) {
-        if (want_nc && (geo[0] != want_nc || geo[1] != want_r)) continue;
-        if (!rs_kernel_for<S>(geo[0], geo[1], S::RS_G) || !set_geometry(geo[0], geo[1], S::RS_G, false, 3)) continue;
-        int rc2 = derive();
-        if (rc2) return -rc2;
-        if (shape_matches<S>(k) && rs_proofs_hold(S::ACC_RK)) {
-          for (int g : rs_slot_counts) f->rs_kernel[g] = rs_kernel_for<S>(geo[0], geo[1], g);
-          f->kernel = f->rs_kernel[S::RS_G];
-          f->rs = true;
-          f->rs_gmax = S::RS_G;
-          return 1;
+      int rk[K_MAX_ACC];
+      int m = rs_search(rk, [&](int j) { return shape_matches<S>(k) && rs_proof(j, S::ACC_RK[j]) ? S::ACC_RK[j] : -1; });
+      if (m < 0) return m;
+      if (m > 0) {
+        for (int g : rs_slot_counts) {
+          f->rs_kernel[g] = static_kernel<S>(f->nc, f->r, g);
+          f->rs_tried[g] = true;
         }
+        f->rs = true;
+        return 1;
       }
-      default_geometry();               // no register-slot geometry qualified: back to the shared-memory tables
-      int rc2 = derive();
-      if (rc2) return -rc2;
     }
+    f->kernel = static_kernel<S>(f->nc, f->r, 0);
     return 1;
   };
   if (!getenv("VDL_GENERIC_ONLY")) {
@@ -549,6 +541,7 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     if (m == 0) m = try_shape(ShapeSel1Key2Sum5{});
     if (m < 0) { vdl_fused_destroy(f); return -m; }
   }
+  if (!f->rs && !f->kernel) f->kernel = static_kernel<GenericShape>(f->nc, f->r, 0);
   if (getenv("VDL_DEBUG_SHAPE")) {
     fprintf(stderr, "[vdl] fused scan: shape=%s%s nc=%d r=%d stages=%d gmax=%d npreds=%d nkeys=%d nacc=%d smem=%zu\n", f->shape, f->rs ? " (register slots)" : "", f->nc, f->r, k.stages, k.gmax, k.npreds, k.nkeys, k.nacc, f->smem_bytes);
     for (int i = 0; i < k.npreds; i++) fprintf(stderr, "[vdl]   pred %d: mode=%d shr=%d\n", i, k.pred[i].w4, k.pred[i].shr);
@@ -598,10 +591,10 @@ extern "C" int vdl_fused_prepare(vdl_ctx *ctx, const vdl_fused_desc *desc, vdl_f
     cudaFuncGetAttributes(&fa, fused_init_kernel); cudaFuncGetAttributes(&fa, fused_choose_kernel);
     cudaGetLastError();
   }
-  cudaError_t e = cudaFuncSetAttribute(f->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+  cudaError_t e = f->kernel ? cudaFuncSetAttribute(f->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, f->smem_max) : cudaSuccess;
   if (e != cudaSuccess) { vdl_fused_destroy(f); return vdl_cuda_fail(ctx, e, "cudaFuncSetAttribute(fused_scan_fold_kernel)"); }
   for (int g : rs_slot_counts)
-    if (f->rs && f->rs_kernel[g] && (e = cudaFuncSetAttribute(f->rs_kernel[g], cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max)) != cudaSuccess) {
+    if (f->rs_kernel[g] && (e = cudaFuncSetAttribute(f->rs_kernel[g], cudaFuncAttributeMaxDynamicSharedMemorySize, f->smem_max)) != cudaSuccess) {
       vdl_fused_destroy(f);
       return vdl_cuda_fail(ctx, e, "cudaFuncSetAttribute(fused_scan_fold_kernel, register slots)");
     }
@@ -628,21 +621,19 @@ extern "C" int vdl_fused_launch_ex(vdl_fused *f, int self_finalize) {
     f->cb.table_clean = true;
   }
   VDL_TRY(f->timer.begin(ctx));
-  cudaKernel_t jit_launch = f->jit ? f->jit_kernel : nullptr;
+  const void *kernel = f->kernel;
   if (f->rs) {
-    int g = f->rs_gmax;
+    int g = 8;                    // the slots of prepare's register-slot kernel
     if (f->groups_seen >= 0 && !getenv("VDL_RS_ALL_SLOTS"))
       for (int c : rs_slot_counts)
         if (c >= f->groups_seen && c < g) {
-          if (f->jit && !f->jit_rs_tried[c]) {        // the variant with fewer register slots: compiled on first use
-            f->jit_rs_tried[c] = true;
-            const int smem_max = ctx->smem_optin > 0 ? ctx->smem_optin : 232448;
-            f->jit_rs_kernel[c] = jit_scan_compile(ctx, f->jit_struct, f->nc, f->r, c, smem_max);
+          if (!f->rs_tried[c]) {        // a run-time compiled variant with fewer register slots: compiled on first use
+            f->rs_tried[c] = true;
+            f->rs_kernel[c] = jit_scan_compile(f, c);
           }
-          if (f->jit ? f->jit_rs_kernel[c] != nullptr : f->rs_kernel[c] != nullptr) g = c;
+          if (f->rs_kernel[c]) g = c;
         }
-    if (f->jit) jit_launch = f->jit_rs_kernel[g];
-    else f->kernel = f->rs_kernel[g];
+    kernel = f->rs_kernel[g];
     f->kd.gmax = g;
   }
   const bool scan = f->kd.rows > 0 && !f->always_false;
@@ -652,12 +643,8 @@ extern "C" int vdl_fused_launch_ex(vdl_fused *f, int self_finalize) {
     cb.fd.parts = f->kd.table;           // the epilogue's single-rank finalize
     if (self_finalize) cb.fd.seq++;
     f->kd.epilogue = self_finalize == 2 ? 3 : (self_finalize ? 2 : 1);
-    if (jit_launch) {
-      void *args[] = {(void *)&f->kd, (void *)&cb.fd, (void *)&cb.xd};
-      VDL_CUDA(ctx, cudaLaunchKernel((const void *)jit_launch, dim3(f->grid), dim3(f->nc + 32), args, f->smem_bytes, ctx->stream));
-    } else {
-      f->kernel<<<f->grid, f->nc + 32, f->smem_bytes, ctx->stream>>>(f->kd, cb.fd, cb.xd);
-    }
+    void *args[] = {(void *)&f->kd, (void *)&cb.fd, (void *)&cb.xd};
+    VDL_CUDA(ctx, cudaLaunchKernel(kernel, dim3(f->grid), dim3(f->nc + 32), args, f->smem_bytes, ctx->stream));
     ctx->launches++;
     f->cb.table_clean = self_finalize != 0;
   } else if (self_finalize == 2) {       // nothing to scan here, but the other ranks wait for this rank's table

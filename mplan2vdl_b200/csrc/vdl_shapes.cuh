@@ -1,10 +1,11 @@
 // Static shapes of the fused scan: compile-time answers to the structural questions of a descriptor
-// (see "SHAPES" in vdl_fused.cu).  A shape only fixes STRUCTURE -- counts, column widths, which of
+// (see "SHAPES" in vdl_fused_kernel.cuh).  A shape only fixes STRUCTURE -- counts, column widths, which of
 // shr / a / b are trivial, what fits 32 bits; every constant stays a run-time descriptor field, so a shape
 // serves any plan of that structure (other columns, other bounds, other scale factors).  The host checks all
-// of a shape's assumptions against the prepared descriptor (shape_matches) before launching it and otherwise
-// uses GenericShape; results are identical.  tools/print_shape.py prints the struct for a plan (needs a GPU:
-// narrowing depends on the column statistics).
+// of a shape's assumptions against the prepared descriptor (shape_matches, vdl_fused.cu) before launching it and
+// otherwise uses GenericShape; results are identical.  To see the struct a plan needs, run it with VDL_DEBUG_JIT=1
+// and VDL_SCAN_JIT_MIN_ROWS=0: the scan prints the `ShapeJit` it generates for the prepared descriptor, in these
+// fields (needs a GPU: narrowing depends on the column statistics).
 #pragma once
 
 #define FF_COLN (FF_SHR0 | FF_B1 | FF_A0 | FF_NARROW)      /* a plain 8-byte column whose values fit int32 */

@@ -457,6 +457,14 @@ def _cases(n=40_000, seed=1):
                      (SUM, [T(4), T(5, 0, 100, -1), T(6, 0, 100)]), (SUM, [T(5)]), (COUNT, [])],
               posts=[(DIVIDE, (P_FOLD, 2), (P_FOLD, 7)), (DIVIDE, (P_FOLD, 3), (P_FOLD, 7))])
     out["q1_32_keys"] = (q1, dict(RS, static="sel1_key2_sum5", static_tables="sel1_key2_sum5"))
+    # the same with only 4 of the 32 keys present, as TPC-H Q1's four flag / status pairs: the second step of _check
+    # launches the 4-slot variant of the static and of the run-time compiled register-slot kernels (own generator: the
+    # other cases keep their data)
+    rng4 = np.random.default_rng([seed, 4])
+    pair = rng4.choice(np.array([(2, 2), (3, 2), (3, 3), (4, 2)]), n)
+    rf4, ls4 = 8 * pair[:, 0] + rng4.integers(0, 8, n), 8 * pair[:, 1] + rng4.integers(0, 8, n)
+    out["q1_4_keys"] = (dict(q1, cols=[date, rf4, ls4, qty, price, disc, tax]),
+                        dict(RS, static="sel1_key2_sum5", static_tables="sel1_key2_sum5"))
     # shifted 8-byte columns whose raw values do not fit int32: predicates (mode 2), factors (FF_NARROW)
     x = rng.integers(2**31, 2**48, n)
     x2 = rng.integers(2**31, 2**32, n)
