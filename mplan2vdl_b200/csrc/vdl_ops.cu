@@ -521,35 +521,10 @@ extern "C" int vdl_op_cross_product(vdl_ctx *ctx, vdl_vec left, vdl_vec right, i
   return VDL_OK;
 }
 
-// ---------------------------------------------------------------------------------- Partition
-// Vlite.hs:1082-1098 emits Partition(key, RangeC(min,1,max-min+1)); its result is the scatter position that
-// sorts rows stably by key (1057-1060, 1172).  bucket(v) = number of pivots below v (App. G3); the
-// permutation is a stable LSD radix sort of row ids by bucket, 8 bits per pass over the bits the pivot
-// count needs (Q1: 6 bits = 1 pass; Q3's 38-bit composite key = 5 passes).
+// ---------------------------------------------------------------------------------- stable LSD radix sort (Partition, Order)
+// 8 bits per pass over tiles of RDX_TILE rows: a digit histogram per tile, one exclusive scan over all of them (digit-major:
+// the global stable order), a stable scatter of key and row id.
 #define RDX_TILE 4096
-
-__device__ __forceinline__ u64 bucket_of(i64 v, i64 pfrom, i64 pstep, i64 pcount) {
-  if (v <= pfrom) return 0;
-  u64 d = (u64)v - (u64)pfrom;
-  u64 b = pstep == 1 ? d : (d + (u64)pstep - 1) / (u64)pstep;     // every emitted Partition has unit-step pivots (Vlite.hs:1088-1091)
-  return b > (u64)pcount ? (u64)pcount : b;
-}
-
-__global__ void __launch_bounds__(256) bucket_kernel(Operand data, i64 n, i64 pfrom, i64 pstep, i64 pcount, u64 *__restrict__ key, i64 *__restrict__ idx) {
-  i64 stride = (i64)gridDim.x * blockDim.x;
-  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-    i64 v = op_ld(data, i);
-    u64 b;
-    if (v <= pfrom) b = 0;
-    else {
-      u64 d = (u64)v - (u64)pfrom;
-      b = (d + (u64)pstep - 1) / (u64)pstep;
-      if (b > (u64)pcount) b = (u64)pcount;
-    }
-    key[i] = b;
-    idx[i] = i;
-  }
-}
 
 // digit histogram per block, stored digit-major: hist[d * nblocks + block]
 __global__ void __launch_bounds__(256) radix_hist_kernel(const u64 *__restrict__ key, i64 n, int shift, i64 nblocks, i64 *__restrict__ hist) {
@@ -565,7 +540,8 @@ __global__ void __launch_bounds__(256) radix_hist_kernel(const u64 *__restrict__
   hist[(i64)threadIdx.x * nblocks + blockIdx.x] = h[threadIdx.x];
 }
 
-// stable scatter: rank inside the block = elements with the same digit earlier in the block
+// stable scatter: rank inside the block = elements with the same digit earlier in the block.  No idx_in: the row ids are
+// the positions themselves (the first pass of a sort)
 __global__ void __launch_bounds__(256) radix_scatter_kernel(const u64 *__restrict__ key_in, const i64 *__restrict__ idx_in, i64 n, int shift,
                                                             i64 nblocks, const i64 *__restrict__ offs, u64 *__restrict__ key_out,
                                                             i64 *__restrict__ idx_out) {
@@ -601,9 +577,80 @@ __global__ void __launch_bounds__(256) radix_scatter_kernel(const u64 *__restric
     if (valid) {
       i64 dst = offs[(i64)d * nblocks + blockIdx.x] + wbase[warp][d] + rank_in_warp;
       key_out[dst] = k;
-      idx_out[dst] = idx_in[i];
+      idx_out[dst] = idx_in ? idx_in[i] : i;
     }
   }
+}
+
+__global__ void __launch_bounds__(256) order_gather_kernel(const u64 *__restrict__ src, const i64 *__restrict__ pos, i64 n, u64 *__restrict__ dst) {
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) dst[i] = src[pos[i]];
+}
+
+namespace {
+struct VecScope {      // temporaries of one op, released (stream-ordered) when it returns
+  vdl_ctx *ctx;
+  std::vector<vdl_vec> v;
+  ~VecScope() { for (vdl_vec h : v) vdl_vec_free(ctx, h); }
+};
+}  // namespace
+
+// Stable sort of positions 0..n-1 (n >= 1) by packed words: word w of position i at words[w * n + i], word 0 the least
+// significant, wbits[w] >= 1 bits of it in use (Order packs only the keys that are not constant, Partition has at least one
+// pivot).  *out = the positions in sorted order, a new vector of length n.  Words are sorted least significant first, each
+// gathered into the order reached so far.
+static int lsd_sort(vdl_ctx *ctx, const u64 *words, int nwords, const int *wbits, i64 n, vdl_vec *out) {
+  const i64 nb = (n + RDX_TILE - 1) / RDX_TILE;
+  vdl_vec tk[2], ti[2];
+  VecScope tmp{ctx, {}};
+  for (int k = 0; k < 2; k++) {
+    VDL_TRY(vec_new(ctx, VDL_I64, n, &tk[k])); tmp.v.push_back(tk[k]);
+    VDL_TRY(vec_new(ctx, VDL_I64, n, &ti[k])); tmp.v.push_back(ti[k]);
+  }
+  int cur = 0;
+  VDL_TRY(scratch_reserve(ctx, scan_elems(256 * nb) * 8));
+  i64 *hist = (i64 *)ctx->scratch;
+  u64 *key[2] = {(u64 *)ctx->vecs[tk[0]].ptr, (u64 *)ctx->vecs[tk[1]].ptr};
+  i64 *idx[2] = {(i64 *)ctx->vecs[ti[0]].ptr, (i64 *)ctx->vecs[ti[1]].ptr};
+  const i64 *ids = nullptr;       // the positions in the order reached so far; none before the first pass
+  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
+  for (int w = 0; w < nwords; w++) {
+    const u64 *kin = words + (i64)w * n;
+    if (w > 0) {          // the next more significant word, in the order reached so far
+      order_gather_kernel<<<grid, 256, 0, ctx->stream>>>(kin, ids, n, key[cur]);
+      ctx->launches++;
+      kin = key[cur];
+    }
+    for (int shift = 0; shift < wbits[w]; shift += 8) {
+      radix_hist_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, n, shift, nb, hist);
+      device_exclusive_scan(ctx, hist, 256 * nb);
+      radix_scatter_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, ids, n, shift, nb, hist, key[cur ^ 1], idx[cur ^ 1]);
+      ctx->launches += 2;
+      cur ^= 1;
+      kin = key[cur];
+      ids = idx[cur];
+    }
+  }
+  VDL_CUDA(ctx, cudaGetLastError());
+  tmp.v.erase(std::find(tmp.v.begin(), tmp.v.end(), ti[cur]));
+  *out = ti[cur];
+  return VDL_OK;
+}
+
+// ---------------------------------------------------------------------------------- Partition
+// Vlite.hs:1082-1098 emits Partition(key, RangeC(min,1,max-min+1)); its result is the scatter position that
+// sorts rows stably by key (1057-1060, 1172).  bucket(v) = number of pivots below v (App. G3).  Up to 256 buckets of
+// unit-step pivots the permutation comes from a counting partition; otherwise it is lsd_sort of the rows by bucket (one
+// word of the bits the pivot count needs: Q3's 38-bit composite key = 5 passes), inverted.
+__device__ __forceinline__ u64 bucket_of(i64 v, i64 pfrom, i64 pstep, i64 pcount) {
+  if (v <= pfrom) return 0;
+  u64 d = (u64)v - (u64)pfrom;
+  u64 b = pstep == 1 ? d : (d + (u64)pstep - 1) / (u64)pstep;     // every emitted Partition has unit-step pivots (Vlite.hs:1088-1091)
+  return b > (u64)pcount ? (u64)pcount : b;
+}
+
+__global__ void __launch_bounds__(256) bucket_kernel(Operand data, i64 n, i64 pfrom, i64 pstep, i64 pcount, u64 *__restrict__ key) {
+  i64 stride = (i64)gridDim.x * blockDim.x;
+  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) key[i] = bucket_of(op_ld(data, i), pfrom, pstep, pcount);
 }
 
 // Counting partition for <= 256 buckets (every low-cardinality group-by: Q1's 32, Q5's 128): two passes over the keys, no
@@ -621,9 +668,7 @@ __global__ void __launch_bounds__(256) radix_scatter_kernel(const u64 *__restric
 template <int KIND>
 __device__ __forceinline__ int bucket_at(const Operand &o, i64 i, i64 pfrom, i64 pcount) {
   const i64 v = KIND == 0 ? __ldg((const i64 *)o.p + i) : (KIND == 1 ? (i64)__ldg((const int *)o.p + i) : (i64)((u64)o.from + (u64)i * (u64)o.step));
-  if (v <= pfrom) return 0;
-  const u64 d = (u64)v - (u64)pfrom;
-  return (int)(d > (u64)pcount ? (u64)pcount : d);
+  return (int)bucket_of(v, pfrom, 1, pcount);
 }
 // lanes whose bucket index has bit K set.  Written in PTX so that the test stays "and, compare with zero" (one LOP3 with a
 // predicate result): the compiler's own canonical form is shift, mask, compare -- three instructions of the pipe that bounds
@@ -854,6 +899,9 @@ extern "C" int vdl_op_partition(vdl_ctx *ctx, vdl_vec data, int64_t pfrom, int64
     VDL_CUDA(ctx, cudaGetLastError());
     return VDL_OK;
   }
+  VecScope tmp{ctx, {}};
+  vdl_vec sorted = -1;
+  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
   if (n > 0) {
     // one cheap pass first: keys that are already in bucket order sort to the identity permutation, which stays a
     // virtual range -- no radix passes, and a Scatter by it is the source vector itself
@@ -865,34 +913,23 @@ extern "C" int vdl_op_partition(vdl_ctx *ctx, vdl_vec data, int64_t pfrom, int64
     ctx->launches++;
     VDL_TRY(read_scalar(ctx, d_desc, &h_desc, sizeof(int)));
     if (h_desc == 0) return vec_new_range(ctx, 0, 1, n, out);      // (its domain is n: positions 0..n-1)
+    // the rows in stable bucket order: one word of `bits` bits per row
+    vdl_vec kv;
+    VDL_TRY(vec_new(ctx, VDL_I64, n, &kv));
+    tmp.v.push_back(kv);
+    bucket_kernel<<<grid, 256, 0, ctx->stream>>>(od, n, pfrom, pstep, pcount, (u64 *)ctx->vecs[kv].ptr);
+    ctx->launches++;
+    VDL_TRY(lsd_sort(ctx, (const u64 *)ctx->vecs[kv].ptr, 1, &bits, n, &sorted));
+    tmp.v.push_back(sorted);
   }
+  // allocated after the sort, whose temporaries are released by then: the peak stays at five n-row vectors
   VDL_TRY(vec_new(ctx, VDL_I64, n, out));
   ctx->vecs[*out].domain = n;
   ctx->vecs[*out].is_perm = true;
   if (n == 0) return VDL_OK;
-  i64 nb = (n + RDX_TILE - 1) / RDX_TILE;
-  // temporaries: key/idx ping-pong + histogram
-  vdl_vec tk[2], ti[2];
-  for (int k = 0; k < 2; k++) { VDL_TRY(vec_new(ctx, VDL_I64, n, &tk[k])); VDL_TRY(vec_new(ctx, VDL_I64, n, &ti[k])); }
-  VDL_TRY(scratch_reserve(ctx, scan_elems(256 * nb) * 8));
-  i64 *hist = (i64 *)ctx->scratch;
-  u64 *key[2] = {(u64 *)ctx->vecs[tk[0]].ptr, (u64 *)ctx->vecs[tk[1]].ptr};
-  i64 *idx[2] = {(i64 *)ctx->vecs[ti[0]].ptr, (i64 *)ctx->vecs[ti[1]].ptr};
-  int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
-  bucket_kernel<<<grid, 256, 0, ctx->stream>>>(od, n, pfrom, pstep, pcount, key[0], idx[0]);
-  ctx->launches++;
-  int cur = 0;
-  for (int shift = 0; shift < bits; shift += 8) {
-    radix_hist_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(key[cur], n, shift, nb, hist);
-    device_exclusive_scan(ctx, hist, 256 * nb);
-    radix_scatter_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(key[cur], idx[cur], n, shift, nb, hist, key[cur ^ 1], idx[cur ^ 1]);
-    ctx->launches += 2;
-    cur ^= 1;
-  }
-  invert_perm_kernel<<<grid, 256, 0, ctx->stream>>>(idx[cur], n, (i64 *)ctx->vecs[*out].ptr);
+  invert_perm_kernel<<<grid, 256, 0, ctx->stream>>>((const i64 *)ctx->vecs[sorted].ptr, n, (i64 *)ctx->vecs[*out].ptr);
   ctx->launches++;
   VDL_CUDA(ctx, cudaGetLastError());
-  for (int k = 0; k < 2; k++) { VDL_TRY(vdl_vec_free(ctx, tk[k])); VDL_TRY(vdl_vec_free(ctx, ti[k])); }
   return VDL_OK;
 }
 
@@ -900,8 +937,7 @@ extern "C" int vdl_op_partition(vdl_ctx *ctx, vdl_vec data, int64_t pfrom, int64
 // Every key becomes its distance from its minimum (ascending) or from its maximum (descending) in uint64 -- exact at
 // INT64_MIN / INT64_MAX, where -x is not -- and the distances are bit-packed: the last key in the least significant bits,
 // each key in the bits its range needs, a constant key in none.  Keys that do not fit one 64-bit word spill into further
-// words (word 0 least significant).  A full order is Partition's stable LSD radix sort (radix_hist_kernel,
-// device_exclusive_scan, radix_scatter_kernel), least significant word first, over the bits that are set.  With a LIMIT a
+// words (word 0 least significant).  A full order is lsd_sort over the packed words, the one Partition uses.  With a LIMIT a
 // radix select comes first: the pack kernel also counts the top 8-bit digit, the host finds the digit at which the count
 // reaches the limit, the rows at or below it are compacted in row order by FoldSelect (so ties stay stable) -- refined digit
 // by digit while there are many more of them than the limit -- and only those candidates are sorted.
@@ -992,62 +1028,6 @@ __global__ void __launch_bounds__(256) order_candidate_kernel(const u64 *__restr
   for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) flag[i] = (top[i] >> s) <= prefix;
 }
 
-__global__ void __launch_bounds__(256) order_gather_kernel(const u64 *__restrict__ src, const i64 *__restrict__ pos, i64 n, u64 *__restrict__ dst) {
-  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) dst[i] = src[pos[i]];
-}
-
-__global__ void __launch_bounds__(256) order_iota_kernel(i64 *__restrict__ out, i64 n) {
-  for (i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) out[i] = i;
-}
-
-namespace {
-struct VecScope {      // temporaries of one op, released (stream-ordered) when it returns
-  vdl_ctx *ctx;
-  std::vector<vdl_vec> v;
-  ~VecScope() { for (vdl_vec h : v) vdl_vec_free(ctx, h); }
-};
-}  // namespace
-
-// Stable LSD sort of positions 0..n-1 by packed words (word w of position i at words[w * n + i], w = 0 least significant,
-// wbits[w] bits used): *out = the positions in order, a new vector of length n.
-static int order_lsd(vdl_ctx *ctx, const u64 *words, int nwords, const int *wbits, i64 n, vdl_vec *out) {
-  const i64 nb = (n + RDX_TILE - 1) / RDX_TILE;
-  vdl_vec tk[2], ti[2];
-  VecScope tmp{ctx, {}};
-  for (int k = 0; k < 2; k++) {
-    VDL_TRY(vec_new(ctx, VDL_I64, n, &tk[k])); tmp.v.push_back(tk[k]);
-    VDL_TRY(vec_new(ctx, VDL_I64, n, &ti[k])); tmp.v.push_back(ti[k]);
-  }
-  int cur = 0;
-  VDL_TRY(scratch_reserve(ctx, scan_elems(256 * nb) * 8));
-  i64 *hist = (i64 *)ctx->scratch;
-  u64 *key[2] = {(u64 *)ctx->vecs[tk[0]].ptr, (u64 *)ctx->vecs[tk[1]].ptr};
-  i64 *idx[2] = {(i64 *)ctx->vecs[ti[0]].ptr, (i64 *)ctx->vecs[ti[1]].ptr};
-  const int grid = (int)std::max<i64>(1, std::min<i64>((n + 255) / 256, (i64)ctx->sm_count * 16));
-  order_iota_kernel<<<grid, 256, 0, ctx->stream>>>(idx[0], n);
-  ctx->launches++;
-  for (int w = 0; w < nwords; w++) {
-    const u64 *kin = words + (i64)w * n;
-    if (w > 0) {          // the next more significant word, in the order reached so far
-      order_gather_kernel<<<grid, 256, 0, ctx->stream>>>(kin, idx[cur], n, key[cur]);
-      ctx->launches++;
-      kin = key[cur];
-    }
-    for (int shift = 0; shift < wbits[w]; shift += 8) {
-      radix_hist_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, n, shift, nb, hist);
-      device_exclusive_scan(ctx, hist, 256 * nb);
-      radix_scatter_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(kin, idx[cur], n, shift, nb, hist, key[cur ^ 1], idx[cur ^ 1]);
-      ctx->launches += 2;
-      cur ^= 1;
-      kin = key[cur];
-    }
-  }
-  VDL_CUDA(ctx, cudaGetLastError());
-  tmp.v.erase(std::find(tmp.v.begin(), tmp.v.end(), ti[cur]));
-  *out = ti[cur];
-  return VDL_OK;
-}
-
 extern "C" int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const int *descending, int64_t limit, vdl_vec *out) {
   if (!ctx || !out || (nkeys > 0 && !keys)) return VDL_EINVAL;
   if (nkeys < 0 || nkeys > VDL_MAX_ORDER_KEYS) return vdl_fail(ctx, VDL_EINVAL, "Order: %d keys (at most %d)", nkeys, VDL_MAX_ORDER_KEYS);
@@ -1122,7 +1102,7 @@ extern "C" int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const 
   ctx->launches++;
   VDL_CUDA(ctx, cudaGetLastError());
   if (!select) {
-    VDL_TRY(order_lsd(ctx, words, nwords, wbits, n, out));
+    VDL_TRY(lsd_sort(ctx, words, nwords, wbits, n, out));
     ctx->vecs[*out].domain = n;
     ctx->vecs[*out].is_perm = true;
     return VDL_OK;
@@ -1169,7 +1149,7 @@ extern "C" int vdl_op_order(vdl_ctx *ctx, int nkeys, const vdl_vec *keys, const 
   const int cgrid = (int)std::max<i64>(1, std::min<i64>((c + 255) / 256, (i64)ctx->sm_count * 16));
   for (int w = 0; w < nwords; w++) order_gather_kernel<<<cgrid, 256, 0, ctx->stream>>>(words + (i64)w * n, cpos, c, cwords + (i64)w * c);
   ctx->launches += nwords;
-  VDL_TRY(order_lsd(ctx, cwords, nwords, wbits, c, &sorted));
+  VDL_TRY(lsd_sort(ctx, cwords, nwords, wbits, c, &sorted));
   tmp.v.push_back(sorted);
   ctx->vecs[sorted].len = m;                        // the first m candidates in order, mapped back to row positions
   return vdl_op_gather(ctx, cand, sorted, out);

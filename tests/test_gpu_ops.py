@@ -76,6 +76,33 @@ def test_partition_wide_keys_multi_pass():
     np.testing.assert_array_equal(r["sorted"], np.sort(k))
 
 
+# The radix sort that Partition shares with Order: its first pass takes the row ids from the positions, so ties (here
+# also the clamped buckets below the first pivot and above the last) check that it is stable.
+@pytest.mark.parametrize("n", [1, 4095, 4097, 200_003])                   # around the radix sort's 4096-row tiles
+@pytest.mark.parametrize("keys", ["unique", "ties", "ordered"])
+@pytest.mark.parametrize("pfrom,pcount,pstep", [
+    pytest.param(0, 256, 1, id="count256"),           # the first count past the counting partition: 2 passes
+    pytest.param(-5000, 70_000, 1, id="count70000"),  # 3 passes
+    pytest.param(0, 2**38, 1, id="count2e38"),        # Q3's composite key: 5 passes
+    pytest.param(7, 10, 3, id="step3")])              # a non-unit step takes the radix sort at any count
+def test_partition_radix_sort_stable(pfrom, pcount, pstep, keys, n):
+    plan = K.PART.replace("3,RangeC,val,0,4,1", f"3,RangeC,val,{pfrom},{pcount},{pstep}")
+    rng = np.random.default_rng(n)
+    last = pfrom + (pcount - 1) * pstep
+    if keys == "unique":
+        k = pfrom + rng.permutation(n).astype(I64) * max(1, pcount * pstep // n)
+    else:       # few distinct values, with some at or below the first pivot and above the last (the clamped buckets)
+        pool = np.array([np.iinfo(I64).min, pfrom - 1, pfrom, pfrom + 1, pfrom + pstep * (pcount // 2), last, last + 1,
+                         np.iinfo(I64).max], I64)
+        k = pool[rng.integers(0, len(pool), n)]
+        if keys == "ordered":
+            k = np.sort(k)
+    r = both(plan, k=k)
+    d = k.astype(np.uint64) - np.uint64(pfrom % 2**64)                  # bucket = pivots below the key
+    b = np.where(k <= pfrom, 0, np.minimum((d + np.uint64(pstep - 1)) // np.uint64(pstep), np.uint64(pcount)))
+    np.testing.assert_array_equal(r["sorted"], k[np.argsort(b, kind="stable")])
+
+
 def test_scatter_index_space():
     plan = ("1,Load,t.p\n2,Project,val,Id 1,p\n3,RangeV,val,0,Id 2,1\n4,FoldSelect,val,Id 3,val,Id 2,val\n"
             "5,RangeV,val,1,Id 4,0\n6,RangeV,val,0,Id 5,1\n7,Scatter,Id 5,Id 6,val,Id 4,val\n"
